@@ -2,6 +2,7 @@
 """Benchmark of the generation.py hot path (seed->cloud kNN, gather/centre, fn, rotate, fd, x + n*d).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1|3|4|5] [--mode fp32|tc|tf32|fast]
+                    [--dump-outputs DIR]
 
 Workloads (BASELINE.json `configs`, 0-based in the file; the numbers below are the file's positions 1..4 + 1):
   --config 1 (default)  configs[1]: one 2,048-pt sphere cloud x4 -> 8,192 seeds PER GPU (weak scaling), parity mode `tc`
@@ -219,6 +220,16 @@ def run_reference(args):
     print(json.dumps(line))
 
 
+def dump_points(path, pts, limit=64 << 20):
+    """--dump-outputs: the [S,3] f64 points of the last timed step as <path>/points.npy, so that two builds can be compared
+    output for output.  Above `limit` bytes, a fixed seeded sample of rows (ascending order) that is the same at every run."""
+    if pts.nbytes > limit:
+        n = limit // pts.itemsize // pts.shape[1]
+        pts = pts[np.sort(np.random.default_rng(0).choice(pts.shape[0], n, replace=False))]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "points.npy"), pts)
+
+
 def kernel_rooflines(report, steps, peaks, step_ms_total, products=1):
     """Per-kernel roofline entries from the library's live recording: each label is graded on the roofline that binds it
     (tensor: FLOPs vs the measured sustained bf16 peak -- `frac` is ALGORITHMIC, the bound is chosen on the ISSUED products,
@@ -341,6 +352,7 @@ def run_ours(args):
     value = S_total * args.steps / (ms_total / 1e3)
     assert out.shape == (S_total, 3) and bool(torch.isfinite(out).all())
     N.check_device("bench")
+    last_out = out.cpu().numpy() if args.dump_outputs and rank == 0 else None      # before the e2e leg reuses the generator
 
     # ---- end to end through the public host API: every step copies the cloud and the rank's seeds from pinned host memory,
     # runs the pipeline, all-gathers, and copies the gathered [S,3] points back to the host (L2 flushed between steps)
@@ -425,6 +437,8 @@ def run_ours(args):
             "gpu_eager_baseline": gpu_eager,
         }
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_points(args.dump_outputs, last_out)
     if world > 1:
         dist.destroy_process_group()
 
@@ -443,7 +457,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-API end-to-end leg (large configs)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-eager", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the points the last one computed as DIR/points.npy (f64; a fixed sample above 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -24,7 +24,10 @@ def test_library_exports_every_declared_symbol():
     for name in declared:
         assert hasattr(lib, name), name
     assert lib.sapcu_abi_version() == 1
-    assert lib.sapcu_launch_count() == 0
+    # the counter is per process, and GPU tests of the same session may have launched kernels already: load a fresh copy
+    fresh = subprocess.run([sys.executable, "-c", "import sys; sys.path.insert(0, %r); import sapcu_b200; "
+                            "print(sapcu_b200.lib().sapcu_launch_count())" % ROOT], capture_output=True, text=True, check=True)
+    assert fresh.stdout.strip() == "0"
     assert lib.sapcu_knn_workspace_bytes(2048) >= 2048 * 12 + 256
 
 
@@ -82,9 +85,10 @@ def test_config_and_checkpoint_boundary(tmp_path):
 
 
 def test_reference_yaml_loads_unchanged():
-    ref = "/root/reference/config"
-    if not os.path.isdir(ref):
-        pytest.skip("reference checkout not present (GPU box)")
+    """The reference's own full config files (SAPCU_REFERENCE names its checkout) load through our loaders."""
+    ref = os.path.join(os.environ.get("SAPCU_REFERENCE", ""), "config")
+    if not os.environ.get("SAPCU_REFERENCE") or not os.path.isdir(ref):
+        pytest.skip("SAPCU_REFERENCE does not name a checkout of the reference")
     from sapcu_b200.fn import config as fc
     from sapcu_b200.fd import config as dc
     assert fc.get_model(fc.load_config(ref + "/fn.yaml"))._cfg_ints() == [24, 18, 12, 640, 6, 8]

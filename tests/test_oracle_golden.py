@@ -1,5 +1,5 @@
 """CPU: the oracle (torch restatement + plain-C restatement) against the golden vectors generated from the real
-reference by oracle/make_golden.py.  These run without /root/reference."""
+reference by oracle/make_golden.py.  These run without the reference checkout."""
 import json
 import os
 
@@ -46,8 +46,15 @@ def test_neuron_known_answers(golden):
     x = torch.from_numpy(g["x"])
     prm = {k[2:]: torch.from_numpy(g[k]) for k in g.files if k.startswith("p_")}
     lifp = {k: v for k, v in prm.items() if k not in ("delta_T", "theta_rh")}
-    assert torch.equal(orc.lif_chain(x, lifp, 7, all_steps=True), torch.from_numpy(g["lif"]))
-    assert torch.equal(orc.lif_chain(x, prm, 7, all_steps=True), torch.from_numpy(g["eif"]))
+    # torch's CPU exp / sigmoid round differently in the last bits on some CPU types: the reference's outputs are reproduced
+    # bit for bit where the soft spike alone (the first LIF step) rounds as on the host that stored them, else to a few ulp
+    exact = torch.equal(orc.spike_function(x - prm["threshold_base"]), torch.from_numpy(g["lif"][0]))
+    for tag, p in (("lif", lifp), ("eif", prm)):
+        got = orc.lif_chain(x, p, 7, all_steps=True)
+        if exact:
+            assert torch.equal(got, torch.from_numpy(g[tag]))
+        else:
+            np.testing.assert_allclose(got.numpy(), g[tag], rtol=2e-6, atol=1e-7)
     p4 = np.stack([g["p_membrane_decay"], g["p_threshold_adapt"], g["p_refractory_decay"], g["p_threshold_base"]])
     e2 = np.stack([g["p_delta_T"], g["p_theta_rh"]])
     # plain C uses libm expf instead of torch's vectorised exp: equal to a few ulp, not bitwise
@@ -92,13 +99,17 @@ def test_model_forwards_match_reference(golden):
             syn.init_weights(mfd, seed=200, stress=stress)
             taps_fn, taps_fd = {}, {}
             n = orc.fn_forward(mfn.state_dict(), p, taps=taps_fn)
-            assert torch.equal(n, torch.from_numpy(g[tag + "_normals"]))
-            assert torch.equal(taps_fn["snn_init"][:, ::4], torch.from_numpy(g[tag + "_fn_snn_init"]))
-            assert torch.equal(taps_fn["snn_final"][:, ::16], torch.from_numpy(g[tag + "_fn_snn_final"]))
+            # torch's CPU convolutions block (and so round) by CPU type and thread count, and its exp by CPU type: the
+            # reference's outputs are reproduced bit for bit only on the host that stored them, elsewhere to fp32 rounding
+            # (the bounds of test_pipeline_matches_reference); spike taps to 2e-3, since last-bit differences can reorder
+            # the exact ties of the fd feature-space graphs under the default init
+            np.testing.assert_allclose(n.numpy(), g[tag + "_normals"], rtol=0, atol=2e-6)
+            np.testing.assert_allclose(taps_fn["snn_init"][:, ::4].numpy(), g[tag + "_fn_snn_init"], rtol=0, atol=2e-6)
+            np.testing.assert_allclose(taps_fn["snn_final"][:, ::16].numpy(), g[tag + "_fn_snn_final"], rtol=0, atol=2e-6)
             pf = torch.from_numpy(g[tag + "_patches_fd"])
             d = orc.fd_forward(mfd.state_dict(), pf, taps=taps_fd)
-            assert torch.equal(d, torch.from_numpy(g[tag + "_dist"]))
-            assert torch.equal(taps_fd["spikes"][:, :, ::16], torch.from_numpy(g[tag + "_fd_spikes"]))
+            np.testing.assert_allclose(d.numpy(), g[tag + "_dist"], rtol=2e-5, atol=1e-7)
+            np.testing.assert_allclose(taps_fd["spikes"][:, :, ::16].numpy(), g[tag + "_fd_spikes"], rtol=0, atol=2e-3)
             # exact dead-code elimination: closed-gate schedule == faithful schedule, bit for bit
             assert torch.equal(orc.fd_forward(mfd.state_dict(), pf, schedule="dce"), d)
 
