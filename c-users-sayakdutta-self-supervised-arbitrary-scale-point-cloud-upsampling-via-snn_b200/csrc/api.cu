@@ -30,24 +30,11 @@ static int env_int(const char* name, int dflt) { const char* e = getenv(name); r
 const Settings& settings() {
   static const Settings s = [] {
     Settings t;
-    t.tc_2cta = env_int("SAPCU_TC_2CTA", 1) != 0;
     t.fuse_attnout = env_int("SAPCU_TC_FUSE_ATTNOUT", 1) != 0;
     t.factor_attnin = env_int("SAPCU_TC_FACTOR_ATTNIN", 1) != 0;
     t.fuse_pool = env_int("SAPCU_TC_FUSE_POOL", 1) != 0;
-    t.fp16x3 = env_int("SAPCU_TC_FP16X3", 1) != 0;
-    t.spike_planes = env_int("SAPCU_TC_SPIKE_PLANES", 1) != 0;
     t.fast_tables = env_int("SAPCU_FAST_LIF_TABLES", 1) != 0;
-    t.tc_tables = env_int("SAPCU_TC_LIF_TABLES", 1) != 0;
-    t.tc_pos_copy = env_int("SAPCU_TC_POS_COPY", 1) != 0;
-    t.tc_qkv_planes = env_int("SAPCU_TC_QKV_PLANES", 1) != 0;
-    t.tc_pq_unit = env_int("SAPCU_TC_PQ_FP16X3", 1) != 0;
-    t.tc_fc1_table = env_int("SAPCU_TC_FC1_TABLE", 1) != 0;
     t.sync_check = env_int("SAPCU_TC_SYNC_CHECK", 0) != 0;
-    t.h2_planes = env_int("SAPCU_TC_H2_PLANES", 1);
-    t.l2pf = env_int("SAPCU_TC_L2PF", 4);
-    t.tc_bn = env_int("SAPCU_TC_BN", 256) == 128 ? 128 : 256;
-    t.tc_epi = env_int("SAPCU_TC_EPI", 16) == 8 ? 8 : 16;
-    t.tc_rawhi = env_int("SAPCU_TC_RAWHI", 1) != 0 ? 1 : 0;
     return t;
   }();
   return s;

@@ -58,11 +58,13 @@ static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; 
 
 constexpr int kNumSMs = 148;   // B200
 
-// Process-wide A/B switches (environment, DESIGN.md section 5), read ONCE under C++11 static-initialisation locking and
+// Process-wide switches (environment, DESIGN.md section 5), read ONCE under C++11 static-initialisation locking and
 // immutable afterwards: concurrent forwards from several threads / streams all see the same values.
+//   fuse_attnout, factor_attnin, fuse_pool  the unfused tensor-core schedule, reference of the fused-epilogue tests
+//   fast_tables                             the fast mode's 2-MUFU recurrence instead of the LIF tables
+//   sync_check                              every forward synchronises its stream before checking the watchdog flag
 struct Settings {
-  bool tc_2cta, fuse_attnout, factor_attnin, fuse_pool, fp16x3, spike_planes, fast_tables, tc_tables, tc_pos_copy, tc_qkv_planes, tc_pq_unit, tc_fc1_table, sync_check;
-  int h2_planes, l2pf, tc_bn, tc_epi, tc_rawhi;
+  bool fuse_attnout, factor_attnin, fuse_pool, fast_tables, sync_check;
 };
 const Settings& settings();
 

@@ -204,12 +204,6 @@ int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
   };
   const bool factorise = settings().factor_attnin;
   const bool use_tables = settings().fast_tables;       // 0: reduced-MUFU chains (A/B)
-  // fp16-plane hand-overs: 0 off; 1 (default) pos-enc layer 1 -> fc_delta2 and fc_gamma -> fc_gamma2; 2 / 3 only the first /
-  // second; 4 only pos (fc_delta2 -> fc_gamma + attention tail); 5 all three.  The pos planes are measured slower (the
-  // attention tail then issues two 2-byte loads per operand instead of one 4-byte load) and stay off.
-  const int h2_env = settings().h2_planes;
-  const bool h2_delta_env = h2_env == 1 || h2_env == 2 || h2_env == 5, h2_gamma_env = h2_env == 1 || h2_env == 3 || h2_env == 5,
-             h2_pos_env = h2_env == 4 || h2_env == 5;
   for (int b = 0; b < 3; ++b) {
     if (stop_block && b >= stop_block) return 0;            // debug: leave block `stop_block`'s intermediates in the workspace
     const FnBlock& k = f.blk[b];
@@ -226,17 +220,17 @@ int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
       GemmArgs a1 = g.args(k.fc1, fin, ldin, P, p.X, D, ACT_LIF, &k.snn1, 4);
       GemmArgs a2 = g.args(k.qkv, p.X, D, P, p.QKV, 3 * D, ACT_LIF, &k.snn_qkv, 4);
       bool x_planes = false;
-      if (mode == SAPCU_MODE_TC && settings().tc_qkv_planes) {
+      if (mode == SAPCU_MODE_TC) {
         GemmArgs t1 = a1, t2 = a2;
         t1.out_h2 = true; t2.x_h2 = true; t2.x_unit = true; t1.tc2_any_rows = t2.tc2_any_rows = true;
         x_planes = D % 256 == 0 && gemm_tc2_supported(t1, A_PLAIN) && gemm_tc2_supported(t2, A_PLAIN) && gemm_tc2_fp16x3(t2);
         if (x_planes) {
           a1 = t1; a2 = t2;
-          if (settings().tc_tables && k.snn_qkv.tab_ok && k.snn_qkv.tab_T == 4 && k.snn_qkv.tab_stride <= LT_SMEM_BUDGET_TC) {
+          if (k.snn_qkv.tab_ok && k.snn_qkv.tab_T == 4 && k.snn_qkv.tab_stride <= LT_SMEM_BUDGET_TC) {
             a2.lif_tab = k.snn_qkv.tab; a2.lif_tab_stride = k.snn_qkv.tab_stride;
           }
           // fc1 itself keeps 3xTF32 products (its input is not a spike tensor) and reads its chain from the table as well
-          if (settings().tc_tables && settings().tc_fc1_table && k.snn1.tab_ok && k.snn1.tab_T == 4 && k.snn1.tab_stride <= LT_SMEM_BUDGET_TC) {
+          if (k.snn1.tab_ok && k.snn1.tab_T == 4 && k.snn1.tab_stride <= LT_SMEM_BUDGET_TC) {
             a1.lif_tab = k.snn1.tab; a1.lif_tab_stride = k.snn1.tab_stride;
           }
         }
@@ -287,13 +281,13 @@ int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
         continue;
       }
     }
-    // Parity-grade mode with tabulated LIF^T chains (SAPCU_TC_LIF_TABLES, default on): the three per-edge LIF layers of a block
-    // whose tables fit next to two pipeline stages read their chains from the tables (lif_table.cuh, |error| <= 4e-5, far
-    // inside the spike tolerance); all three edge tensors are then handed over as fp16 (hi, lo) planes.
-    const bool blk_tab = mode == SAPCU_MODE_TC && settings().tc_tables && factorise && kk >= 2 &&
+    // Parity-grade mode with tabulated LIF^T chains: the three per-edge LIF layers of a block whose tables fit next to two
+    // pipeline stages read their chains from the tables (lif_table.cuh, |error| <= 4e-5, far inside the spike tolerance); all
+    // three edge tensors are then handed over as fp16 (hi, lo) planes.  Without the tables pos stays fp32 (measured slower as
+    // planes: the attention tail then issues two 2-byte loads per operand instead of one 4-byte load).
+    const bool blk_tab = mode == SAPCU_MODE_TC && factorise && kk >= 2 &&
                          k.snn_delta.tab_ok && k.snn_delta2.tab_ok && k.snn_gamma.tab_ok && k.snn_delta.tab_stride <= LT_SMEM_BUDGET &&
                          k.snn_delta2.tab_stride <= LT_SMEM_BUDGET_TC && k.snn_gamma.tab_stride <= LT_SMEM_BUDGET_TC;
-    const bool h2_delta = blk_tab || h2_delta_env, h2_gamma = blk_tab || h2_gamma_env, h2_pos = blk_tab || h2_pos_env;
     if (mode != SAPCU_MODE_FP32) {
       // fc_delta2 on the pos-enc layer-1 spikes.  When it runs on the fp16x3 path, edge_pos_lif hands the spikes over as
       // fp16 (hi, lo) planes of x * 2^13 (same bytes as fp32) and the contraction loads them without converting.
@@ -305,12 +299,12 @@ int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
         a.Y = p.E2; a.ldc = D; a.Wh = L.Wh; a.Wl = L.Wl; a.winv = L.winv; a.x_unit = true;   // input: LIF output
         a.tc_passes = (mode == SAPCU_MODE_TF32 || mode == SAPCU_MODE_FAST) ? 1 : 3;
         a.x_h2 = true;                                              // tentatively: 128-channel layers run on the 2-CTA engine only from planes
-        a.x_h2 = h2_delta && gemm_tc2_supported(a, A_PLAIN) && gemm_tc2_fp16x3(a);
+        a.x_h2 = gemm_tc2_supported(a, A_PLAIN) && gemm_tc2_fp16x3(a);
         {   // pos (E2) has two readers, fc_gamma's contraction and the fused attention tail: planes when both take them
           GemmArgs a1 = gamma_args(b, p.E2, Xb, p.QK), a2 = gamma2_args(b, Xb, p.E2);
           a1.tc_passes = a2.tc_passes = a.tc_passes;
           a1.x_h2 = a2.x_h2 = a2.pos_h2 = true;                    // the formats this hand-over would give them
-          e2_h2 = h2_pos && a.x_h2 && factorise && kk >= 2 && gemm_tc2_supported(a, A_PLAIN) && gemm_tc2_supported(a1, A_PLAIN) &&
+          e2_h2 = blk_tab && a.x_h2 && factorise && kk >= 2 && gemm_tc2_supported(a, A_PLAIN) && gemm_tc2_supported(a1, A_PLAIN) &&
                   gemm_tc2_fp16x3(a1) && gemm_tc2_supported(a2, A_PLAIN) && gemm_tc2_fp16x3(a2);
         }
         a.out_h2 = e2_h2;
@@ -318,7 +312,7 @@ int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
         const bool tab_on = blk_tab && a.x_h2 && e2_h2;           // the whole chain of plane hand-overs is in place
         // pos has two readers: fc_gamma's contraction takes the planes, the attention tail gathers it per edge and prefers one
         // 4-byte load over two 2-byte loads -- with the table-driven (ALU-bound) epilogue the extra fp32 store is free
-        pos32 = tab_on && settings().tc_pos_copy;
+        pos32 = tab_on;
         if (pos32) a.Y2 = p.E3;
         if (tab_on) {
           ProfWork w; w.elsteps = (double)E * D * 4; w.bytes = (double)E * D * 4.0;
@@ -339,7 +333,7 @@ int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
           GemmArgs a2 = gamma2_args(b, Xb, p.E2);
           a2.x_h2 = true; a2.pos_h2 = e2_h2;
           GemmArgs at = a; at.x_h2 = e2_h2;
-          xb_h2 = h2_gamma && factorise && kk >= 2 && gemm_tc2_supported(at, A_PLAIN) && gemm_tc2_supported(a2, A_PLAIN) && gemm_tc2_fp16x3(a2);
+          xb_h2 = factorise && kk >= 2 && gemm_tc2_supported(at, A_PLAIN) && gemm_tc2_supported(a2, A_PLAIN) && gemm_tc2_fp16x3(a2);
         }
         a.out_h2 = xb_h2; a.x_h2 = e2_h2;
         g_tap_gamma_h2 = xb_h2 ? 1 : 0;
@@ -428,14 +422,13 @@ int fd_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
     c5.Wh = L.Wh; c5.Wl = L.Wl; c5.winv = L.winv; c5.x_unit = true;                   // the spike tensor
     c5.tc_passes = (mode == SAPCU_MODE_TF32 || mode == SAPCU_MODE_FAST) ? 1 : 3;
   }
-  const bool fuse_pool = settings().fuse_pool, spk_planes = settings().spike_planes;
-  const bool pooled = mode != SAPCU_MODE_FP32 && fuse_pool && gemm_tc2_supported(c5, A_PLAIN);
+  const bool pooled = mode != SAPCU_MODE_FP32 && settings().fuse_pool && gemm_tc2_supported(c5, A_PLAIN);
   // When conv5 runs on the fp16x3 path the spike tensor is stored as fp16 (hi, lo) planes of s * 2^13 (rows = point*T + t)
   // that it loads without converting; the step-0 spikes, which the graphs and EdgeConvs of the next block read, are
   // also kept in fp32 (SPK0, [P, 960]).
   bool spk_fast = false;
-  if (mode == SAPCU_MODE_FAST && pooled && spk_planes) { c5.fast = true; c5.x_h2 = true; spk_fast = gemm_tc2_fast(c5); c5.fast = spk_fast; c5.x_h2 = false; }
-  const bool spk_h2 = pooled && spk_planes && (spk_fast || gemm_tc2_fp16x3(c5));
+  if (mode == SAPCU_MODE_FAST && pooled) { c5.fast = true; c5.x_h2 = true; spk_fast = gemm_tc2_fast(c5); c5.fast = spk_fast; c5.x_h2 = false; }
+  const bool spk_h2 = pooled && (spk_fast || gemm_tc2_fp16x3(c5));
   g_tap_spk_h2 = spk_fast ? 2 : (spk_h2 ? 1 : 0);
   const int64_t plane = spk_fast ? 0 : P * T * 960;         // fast mode: hi plane only
   const float* S0 = spk_h2 ? p.SPK0 : p.SPK;                     // step-0 spikes: row stride ld0
@@ -459,7 +452,7 @@ int fd_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
         // the input is a slice of the step-0 spike tensor: parity-grade mode -> fp16x3 products (the splitter converts the fp32
         // rows), on the 2-CTA engine from 1,024 rows on so that the arithmetic does not depend on the chunking
         GemmArgs a = g.args(L, S0 + off_in[b], ld0, P, p.PQ, 2 * cout[b], ACT_NONE);
-        if (mode == SAPCU_MODE_TC && settings().tc_pq_unit) {
+        if (mode == SAPCU_MODE_TC) {
           GemmArgs t = a; t.x_unit = true; t.tc2_any_rows = true;
           if (gemm_tc2_supported(t, A_PLAIN) && gemm_tc2_fp16x3(t)) a = t;
         }

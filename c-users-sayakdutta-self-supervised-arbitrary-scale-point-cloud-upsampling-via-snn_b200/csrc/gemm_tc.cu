@@ -12,17 +12,16 @@
 // register-resident accumulators, a max over 32 consecutive rows (EdgeConv k = 32) is thread-local, and
 // the 32 lanes of a warp store 32 consecutive channels of one row (one 128-byte line).
 //
-// Persistent, warp-specialised CTA (1 per SM, 640 threads with the default 16 epilogue warps):
+// Persistent, warp-specialised CTA (1 per SM, 640 threads):
 //   warp 0        TMA producer   cp.async.bulk.tensor of the pre-split tf32 W hi/lo tiles and the raw fp32 X tile
 //                                (128B swizzle) + cp.async.bulk.prefetch.tensor L2 look-ahead for X
 //   warp 1        MMA issuer     tcgen05.mma.kind::tf32 (12 per 32-wide k-block), tcgen05.commit; owns TMEM alloc
 //   warps 2..3    splitter       lo = x - trunc_tf32(x) into the second buffer (the raw tile is the hi operand: the
 //                                tensor core ignores the low 13 mantissa bits)
 //   warps 4..19   epilogue       tcgen05.ld -> bias / BN / activation / LIF^T / fused tails -> 128-byte row stores
-// Pipelines: smem ring of 2 stages x 96 KiB at BN = 256 (3 x 64 KiB at BN = 128; mbarriers raw-full / split-full /
-// empty) and 512 / BN TMEM accumulator buffers (mbarriers tmem-full / tmem-empty) so the epilogue of tile i overlaps
-// the MMAs of tile i+1.  Every mbarrier wait carries a clock64() watchdog: a protocol error surfaces as an error
-// code, never as a hung GPU.
+// Pipelines: smem ring of 2 stages x 96 KiB (mbarriers raw-full / split-full / empty) and 2 TMEM accumulator buffers of
+// 256 columns (mbarriers tmem-full / tmem-empty) so the epilogue of tile i overlaps the MMAs of tile i+1.  Every mbarrier
+// wait carries a clock64() watchdog: a protocol error surfaces as an error code, never as a hung GPU.
 //
 // Epilogue flavours (template EXTRA): 0 plain, 1 + residual, 2 edge bias W q_i - W k_j added before BN + LIF (factorised
 // attention input), 3 fused attention tail (softmax over the KK edges of a point and the weighted sum; tc_ptx.cuh).
@@ -39,25 +38,21 @@
 
 namespace sapcu {
 
-// BN = activation rows per tile (UMMA N) is a template parameter: 128 (3 smem stages, 4 TMEM accumulators)
-// or 256 (2 stages, 2 accumulators; 25 % fewer operand bytes per FLOP)
-#ifndef SAPCU_TC_SPLIT_WARPS
-#define SAPCU_TC_SPLIT_WARPS 2     // 2 + 2 + 16 warps = 640 threads: 96 registers per thread for the epilogue
-#endif
-constexpr int TC_SPLIT_WARP0 = 2, TC_SPLIT_WARPS = SAPCU_TC_SPLIT_WARPS;
-constexpr int TC_EPI_WARP0 = TC_SPLIT_WARP0 + TC_SPLIT_WARPS;                                // epilogue warps: 8 or 16 (template parameter EPI)
-constexpr size_t TC_SMEM_BYTES = (size_t)3 * 4 * TC_TILE_BYTES + 1024 /*align slack*/ + 256 /*barriers*/;   // same for both BN
+constexpr int TC_BN = 256;                      // activation rows per tile (UMMA N)
+constexpr int TC_STAGES = 2, TC_ACC = 2;        // smem stages, TMEM accumulators of TC_BN columns
+constexpr int TC_SPLIT_WARP0 = 2, TC_SPLIT_WARPS = 2;
+constexpr int TC_EPI_WARP0 = TC_SPLIT_WARP0 + TC_SPLIT_WARPS, TC_EPI = 16;   // 2 + 2 + 16 warps = 640 threads: 96 registers per thread for the epilogue
+constexpr int TC_THREADS = (TC_EPI_WARP0 + TC_EPI) * 32;
+constexpr uint32_t TC_X_BYTES = TC_BN * TC_BK * 4;
+constexpr uint32_t TC_STAGE_BYTES = 2 * TC_TILE_BYTES + 2 * TC_X_BYTES;       // W_hi, W_lo, X_hi, X_lo
+constexpr size_t TC_SMEM_BYTES = (size_t)TC_STAGES * TC_STAGE_BYTES + 1024 /*align slack*/ + 256 /*barriers*/;
 
 
 // ------------------------------------------------------------------------------------------------ kernel
-template <int ACT, int EXTRA, int EPI, int TC_BN, int KK = 1>
-__global__ void __launch_bounds__((TC_EPI_WARP0 + EPI) * 32, 1)
+template <int ACT, int EXTRA, int KK = 1>
+__global__ void __launch_bounds__(TC_THREADS, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUtensorMap map_wlo,
                const __grid_constant__ CUtensorMap map_x, const TcParams p) {
-  constexpr int TC_STAGES = (TC_BN == 128) ? 3 : 2;
-  constexpr int TC_ACC = 512 / TC_BN;
-  constexpr uint32_t X_BYTES = TC_BN * TC_BK * 4;
-  constexpr uint32_t TC_STAGE_BYTES = 2 * TC_TILE_BYTES + 2 * X_BYTES;       // W_hi, W_lo, X_hi, X_lo
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;            // 128B swizzle needs 1024 B alignment
   uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
@@ -79,7 +74,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < TC_STAGES; ++s) { mbar_init(bar_raw(s), 1); mbar_init(bar_split(s), TC_SPLIT_WARPS * 32); mbar_init(bar_empty(s), 1); }
-    for (int a = 0; a < TC_ACC; ++a) { mbar_init(bar_tfull(a), 1); mbar_init(bar_tempty(a), EPI); }
+    for (int a = 0; a < TC_ACC; ++a) { mbar_init(bar_tfull(a), 1); mbar_init(bar_tempty(a), TC_EPI); }
     fence_barrier_init();
     tma_prefetch_desc(&map_w);
     tma_prefetch_desc(&map_wlo);
@@ -102,15 +97,13 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
         const int m_t = (int)(t % p.m_tiles);
         const int64_t n_t = t / p.m_tiles;
         for (int kb = 0; kb < nk; ++kb) {
-          if (p.l2_prefetch > 0) {
-            // pull the activation tile `l2_prefetch` k-blocks ahead (possibly in this CTA's next tile) into L2
-            int kp = kb + p.l2_prefetch; int64_t tp = t;
-            if (kp >= nk) { kp -= nk; tp += gridDim.x; }
-            if (kp < nk && tp < total_tiles) tma_prefetch_l2_2d(&map_x, kp * TC_BK, (int)((tp / p.m_tiles) * TR));
-          }
+          // pull the activation tile TC_L2_PREFETCH k-blocks ahead (possibly in this CTA's next tile) into L2
+          int kp = kb + TC_L2_PREFETCH; int64_t tp = t;
+          if (kp >= nk) { kp -= nk; tp += gridDim.x; }
+          if (kp < nk && tp < total_tiles) tma_prefetch_l2_2d(&map_x, kp * TC_BK, (int)((tp / p.m_tiles) * TR));
           if (!(ok = mbar_wait(bar_empty(s), ph ^ 1u, p.err))) break;
           const uint32_t st = smem_base + s * TC_STAGE_BYTES;
-          mbar_expect_tx(bar_raw(s), ((p.split_w || p.passes == 1) ? 1 : 2) * TC_TILE_BYTES + X_BYTES);
+          mbar_expect_tx(bar_raw(s), ((p.split_w || p.passes == 1) ? 1 : 2) * TC_TILE_BYTES + TC_X_BYTES);
           tma_load_2d(st, &map_w, bar_raw(s), kb * TC_BK, m_t * TC_BM);
           if (!p.split_w && p.passes == 3) tma_load_2d(st + TC_TILE_BYTES, &map_wlo, bar_raw(s), kb * TC_BK, m_t * TC_BM);
           tma_load_2d(st + 2 * TC_TILE_BYTES, &map_x, bar_raw(s), kb * TC_BK, (int)(n_t * TR));
@@ -131,7 +124,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
           tc_fence_after();
           const uint32_t st = smem_base + s * TC_STAGE_BYTES;
           const uint64_t w_hi = umma_desc_sw128(st), w_lo = umma_desc_sw128(st + TC_TILE_BYTES);
-          const uint64_t x_hi = umma_desc_sw128(st + 2 * TC_TILE_BYTES), x_lo = umma_desc_sw128(st + 2 * TC_TILE_BYTES + X_BYTES);
+          const uint64_t x_hi = umma_desc_sw128(st + 2 * TC_TILE_BYTES), x_lo = umma_desc_sw128(st + 2 * TC_TILE_BYTES + TC_X_BYTES);
 #pragma unroll
           for (int k8 = 0; k8 < TC_BK / 8; ++k8) {
             const uint64_t adv = (uint64_t)(k8 * 2);            // 8 tf32 = 32 B = 2 x 16 B along the swizzled row
@@ -162,34 +155,20 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
         for (int op = 0; op < 2; ++op) {                          // 0: W tile (only when it arrives raw), 1: X tile
           if (p.passes == 1) continue;                            // single-pass TF32: the raw tiles are the operands
           if (op == 0 && !p.split_w) continue;
-          const uint32_t bytes = op ? X_BYTES : TC_TILE_BYTES;
+          const uint32_t bytes = op ? TC_X_BYTES : TC_TILE_BYTES;
           float4* hi = reinterpret_cast<float4*>(st + op * 2 * TC_TILE_BYTES);
           float4* lo = reinterpret_cast<float4*>(st + op * 2 * TC_TILE_BYTES + bytes);
           const int iters = (int)(bytes / 16) / (TC_SPLIT_WARPS * 32);
-          if (p.raw_hi) {
 #pragma unroll
-            for (int i = 0; i < iters; ++i) {
-              const int e = tid + i * TC_SPLIT_WARPS * 32;
-              const float4 v = hi[e];
-              float4 l;
-              l.x = v.x - __uint_as_float(__float_as_uint(v.x) & 0xFFFFE000u);
-              l.y = v.y - __uint_as_float(__float_as_uint(v.y) & 0xFFFFE000u);
-              l.z = v.z - __uint_as_float(__float_as_uint(v.z) & 0xFFFFE000u);
-              l.w = v.w - __uint_as_float(__float_as_uint(v.w) & 0xFFFFE000u);
-              lo[e] = l;
-            }
-          } else {
-#pragma unroll
-            for (int i = 0; i < iters; ++i) {
-              const int e = tid + i * TC_SPLIT_WARPS * 32;
-              const float4 v = hi[e];
-              float4 h, l;
-              h.x = tf32_rna(v.x); l.x = v.x - h.x;
-              h.y = tf32_rna(v.y); l.y = v.y - h.y;
-              h.z = tf32_rna(v.z); l.z = v.z - h.z;
-              h.w = tf32_rna(v.w); l.w = v.w - h.w;
-              hi[e] = h; lo[e] = l;
-            }
+          for (int i = 0; i < iters; ++i) {
+            const int e = tid + i * TC_SPLIT_WARPS * 32;
+            const float4 v = hi[e];
+            float4 l;
+            l.x = v.x - __uint_as_float(__float_as_uint(v.x) & 0xFFFFE000u);
+            l.y = v.y - __uint_as_float(__float_as_uint(v.y) & 0xFFFFE000u);
+            l.z = v.z - __uint_as_float(__float_as_uint(v.z) & 0xFFFFE000u);
+            l.w = v.w - __uint_as_float(__float_as_uint(v.w) & 0xFFFFE000u);
+            lo[e] = l;
           }
         }
         fence_proxy_async();                                      // generic-proxy writes -> visible to the tensor core
@@ -200,7 +179,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
   } else {
     // ======================================================================== epilogue
     const int q = warp & 3;                                       // TMEM lane quarter this warp may access
-    constexpr int CHUNKS = (TC_BN / 32) / (EPI / 4);              // 32-column chunks per warp
+    constexpr int CHUNKS = (TC_BN / 32) / (TC_EPI / 4);              // 32-column chunks per warp
     const int part = (warp - TC_EPI_WARP0) >> 2;                  // which slice of the 128-column tile
     int a = 0; uint32_t aph = 0; bool ok = true;
     for (int64_t t = blockIdx.x; t < total_tiles && ok; t += gridDim.x) {
@@ -220,13 +199,13 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
         // fused attention tail (see gemm_tc2.cu): the tile holds TR / KK whole points; a warp takes every `parts`-th
         // point, one channel per lane: logits -> softmax over the KK edges -> sum_j a_j (v[nb_j] + pos[e_j])
         const int npts = TR / KK;
-        constexpr int parts = EPI / 4;
+        constexpr int parts = TC_EPI / 4;
         {   // pull the pos rows of this CTA's NEXT tile (its 128-channel slab: 4 lines per row) into L2
           const int64_t tn = t + gridDim.x;
           if (tn < total_tiles) {
             const int64_t row0 = (tn / p.m_tiles) * TR;
             const int cb = (int)(tn % p.m_tiles) * TC_BM;
-            for (int i = (warp - TC_EPI_WARP0) * 32 + lane; i < TR * 4; i += EPI * 32) {
+            for (int i = (warp - TC_EPI_WARP0) * 32 + lane; i < TR * 4; i += TC_EPI * 32) {
               const int64_t row = row0 + (i >> 2);
               if (row < p.R) prefetch_l2(p.at_pos + row * p.N + cb + (i & 3) * 32);
             }
@@ -427,32 +406,16 @@ bool gemm_tc_supported(const GemmArgs& g, int amode) {
 
 int launch_gemm_tc(const GemmArgs& g, int amode, cudaStream_t st) {
   SAPCU_REQUIRE(gemm_tc_supported(g, amode), "gemm_tc: unsupported problem");
-  static PerDeviceOnce once;
-  {
-    const int rc_attr = once.run([]() -> int {
-#define SAPCU_TC_ATTR1(A, RS, E, B) SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc_kernel<A, RS, E, B>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES))
-#define SAPCU_TC_ATTR(A, RS) SAPCU_TC_ATTR1(A, RS, 8, 128); SAPCU_TC_ATTR1(A, RS, 8, 256); SAPCU_TC_ATTR1(A, RS, 16, 128); SAPCU_TC_ATTR1(A, RS, 16, 256)
-    SAPCU_TC_ATTR(ACT_LIF, 0); SAPCU_TC_ATTR(ACT_LIF, 2); SAPCU_TC_ATTR(ACT_LEAKY, 0); SAPCU_TC_ATTR(ACT_GELU, 0); SAPCU_TC_ATTR(ACT_NONE, 1); SAPCU_TC_ATTR(ACT_NONE, 0);
-    SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc_kernel<ACT_NONE, 3, 16, 256, 12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES));
-    SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc_kernel<ACT_NONE, 3, 16, 256, 18>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES));
-    SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc_kernel<ACT_NONE, 3, 16, 256, 24>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES));
-#undef SAPCU_TC_ATTR
-#undef SAPCU_TC_ATTR1
-      return 0;
-    });
-    if (rc_attr) return rc_attr;
-  }
   int* err = tc_err_flag();
   SAPCU_REQUIRE(err != nullptr, "gemm_tc: cannot allocate the watchdog flag");
-  const int epi_warps = settings().tc_epi, raw_hi = settings().tc_rawhi, bn = settings().tc_bn, l2pf = settings().l2pf;
   const bool presplit = g.Whi != nullptr && g.Wlo != nullptr;
   CUtensorMap mw, mwlo, mx;
   int rc = tc_make_map(&mw, presplit ? g.Whi : g.W, g.N, g.K, g.K, TC_BM);
   if (rc) return rc;
   rc = tc_make_map(&mwlo, presplit ? g.Wlo : g.W, g.N, g.K, g.K, TC_BM);
   if (rc) return rc;
-  const int tile_rows = g.at_pos ? tc_fused_tile_rows(g.kk) : bn;     // the fused attention tail runs the 256-column layout
-  rc = tc_make_map(&mx, g.A, g.R, g.K, g.lda, g.at_pos ? 256 : bn);
+  const int tile_rows = g.at_pos ? tc_fused_tile_rows(g.kk) : TC_BN;
+  rc = tc_make_map(&mx, g.A, g.R, g.K, g.lda, TC_BN);
   if (rc) return rc;
   TcParams p;
   p.R = g.R; p.N = g.N; p.K = g.K; p.bias = g.bias; p.scale = g.scale; p.shift = g.shift; p.act = g.act; p.T = g.T;
@@ -461,32 +424,17 @@ int launch_gemm_tc(const GemmArgs& g, int amode, cudaStream_t st) {
   p.m_tiles = (int)ceil_div(g.N, TC_BM); p.n_tiles = ceil_div(g.R, tile_rows); p.err = err;
   p.pool = nullptr; p.pool_T = 0; p.pool_rows = 0; p.acc_scale = 1.0f; p.x_scale = 1.0f; p.out_h2 = 0; p.pos_h2 = 0;
   p.Y2 = nullptr; p.idx8 = g.idx8; p.ldi8w = g.ldi8w; p.at_pos = g.at_pos; p.at_v = g.at_v; p.at_ldv = g.at_ldv; p.at_sqrt = g.at_sqrt; p.tile_rows = tile_rows;
-  p.split_w = presplit ? 0 : 1; p.raw_hi = raw_hi; p.l2_prefetch = l2pf; p.passes = g.tc_passes == 1 ? 1 : 3;
+  p.split_w = presplit ? 0 : 1; p.passes = g.tc_passes == 1 ? 1 : 3;
   const int64_t total = p.n_tiles * p.m_tiles;
   const int grid = (int)(total < kNumSMs ? total : kNumSMs);
-#define SAPCU_TC_LAUNCH1(A, RS, E, B) gemm_tc_kernel<A, RS, E, B><<<grid, (TC_EPI_WARP0 + E) * 32, TC_SMEM_BYTES, st>>>(mw, mwlo, mx, p)
-#define SAPCU_TC_LAUNCH(A, RS)                                                  \
-  do {                                                                          \
-    if (epi_warps == 8 && bn == 128) SAPCU_TC_LAUNCH1(A, RS, 8, 128);            \
-    else if (epi_warps == 8) SAPCU_TC_LAUNCH1(A, RS, 8, 256);                    \
-    else if (bn == 128) SAPCU_TC_LAUNCH1(A, RS, 16, 128);                        \
-    else SAPCU_TC_LAUNCH1(A, RS, 16, 256);                                       \
-  } while (0)
-  if (g.at_pos) {
-#define SAPCU_TC_LAUNCH3(KQ) gemm_tc_kernel<ACT_NONE, 3, 16, 256, KQ><<<grid, (TC_EPI_WARP0 + 16) * 32, TC_SMEM_BYTES, st>>>(mw, mwlo, mx, p)
-    if (g.kk == 12) SAPCU_TC_LAUNCH3(12); else if (g.kk == 18) SAPCU_TC_LAUNCH3(18); else SAPCU_TC_LAUNCH3(24);
-#undef SAPCU_TC_LAUNCH3
-  }
-  else if (g.act == ACT_LIF && g.edge_bias) SAPCU_TC_LAUNCH(ACT_LIF, 2);
-  else if (g.act == ACT_LIF) SAPCU_TC_LAUNCH(ACT_LIF, 0);
-  else if (g.act == ACT_LEAKY) SAPCU_TC_LAUNCH(ACT_LEAKY, 0);
-  else if (g.act == ACT_GELU) SAPCU_TC_LAUNCH(ACT_GELU, 0);
-  else if (g.residual) SAPCU_TC_LAUNCH(ACT_NONE, 1);
-  else SAPCU_TC_LAUNCH(ACT_NONE, 0);
-#undef SAPCU_TC_LAUNCH
-#undef SAPCU_TC_LAUNCH1
-  SAPCU_LAUNCH_CHECK();
-  return 0;
+  if (g.at_pos)
+    return with_kk(g.kk, [&](auto KQ) { return tc_launch<gemm_tc_kernel<ACT_NONE, 3, decltype(KQ)::value>>(grid, TC_THREADS, TC_SMEM_BYTES, st, mw, mwlo, mx, p); });
+  if (g.act == ACT_LIF && g.edge_bias) return tc_launch<gemm_tc_kernel<ACT_LIF, 2>>(grid, TC_THREADS, TC_SMEM_BYTES, st, mw, mwlo, mx, p);
+  if (g.act == ACT_LIF) return tc_launch<gemm_tc_kernel<ACT_LIF, 0>>(grid, TC_THREADS, TC_SMEM_BYTES, st, mw, mwlo, mx, p);
+  if (g.act == ACT_LEAKY) return tc_launch<gemm_tc_kernel<ACT_LEAKY, 0>>(grid, TC_THREADS, TC_SMEM_BYTES, st, mw, mwlo, mx, p);
+  if (g.act == ACT_GELU) return tc_launch<gemm_tc_kernel<ACT_GELU, 0>>(grid, TC_THREADS, TC_SMEM_BYTES, st, mw, mwlo, mx, p);
+  if (g.residual) return tc_launch<gemm_tc_kernel<ACT_NONE, 1>>(grid, TC_THREADS, TC_SMEM_BYTES, st, mw, mwlo, mx, p);
+  return tc_launch<gemm_tc_kernel<ACT_NONE, 0>>(grid, TC_THREADS, TC_SMEM_BYTES, st, mw, mwlo, mx, p);
 }
 
 // Watchdog status of the current device (0 = fine).  The flag is host-visible, so this never touches a stream unless

@@ -44,14 +44,10 @@ namespace sapcu {
 constexpr int T2_STAGES_MAX = 3;
 constexpr int T2_ACC = 2;                       // 2 x 256 TMEM columns
 constexpr int T2_BN = 256;                      // rows per pair tile (128 staged by each CTA)
-#ifndef SAPCU_T2_SPLIT_WARPS
-#define SAPCU_T2_SPLIT_WARPS 2     // 2 + 2 + 16 warps = 640 threads: 96 registers per thread for the epilogue
-#endif
-constexpr int T2_SPLIT_WARP0 = 2, T2_SPLIT_WARPS = SAPCU_T2_SPLIT_WARPS;
-constexpr int T2_EPI_WARP0 = T2_SPLIT_WARP0 + T2_SPLIT_WARPS, T2_EPI = 16;
-#ifndef SAPCU_T2_FAST_STAGES
-#define SAPCU_T2_FAST_STAGES 4     // pair flavour on compact (32 KiB) stages without a LIF table: stages in flight
-#endif
+constexpr int T2_SPLIT_WARP0 = 2, T2_SPLIT_WARPS = 2;
+constexpr int T2_EPI_WARP0 = T2_SPLIT_WARP0 + T2_SPLIT_WARPS, T2_EPI = 16;   // 2 + 2 + 16 warps = 640 threads: 96 registers per thread for the epilogue
+constexpr int T2_THREADS = (T2_EPI_WARP0 + T2_EPI) * 32;
+constexpr int T2_FAST_STAGES = 4;               // pair flavour on compact (32 KiB) stages without a LIF table: stages in flight
 constexpr size_t T2_SMEM_BYTES = (size_t)T2_STAGES_MAX * 4 * TC_TILE_BYTES + 1024 + 256;   // 3 x 64 KiB (tf32) = 2 x 96 KiB (fp16x3)
 
 __device__ __forceinline__ uint32_t cluster_ctarank() {
@@ -189,7 +185,7 @@ __device__ __forceinline__ void lif_store_piece(const TcParams& p, const float (
 // channels x 256 rows per tile, cta_group::1 MMAs, no cluster): the 128-channel layers of the first fn block in the fast
 // mode, which then share the single-plane operands, the LIF tables and the fused attention tail with the wide layers.
 template <int ACT, int EXTRA, int KK, int HM = 0, int LT = 0, int CG = 2>
-__global__ void __cluster_dims__(CG, 1, 1) __launch_bounds__((T2_EPI_WARP0 + T2_EPI) * 32, 1)
+__global__ void __cluster_dims__(CG, 1, 1) __launch_bounds__(T2_THREADS, 1)
 gemm_tc2_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUtensorMap map_wlo,
                 const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_x2, const TcParams p) {
   // HM: 0 = 3xTF32; 1 = fp16x3, raw fp32 activations converted by the splitter warps; 2 = fp16x3, activations already
@@ -200,7 +196,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant
   constexpr int CW = CG * 128;                               // output channels per tile
   constexpr bool FASTOP = HM == 3 || HM == 4;               // compact stages: one weight tile + one activation tile
   // stages: HM 2 (two fp16 planes per operand, 64 KiB per stage for a pair, 96 KiB single-CTA): 3 / 2 plain, 2 / 1 next to a LIF table
-  constexpr int T2_STAGES = HM == 1 ? 2 : (FASTOP && !LT) ? (CG == 2 ? SAPCU_T2_FAST_STAGES : 4) : (FASTOP && CG == 1) ? 2 : FASTOP ? 3 : (CG == 2 ? (LT ? 2 : 3) : (LT ? 1 : 2));
+  constexpr int T2_STAGES = HM == 1 ? 2 : (FASTOP && !LT) ? (CG == 2 ? T2_FAST_STAGES : 4) : (FASTOP && CG == 1) ? 2 : FASTOP ? 3 : (CG == 2 ? (LT ? 2 : 3) : (LT ? 1 : 2));
   constexpr uint32_t T2_STAGE_BYTES = (HM == 1 ? 6 : FASTOP ? (CG == 2 ? 2 : 3) : (CG == 2 ? 4 : 6)) * TC_TILE_BYTES;   // HM 3/4: W tile + 128 (pair) or 256 activation rows
   constexpr uint32_t X_TILE = FASTOP ? 1 : 2;               // position of the activation (hi) tile inside a stage
   constexpr uint32_t X_LO_OFF = (CG == 2 ? 3 : 4) * TC_TILE_BYTES;   // lo activation tile (HM 0..2): behind the hi tile of 128 / 256 rows
@@ -262,20 +258,18 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant
       const int wrow = m_t * CW + (int)rank * 128;
       const int xrow = (int)(n_t * TR) + (int)rank * HALF;
       int xrow_nx = -1;                                          // activation rows of this pair's next tile (L2 prefetch target)
-      if (p.l2_prefetch > 0 && t + npairs < total_tiles) {
+      if (t + npairs < total_tiles) {
         int m_n; int64_t n_n;
         tile_split(t + npairs, p.m_tiles, m_n, n_n);
         xrow_nx = (int)(n_n * TR) + (int)rank * HALF;
       }
       for (int kb = 0; kb < nk; ++kb) {
-        if (p.l2_prefetch > 0) {
-          int kp = kb + p.l2_prefetch, xr = xrow;
-          if (kp >= nk) { kp -= nk; xr = xrow_nx; }
-          if (kp < nk && xr >= 0 && elect_one()) {
-            tma_prefetch_l2_2d(&map_x, kp * BKE, xr);
-            if (HM == 1) tma_prefetch_l2_2d(&map_x, kp * BKE + 32, xr);
-            if (HM == 2) tma_prefetch_l2_2d(&map_x2, kp * BKE, xr);
-          }
+        int kp = kb + TC_L2_PREFETCH, xr = xrow;
+        if (kp >= nk) { kp -= nk; xr = xrow_nx; }
+        if (kp < nk && xr >= 0 && elect_one()) {
+          tma_prefetch_l2_2d(&map_x, kp * BKE, xr);
+          if (HM == 1) tma_prefetch_l2_2d(&map_x, kp * BKE + 32, xr);
+          if (HM == 2) tma_prefetch_l2_2d(&map_x2, kp * BKE, xr);
         }
         if (!(ok = mbar_wait_warp(bar_empty(s), ph ^ 1u, p.err))) break;
         const uint32_t st = smem_base + s * T2_STAGE_BYTES;
@@ -679,11 +673,10 @@ int launch_fill(float* p, int64_t n, float v, cudaStream_t st) {
 
 // ------------------------------------------------------------------------------------------------ host side
 bool gemm_tc2_supported(const GemmArgs& g, int amode) {
-  const bool enabled = settings().tc_2cta;
   const bool fuse = tc_fuse_attn_out_enabled();
   GemmArgs base = g;
   base.at_pos = nullptr; base.pool = nullptr; base.x_h2 = false; base.out_h2 = false; base.pos_h2 = false;
-  if (!enabled || !gemm_tc_supported(base, amode)) return false;
+  if (!gemm_tc_supported(base, amode)) return false;
   if (g.act == ACT_GELU) return false;
   // 128-channel layers: the single-CTA flavour takes ready-made operands only (fp16 planes of the parity-grade mode, fast-mode formats)
   if (g.N % 256 != 0 && !(g.N % 128 == 0 && (gemm_tc2_fast(g) || gemm_tc2_fast_tf32(g) || (g.x_h2 && gemm_tc2_fp16x3(g))))) return false;
@@ -705,7 +698,7 @@ bool gemm_tc2_supported(const GemmArgs& g, int amode) {
 // fp16x3 operands: only where the activations are LIF outputs, the weights carry their half split and the epilogue
 // flavour is instantiated
 bool gemm_tc2_fp16x3(const GemmArgs& g) {
-  return settings().fp16x3 && g.x_unit && g.Wh && g.Wl && g.K % 64 == 0 && g.tc_passes != 1 && !g.residual &&
+  return g.x_unit && g.Wh && g.Wl && g.K % 64 == 0 && g.tc_passes != 1 && !g.residual &&
          (g.at_pos || g.act == ACT_LIF || (g.act == ACT_LEAKY && g.pool) || g.act == ACT_NONE);
 }
 
@@ -724,57 +717,15 @@ bool gemm_tc2_fast_tf32(const GemmArgs& g) {
 }
 
 namespace {
-constexpr size_t t2_smem_fast(bool lt, uint32_t tab_stride, int cg = 2) {
-  return (size_t)(lt ? (cg == 2 ? 3 : 2) : (cg == 2 ? SAPCU_T2_FAST_STAGES : 4)) * (cg == 2 ? 2 : 3) * TC_TILE_BYTES + 1024 + 256 + (lt ? tab_stride : 0);
-}
-// cudaFuncAttributeMaxDynamicSharedMemorySize is a per-device function attribute: set it once per device
-int t2_set_attrs_impl() {
-#define SAPCU_T2_ATTR(A, X, KQ) SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc2_kernel<A, X, KQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T2_SMEM_BYTES))
-  SAPCU_T2_ATTR(ACT_LIF, 0, 1); SAPCU_T2_ATTR(ACT_LIF, 2, 1); SAPCU_T2_ATTR(ACT_LEAKY, 0, 1); SAPCU_T2_ATTR(ACT_LEAKY, 4, 1); SAPCU_T2_ATTR(ACT_NONE, 1, 1); SAPCU_T2_ATTR(ACT_NONE, 0, 1);
-  SAPCU_T2_ATTR(ACT_NONE, 3, 12); SAPCU_T2_ATTR(ACT_NONE, 3, 18); SAPCU_T2_ATTR(ACT_NONE, 3, 24);
-#undef SAPCU_T2_ATTR
-#define SAPCU_T2_ATTR_H(A, X, KQ) SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc2_kernel<A, X, KQ, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T2_SMEM_BYTES))
-  SAPCU_T2_ATTR_H(ACT_LIF, 0, 1); SAPCU_T2_ATTR_H(ACT_LIF, 2, 1); SAPCU_T2_ATTR_H(ACT_LEAKY, 4, 1); SAPCU_T2_ATTR_H(ACT_NONE, 0, 1);
-  SAPCU_T2_ATTR_H(ACT_NONE, 3, 12); SAPCU_T2_ATTR_H(ACT_NONE, 3, 18); SAPCU_T2_ATTR_H(ACT_NONE, 3, 24);
-#undef SAPCU_T2_ATTR_H
-#define SAPCU_T2_ATTR_P(A, X, KQ) SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc2_kernel<A, X, KQ, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T2_SMEM_BYTES))
-  // parity-grade mode with tabulated LIF^T chains: two 64 KiB stages + the table
-  SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc2_kernel<ACT_LIF, 0, 1, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * 4 * TC_TILE_BYTES + 1024 + 256 + LT_SMEM_BUDGET_TC)));
-  SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc2_kernel<ACT_LIF, 0, 1, 2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * 4 * TC_TILE_BYTES + 1024 + 256 + LT_SMEM_BUDGET_TC)));
-  SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc2_kernel<ACT_LIF, 2, 1, 2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * 4 * TC_TILE_BYTES + 1024 + 256 + LT_SMEM_BUDGET_TC)));
-  SAPCU_T2_ATTR_P(ACT_LIF, 0, 1); SAPCU_T2_ATTR_P(ACT_LIF, 2, 1); SAPCU_T2_ATTR_P(ACT_LEAKY, 4, 1); SAPCU_T2_ATTR_P(ACT_NONE, 3, 12); SAPCU_T2_ATTR_P(ACT_NONE, 3, 18); SAPCU_T2_ATTR_P(ACT_NONE, 3, 24);
-#undef SAPCU_T2_ATTR_P
-#define SAPCU_T2_ATTR_F(A, X, KQ, LTQ) SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc2_kernel<A, X, KQ, 3, LTQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t2_smem_fast(LTQ != 0, LT_SMEM_BUDGET)))
-  SAPCU_T2_ATTR_F(ACT_LIF, 0, 1, 0); SAPCU_T2_ATTR_F(ACT_LIF, 0, 1, 1); SAPCU_T2_ATTR_F(ACT_LIF, 2, 1, 0); SAPCU_T2_ATTR_F(ACT_LIF, 2, 1, 1);
-  SAPCU_T2_ATTR_F(ACT_LEAKY, 4, 1, 0); SAPCU_T2_ATTR_F(ACT_NONE, 3, 12, 0); SAPCU_T2_ATTR_F(ACT_NONE, 3, 18, 0); SAPCU_T2_ATTR_F(ACT_NONE, 3, 24, 0);
-#undef SAPCU_T2_ATTR_F
-#define SAPCU_T2_ATTR_F1(A, X, KQ, LTQ) SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc2_kernel<A, X, KQ, 3, LTQ, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t2_smem_fast(LTQ != 0, LT_SMEM_BUDGET, 1)))
-  SAPCU_T2_ATTR_F1(ACT_LIF, 0, 1, 0); SAPCU_T2_ATTR_F1(ACT_LIF, 0, 1, 1); SAPCU_T2_ATTR_F1(ACT_LIF, 2, 1, 0); SAPCU_T2_ATTR_F1(ACT_LIF, 2, 1, 1);
-  SAPCU_T2_ATTR_F1(ACT_NONE, 3, 12, 0); SAPCU_T2_ATTR_F1(ACT_NONE, 3, 18, 0); SAPCU_T2_ATTR_F1(ACT_NONE, 3, 24, 0);
-#undef SAPCU_T2_ATTR_F1
-  // single-CTA flavour on (hi, lo) planes: 2 stages of 96 KiB, or 1 stage + the LIF table
-#define SAPCU_T2_ATTR_P1(A, X, KQ, LTQ) SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc2_kernel<A, X, KQ, 2, LTQ, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((LTQ ? 1 : 2) * 6 * TC_TILE_BYTES + 1024 + 256 + (LTQ ? LT_SMEM_BUDGET : 0))))
-  SAPCU_T2_ATTR_P1(ACT_LIF, 0, 1, 0); SAPCU_T2_ATTR_P1(ACT_LIF, 0, 1, 1); SAPCU_T2_ATTR_P1(ACT_LIF, 2, 1, 0); SAPCU_T2_ATTR_P1(ACT_LIF, 2, 1, 1);
-  SAPCU_T2_ATTR_P1(ACT_NONE, 3, 12, 0); SAPCU_T2_ATTR_P1(ACT_NONE, 3, 18, 0); SAPCU_T2_ATTR_P1(ACT_NONE, 3, 24, 0);
-#undef SAPCU_T2_ATTR_P1
-#define SAPCU_T2_ATTR_T(LTQ, CGQ) SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc2_kernel<ACT_LIF, 0, 1, 4, LTQ, CGQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t2_smem_fast(LTQ != 0, LT_SMEM_BUDGET, CGQ)))
-  SAPCU_T2_ATTR_T(0, 1); SAPCU_T2_ATTR_T(1, 1); SAPCU_T2_ATTR_T(0, 2); SAPCU_T2_ATTR_T(1, 2);
-  SAPCU_CUDA_CHECK(cudaFuncSetAttribute(gemm_tc2_kernel<ACT_NONE, 0, 1, 4, 0, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t2_smem_fast(false, 0, 2)));
-#undef SAPCU_T2_ATTR_T
-  return 0;
-}
-int t2_set_attrs() {
-  static PerDeviceOnce once;
-  return once.run(&t2_set_attrs_impl);
+constexpr size_t t2_smem_fast(bool lt, uint32_t tab_stride, int cg) {
+  return (size_t)(lt ? (cg == 2 ? 3 : 2) : (cg == 2 ? T2_FAST_STAGES : 4)) * (cg == 2 ? 2 : 3) * TC_TILE_BYTES + 1024 + 256 + (lt ? tab_stride : 0);
 }
 }  // namespace
 
 int launch_gemm_tc2(const GemmArgs& g, cudaStream_t st) {
   SAPCU_REQUIRE(gemm_tc2_supported(g, A_PLAIN), "gemm_tc2: unsupported problem");
-  { const int rc = t2_set_attrs(); if (rc) return rc; }
   int* err = tc_err_flag();
   SAPCU_REQUIRE(err != nullptr, "gemm_tc2: cannot allocate the watchdog flag");
-  const int l2pf = settings().l2pf;
   const int tile_rows = g.at_pos ? tc_fused_tile_rows(g.kk) : T2_BN;
   const bool fast = gemm_tc2_fast(g), fast_tf32 = !fast && gemm_tc2_fast_tf32(g);
   const int cg = (g.N % 256 == 0) ? 2 : 1;                   // CTAs per tile: 1 = the single-CTA flavour for 128-channel layers (fast mode)
@@ -807,7 +758,7 @@ int launch_gemm_tc2(const GemmArgs& g, cudaStream_t st) {
   p.pool = g.pool; p.pool_T = g.pool_T; p.pool_rows = (int64_t)g.pool_T * g.pool_M;
   p.idx8 = g.idx8; p.ldi8w = g.ldi8w;
   p.at_pos = g.at_pos; p.at_v = g.at_v; p.at_ldv = g.at_ldv; p.at_sqrt = g.at_sqrt; p.tile_rows = tile_rows;
-  p.m_tiles = g.N / (128 * cg); p.n_tiles = ceil_div(g.R, tile_rows); p.err = err; p.split_w = 0; p.raw_hi = 1; p.l2_prefetch = l2pf; p.passes = g.tc_passes == 1 ? 1 : 3;
+  p.m_tiles = g.N / (128 * cg); p.n_tiles = ceil_div(g.R, tile_rows); p.err = err; p.split_w = 0; p.passes = g.tc_passes == 1 ? 1 : 3;
   p.out_h2 = g.out_h2 ? 1 : 0; p.pos_h2 = g.pos_h2 ? 1 : 0;
   p.lif_tab = nullptr; p.lif_tab_stride = 0;
   p.x_scale = h16 ? 8192.0f : 1.0f;                         // soft spikes lie in (0, 0.7): x * 2^13 < 2^13, residual * 2^13 >= fp16's normal range
@@ -822,13 +773,9 @@ int launch_gemm_tc2(const GemmArgs& g, cudaStream_t st) {
     p.passes = 1; p.x_scale = 1.0f; p.acc_scale = 1.0f;
     const size_t smem = t2_smem_fast(lt, g.lif_tab_stride, cg);
     const int gridf = cg * pairs;
-#define SAPCU_T2_LAUNCH_T(LTQ, CGQ) gemm_tc2_kernel<ACT_LIF, 0, 1, 4, LTQ, CGQ><<<gridf, (T2_EPI_WARP0 + 16) * 32, smem, st>>>(mw, mwlo, mx, mx2, p)
-    if (g.act == ACT_NONE) gemm_tc2_kernel<ACT_NONE, 0, 1, 4, 0, 2><<<gridf, (T2_EPI_WARP0 + 16) * 32, smem, st>>>(mw, mwlo, mx, mx2, p);
-    else if (cg == 2) { if (lt) SAPCU_T2_LAUNCH_T(1, 2); else SAPCU_T2_LAUNCH_T(0, 2); }
-    else { if (lt) SAPCU_T2_LAUNCH_T(1, 1); else SAPCU_T2_LAUNCH_T(0, 1); }
-#undef SAPCU_T2_LAUNCH_T
-    SAPCU_LAUNCH_CHECK();
-    return 0;
+    if (g.act == ACT_NONE) return tc_launch<gemm_tc2_kernel<ACT_NONE, 0, 1, 4, 0, 2>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
+    if (cg == 2) return lt ? tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 4, 1, 2>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p) : tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 4, 0, 2>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
+    return lt ? tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 4, 1, 1>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p) : tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 4, 0, 1>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
   }
   if (fast) {
     // one fp16 product per MAC: map_w = the hi half of the fp16 weight split, map_x = the single activation plane
@@ -840,26 +787,22 @@ int launch_gemm_tc2(const GemmArgs& g, cudaStream_t st) {
     p.x_scale = 8192.0f; p.acc_scale = g.winv / 8192.0f;
     const size_t smem = t2_smem_fast(lt, g.lif_tab_stride, cg);
     const int gridf = cg * pairs;
-#define SAPCU_T2_LAUNCH_F(A, X, KQ, LTQ)                                                                                \
-  do {                                                                                                                  \
-    if (cg == 2) gemm_tc2_kernel<A, X, KQ, 3, LTQ><<<gridf, (T2_EPI_WARP0 + 16) * 32, smem, st>>>(mw, mwlo, mx, mx2, p);    \
-    else gemm_tc2_kernel<A, X, KQ, 3, LTQ, 1><<<gridf, (T2_EPI_WARP0 + 16) * 32, smem, st>>>(mw, mwlo, mx, mx2, p);        \
-  } while (0)
-    if (g.at_pos) {
-      if (g.kk == 12) SAPCU_T2_LAUNCH_F(ACT_NONE, 3, 12, 0); else if (g.kk == 18) SAPCU_T2_LAUNCH_F(ACT_NONE, 3, 18, 0); else SAPCU_T2_LAUNCH_F(ACT_NONE, 3, 24, 0);
-    } else if (g.act == ACT_LEAKY) {
+    if (g.at_pos)
+      return with_kk(g.kk, [&](auto KQ) {
+        constexpr int kq = decltype(KQ)::value;
+        return cg == 2 ? tc_launch<gemm_tc2_kernel<ACT_NONE, 3, kq, 3, 0>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p) : tc_launch<gemm_tc2_kernel<ACT_NONE, 3, kq, 3, 0, 1>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
+      });
+    if (g.act == ACT_LEAKY) {
       SAPCU_REQUIRE(cg == 2, "gemm_tc2(fast): the pooled conv5 epilogue needs N %% 256 == 0");
-      gemm_tc2_kernel<ACT_LEAKY, 4, 1, 3, 0><<<gridf, (T2_EPI_WARP0 + 16) * 32, smem, st>>>(mw, mwlo, mx, mx2, p);
+      return tc_launch<gemm_tc2_kernel<ACT_LEAKY, 4, 1, 3, 0>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
     }
-    else if (g.edge_bias) { if (lt) SAPCU_T2_LAUNCH_F(ACT_LIF, 2, 1, 1); else SAPCU_T2_LAUNCH_F(ACT_LIF, 2, 1, 0); }
-    else { if (lt) SAPCU_T2_LAUNCH_F(ACT_LIF, 0, 1, 1); else SAPCU_T2_LAUNCH_F(ACT_LIF, 0, 1, 0); }
-#undef SAPCU_T2_LAUNCH_F
-    SAPCU_LAUNCH_CHECK();
-    return 0;
+    if (g.edge_bias) {
+      if (cg == 2) return lt ? tc_launch<gemm_tc2_kernel<ACT_LIF, 2, 1, 3, 1>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p) : tc_launch<gemm_tc2_kernel<ACT_LIF, 2, 1, 3, 0>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
+      return lt ? tc_launch<gemm_tc2_kernel<ACT_LIF, 2, 1, 3, 1, 1>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p) : tc_launch<gemm_tc2_kernel<ACT_LIF, 2, 1, 3, 0, 1>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
+    }
+    if (cg == 2) return lt ? tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 3, 1>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p) : tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 3, 0>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
+    return lt ? tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 3, 1, 1>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p) : tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 3, 0, 1>>(gridf, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
   }
-  const int grid = 2 * pairs;
-#define SAPCU_T2_LAUNCH_H(A, X, KQ) gemm_tc2_kernel<A, X, KQ, 1><<<grid, (T2_EPI_WARP0 + 16) * 32, T2_SMEM_BYTES, st>>>(mw, mwlo, mx, mx2, p)
-#define SAPCU_T2_LAUNCH_P(A, X, KQ) gemm_tc2_kernel<A, X, KQ, 2><<<grid, (T2_EPI_WARP0 + 16) * 32, T2_SMEM_BYTES, st>>>(mw, mwlo, mx, mx2, p)
   if (pre && cg == 1) {
     // 128-channel layer on (hi, lo) planes: the single-CTA flavour (fp16x3 products; LIF table next to ONE 96 KiB stage)
     SAPCU_REQUIRE(g.at_pos || g.act == ACT_LIF, "gemm_tc2: the single-CTA plane path serves the LIF layers and the attention tail");
@@ -867,14 +810,10 @@ int launch_gemm_tc2(const GemmArgs& g, cudaStream_t st) {
     if (lt) { pairs = (pairs / p.m_tiles) * p.m_tiles; p.lif_tab = reinterpret_cast<const uint8_t*>(g.lif_tab); p.lif_tab_stride = g.lif_tab_stride; }
     SAPCU_REQUIRE(pairs >= 1, "gemm_tc2(single-CTA planes): empty grid");
     const size_t smem = (size_t)(lt ? 1 : 2) * 6 * TC_TILE_BYTES + 1024 + 256 + (lt ? g.lif_tab_stride : 0);
-#define SAPCU_T2_LAUNCH_P1(A, X, KQ, LTQ) gemm_tc2_kernel<A, X, KQ, 2, LTQ, 1><<<pairs, (T2_EPI_WARP0 + 16) * 32, smem, st>>>(mw, mwlo, mx, mx2, p)
-    if (g.at_pos) {
-      if (g.kk == 12) SAPCU_T2_LAUNCH_P1(ACT_NONE, 3, 12, 0); else if (g.kk == 18) SAPCU_T2_LAUNCH_P1(ACT_NONE, 3, 18, 0); else SAPCU_T2_LAUNCH_P1(ACT_NONE, 3, 24, 0);
-    } else if (g.edge_bias) { if (lt) SAPCU_T2_LAUNCH_P1(ACT_LIF, 2, 1, 1); else SAPCU_T2_LAUNCH_P1(ACT_LIF, 2, 1, 0); }
-    else { if (lt) SAPCU_T2_LAUNCH_P1(ACT_LIF, 0, 1, 1); else SAPCU_T2_LAUNCH_P1(ACT_LIF, 0, 1, 0); }
-#undef SAPCU_T2_LAUNCH_P1
-    SAPCU_LAUNCH_CHECK();
-    return 0;
+    if (g.at_pos)
+      return with_kk(g.kk, [&](auto KQ) { return tc_launch<gemm_tc2_kernel<ACT_NONE, 3, decltype(KQ)::value, 2, 0, 1>>(pairs, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p); });
+    if (g.edge_bias) return lt ? tc_launch<gemm_tc2_kernel<ACT_LIF, 2, 1, 2, 1, 1>>(pairs, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p) : tc_launch<gemm_tc2_kernel<ACT_LIF, 2, 1, 2, 0, 1>>(pairs, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
+    return lt ? tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 2, 1, 1>>(pairs, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p) : tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 2, 0, 1>>(pairs, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
   }
   if (pre && g.act == ACT_LIF && g.lif_tab && g.lif_tab_stride > 0 && g.lif_tab_stride <= LT_SMEM_BUDGET_TC) {
     // fp16x3 products on (hi, lo) planes + the layer's tabulated LIF^T chain: 2 stages of 64 KiB leave room for the table
@@ -882,56 +821,38 @@ int launch_gemm_tc2(const GemmArgs& g, cudaStream_t st) {
     SAPCU_REQUIRE(pairs >= 1, "gemm_tc2(tables): empty grid");
     p.lif_tab = reinterpret_cast<const uint8_t*>(g.lif_tab); p.lif_tab_stride = g.lif_tab_stride;
     const size_t smem = 2 * 4 * (size_t)TC_TILE_BYTES + 1024 + 256 + g.lif_tab_stride;
-    if (g.edge_bias) gemm_tc2_kernel<ACT_LIF, 2, 1, 2, 1><<<2 * pairs, (T2_EPI_WARP0 + 16) * 32, smem, st>>>(mw, mwlo, mx, mx2, p);
-    else gemm_tc2_kernel<ACT_LIF, 0, 1, 2, 1><<<2 * pairs, (T2_EPI_WARP0 + 16) * 32, smem, st>>>(mw, mwlo, mx, mx2, p);
-    SAPCU_LAUNCH_CHECK();
-    return 0;
+    if (g.edge_bias) return tc_launch<gemm_tc2_kernel<ACT_LIF, 2, 1, 2, 1>>(2 * pairs, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
+    return tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 2, 1>>(2 * pairs, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
   }
+  const int grid = 2 * pairs;
   if (pre) {
-    if (g.at_pos) {
-      if (g.kk == 12) SAPCU_T2_LAUNCH_P(ACT_NONE, 3, 12); else if (g.kk == 18) SAPCU_T2_LAUNCH_P(ACT_NONE, 3, 18); else SAPCU_T2_LAUNCH_P(ACT_NONE, 3, 24);
-    } else if (g.act == ACT_LEAKY) SAPCU_T2_LAUNCH_P(ACT_LEAKY, 4, 1);
-    else if (g.edge_bias) SAPCU_T2_LAUNCH_P(ACT_LIF, 2, 1);
-    else SAPCU_T2_LAUNCH_P(ACT_LIF, 0, 1);
-    SAPCU_LAUNCH_CHECK();
-    return 0;
+    if (g.at_pos) return with_kk(g.kk, [&](auto KQ) { return tc_launch<gemm_tc2_kernel<ACT_NONE, 3, decltype(KQ)::value, 2>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p); });
+    if (g.act == ACT_LEAKY) return tc_launch<gemm_tc2_kernel<ACT_LEAKY, 4, 1, 2>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
+    if (g.edge_bias) return tc_launch<gemm_tc2_kernel<ACT_LIF, 2, 1, 2>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
+    return tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 2>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
   }
   if (h16) {
-    if (g.at_pos) {
-      if (g.kk == 12) SAPCU_T2_LAUNCH_H(ACT_NONE, 3, 12); else if (g.kk == 18) SAPCU_T2_LAUNCH_H(ACT_NONE, 3, 18); else SAPCU_T2_LAUNCH_H(ACT_NONE, 3, 24);
-    }
-    else if (g.act == ACT_LIF && g.edge_bias) SAPCU_T2_LAUNCH_H(ACT_LIF, 2, 1);
-    else if (g.act == ACT_LIF) SAPCU_T2_LAUNCH_H(ACT_LIF, 0, 1);
-    else if (g.act == ACT_LEAKY) SAPCU_T2_LAUNCH_H(ACT_LEAKY, 4, 1);
-    else SAPCU_T2_LAUNCH_H(ACT_NONE, 0, 1);
-    SAPCU_LAUNCH_CHECK();
-    return 0;
+    if (g.at_pos) return with_kk(g.kk, [&](auto KQ) { return tc_launch<gemm_tc2_kernel<ACT_NONE, 3, decltype(KQ)::value, 1>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p); });
+    if (g.act == ACT_LIF && g.edge_bias) return tc_launch<gemm_tc2_kernel<ACT_LIF, 2, 1, 1>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
+    if (g.act == ACT_LIF) return tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 1>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
+    if (g.act == ACT_LEAKY) return tc_launch<gemm_tc2_kernel<ACT_LEAKY, 4, 1, 1>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
+    return tc_launch<gemm_tc2_kernel<ACT_NONE, 0, 1, 1>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
   }
-#undef SAPCU_T2_LAUNCH_H
-#undef SAPCU_T2_LAUNCH_P
   if (g.act == ACT_LIF && !g.edge_bias && g.lif_tab && g.lif_tab_stride > 0 && g.lif_tab_stride <= LT_SMEM_BUDGET_TC) {
     // 3xTF32 products (splitter path) + the layer's tabulated LIF^T chain: two 64 KiB stages next to the table
     pairs = (pairs / p.m_tiles) * p.m_tiles;
     SAPCU_REQUIRE(pairs >= 1, "gemm_tc2(3xTF32 + table): empty grid");
     p.lif_tab = reinterpret_cast<const uint8_t*>(g.lif_tab); p.lif_tab_stride = g.lif_tab_stride;
     const size_t smem = 2 * 4 * (size_t)TC_TILE_BYTES + 1024 + 256 + g.lif_tab_stride;
-    gemm_tc2_kernel<ACT_LIF, 0, 1, 0, 1><<<2 * pairs, (T2_EPI_WARP0 + 16) * 32, smem, st>>>(mw, mwlo, mx, mx2, p);
-    SAPCU_LAUNCH_CHECK();
-    return 0;
+    return tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 0, 1>>(2 * pairs, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
   }
-#define SAPCU_T2_LAUNCH(A, X, KQ) gemm_tc2_kernel<A, X, KQ><<<grid, (T2_EPI_WARP0 + 16) * 32, T2_SMEM_BYTES, st>>>(mw, mwlo, mx, mx2, p)
-  if (g.at_pos) {
-    if (g.kk == 12) SAPCU_T2_LAUNCH(ACT_NONE, 3, 12); else if (g.kk == 18) SAPCU_T2_LAUNCH(ACT_NONE, 3, 18); else SAPCU_T2_LAUNCH(ACT_NONE, 3, 24);
-  }
-  else if (g.act == ACT_LIF && g.edge_bias) SAPCU_T2_LAUNCH(ACT_LIF, 2, 1);
-  else if (g.act == ACT_LIF) SAPCU_T2_LAUNCH(ACT_LIF, 0, 1);
-  else if (g.act == ACT_LEAKY && g.pool) SAPCU_T2_LAUNCH(ACT_LEAKY, 4, 1);
-  else if (g.act == ACT_LEAKY) SAPCU_T2_LAUNCH(ACT_LEAKY, 0, 1);
-  else if (g.residual) SAPCU_T2_LAUNCH(ACT_NONE, 1, 1);
-  else SAPCU_T2_LAUNCH(ACT_NONE, 0, 1);
-#undef SAPCU_T2_LAUNCH
-  SAPCU_LAUNCH_CHECK();
-  return 0;
+  if (g.at_pos) return with_kk(g.kk, [&](auto KQ) { return tc_launch<gemm_tc2_kernel<ACT_NONE, 3, decltype(KQ)::value>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p); });
+  if (g.act == ACT_LIF && g.edge_bias) return tc_launch<gemm_tc2_kernel<ACT_LIF, 2, 1>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
+  if (g.act == ACT_LIF) return tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
+  if (g.act == ACT_LEAKY && g.pool) return tc_launch<gemm_tc2_kernel<ACT_LEAKY, 4, 1>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
+  if (g.act == ACT_LEAKY) return tc_launch<gemm_tc2_kernel<ACT_LEAKY, 0, 1>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
+  if (g.residual) return tc_launch<gemm_tc2_kernel<ACT_NONE, 1, 1>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
+  return tc_launch<gemm_tc2_kernel<ACT_NONE, 0, 1>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
 }
 
 }  // namespace sapcu

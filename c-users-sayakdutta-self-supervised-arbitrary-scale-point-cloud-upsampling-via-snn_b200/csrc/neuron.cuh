@@ -44,33 +44,11 @@ __device__ __forceinline__ float rcp_approx_ord(float x) {
   return y;
 }
 
+// also the reciprocal of the fast LIF step, where x = 2 + 2*exp2(.) may overflow to +inf (v << 0): the answer is then 0
 __device__ __forceinline__ float rcp_approx(float x) {
   float y;
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
-}
-
-// 1/x on the FMA pipe (x in [2, inf]): magic-constant seed + 3 Newton steps (relative error < 1e-7).
-// Trades one MUFU.RCP (8 issue cycles of the 16-lane MUFU pipe per warp) for 7 FMA-pipe instructions; the LIF
-// recurrence is MUFU-bound (3 MUFU vs 12 FP per element-step), so this rebalances the two pipes.
-#ifndef SAPCU_LIF_RCP
-#define SAPCU_LIF_RCP rcp_lif
-#endif
-__device__ __forceinline__ float rcp_fma(float x) {
-  float r = __uint_as_float(0x7EF311C7u - __float_as_uint(x));
-  r = r * fmaf(-x, r, 2.0f);
-  r = r * fmaf(-x, r, 2.0f);
-  r = r * fmaf(-x, r, 2.0f);
-  return r;
-}
-
-// reciprocal used by the fast LIF step; x = 2 + 2*exp2(.) may overflow to +inf (v << 0), where the answer is 0
-__device__ __forceinline__ float rcp_lif(float x) {
-#ifdef SAPCU_LIF_RCP_FMA          // measured slower on B200 (321.9 vs 315.3 ms/step): the step is issue-bound, not MUFU-bound
-  return rcp_fma(fminf(x, 1e30f));
-#else
-  return rcp_approx(x);
-#endif
 }
 
 // PRECISE=true : libdevice expf (<= 1 ulp) -- the fp32 parity mode
@@ -148,29 +126,6 @@ __device__ __forceinline__ float lif_chain(float u, const NeuronParams& p, int T
   return s;
 }
 
-// Mixed reciprocal for the interleaved LIF chain: elements i with (i % 8) < SAPCU_LIF_RCP_FMA_N take the FMA-pipe Newton
-// reciprocal, the rest MUFU.RCP.  The recurrence needs 3 MUFU (8 pipe cycles each per warp) against 12 FP
-// instructions per element-step, so in principle moving a few reciprocals over rebalances the two pipes.  Measured on
-// B200 (same box, 8,192-seed step): N = 0: 272.6 ms, 2: 276.3, 4: 276.7, 5: 280.4 -- every extra instruction costs
-// under the board's power cap, so the default stays all-MUFU.
-#ifndef SAPCU_LIF_RCP_FMA_N
-#define SAPCU_LIF_RCP_FMA_N 0
-#endif
-template <int I>
-__device__ __forceinline__ float rcp_lif_mixed(float x) {
-  if ((I & 7) < SAPCU_LIF_RCP_FMA_N) return rcp_fma(fminf(x, 1e30f));
-  return rcp_approx(x);
-}
-template <int NV, int I = 0>
-struct RcpMixed {
-  static __device__ __forceinline__ void run(float (&e)[NV]) {
-    e[I] = rcp_lif_mixed<I>(fmaf(2.0f, e[I], 2.0f));
-    RcpMixed<NV, I + 1>::run(e);
-  }
-};
-template <int NV>
-struct RcpMixed<NV, NV> { static __device__ __forceinline__ void run(float (&)[NV]) {} };
-
 // LIF^T on NV independent accumulators of one channel (interleaved for ILP); fast-math flavour.
 // Algebraically identical to neuron_step, re-associated for the FMA pipe (12 FP + 3 MUFU per element-step):
 //   * the soft spike is > 0, so the refractory gate is open at step 0 only: later steps take no input
@@ -190,7 +145,7 @@ __device__ __forceinline__ void lif_chain_vec_fast(float (&u)[NV], const NeuronP
     const float v = mm - p.th0;
     const float g = exp2f_approx((k_g * v) * v);
     const float e = exp2f_approx(k_s * v);
-    const float s = fmaf(c_g, g, SAPCU_LIF_RCP(fmaf(2.0f, e, 2.0f)));
+    const float s = fmaf(c_g, g, rcp_approx(fmaf(2.0f, e, 2.0f)));
     m[i] = fmaf(-mm, s, mm);
     rho[i] = s;
     th[i] = fmaf(0.95f, p.th0, fmaf(a95, s, c05));
@@ -213,7 +168,8 @@ __device__ __forceinline__ void lif_chain_vec_fast(float (&u)[NV], const NeuronP
     for (int i = 0; i < NV; ++i) e[i] = exp2f_approx_ord(e[i]);
 #pragma unroll
     for (int i = 0; i < NV; ++i) g[i] = exp2f_approx_ord(g[i]);
-    RcpMixed<NV>::run(e);
+#pragma unroll
+    for (int i = 0; i < NV; ++i) e[i] = rcp_approx(fmaf(2.0f, e[i], 2.0f));
 #pragma unroll
     for (int i = 0; i < NV; ++i) {
       const float s = fmaf(c_g, g[i], e[i]);
@@ -289,7 +245,7 @@ __device__ __forceinline__ float neuron_step_fast(float u, float& m, float& th, 
   const float v = mm - (FIRST ? k.th0 : th);
   const float g = exp2f_approx((k_g * v) * v);
   const float e = exp2f_approx(k_s * v);
-  const float s = fmaf(c_g, g, SAPCU_LIF_RCP(fmaf(2.0f, e, 2.0f)));
+  const float s = fmaf(c_g, g, rcp_approx(fmaf(2.0f, e, 2.0f)));
   m = fmaf(-mm, s, mm);
   rho = FIRST ? s : fmaf(rho, k.r, s);
   th = fmaf(0.95f, FIRST ? k.th0 : th, fmaf(k.a95, s, k.c05));

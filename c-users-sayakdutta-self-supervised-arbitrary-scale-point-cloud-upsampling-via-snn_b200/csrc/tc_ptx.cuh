@@ -1,6 +1,7 @@
 // PTX wrappers shared by the tcgen05 GEMM engines (sm_100a): mbarrier, TMA, UMMA descriptors, tcgen05 mma/ld/commit.
 #pragma once
 #include <cstdlib>
+#include <type_traits>
 #include <cuda_fp16.h>
 #include "neuron.cuh"
 #include <cuda.h>
@@ -13,6 +14,7 @@ constexpr int TC_BM = 128;        // output channels per CTA tile (UMMA M per CT
 constexpr int TC_BK = 32;         // fp32 elements per k-block = one 128-byte swizzle row
 constexpr uint32_t TC_TILE_BYTES = TC_BM * TC_BK * 4;          // 16 KiB: a 128-row operand tile
 constexpr long long TC_WATCHDOG_CLOCKS = 6000000000LL;         // ~3 s at 1.9 GHz
+constexpr int TC_L2_PREFETCH = 4;                              // k-blocks of look-ahead for the activation tile's L2 prefetch
 
 // ------------------------------------------------------------------------------------------------ PTX wrappers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -68,13 +70,6 @@ __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.
 __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-// round-to-nearest fp32 -> tf32 (low 13 mantissa bits cleared): an unbiased hi part, |lo| <= 2^-11 |x|
-__device__ __forceinline__ float tf32_rna(float x) {
-  uint32_t r;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-  return __uint_as_float(r);
-}
 
 // K-major, 128-byte swizzled operand tile (rows of 32 fp32 = 128 B, 8-row groups 1024 B apart)
 __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t saddr) {
@@ -202,8 +197,6 @@ struct TcParams {
   int m_tiles; int64_t n_tiles;
   int split_w;                // 1: W arrives raw and is split in shared memory; 0: map_w / map_wlo hold pre-split (hi, lo)
   int passes;                 // 3: w_lo*x_hi + w_hi*x_lo + w_hi*x_hi (fp32-grade); 1: w_hi*x_hi only (plain TF32)
-  int l2_prefetch;            // k-blocks of look-ahead for the activation L2 prefetch (0 = off)
-  int raw_hi;                 // 1: leave the raw X tile as the hi operand (tensor core ignores the low 13 bits), lo by truncation
   int* err;
 };
 
@@ -326,6 +319,26 @@ __device__ __forceinline__ void attn_tail_dispatch(const TcParams& p, uint32_t t
 // host helpers (gemm_tc.cu)
 int tc_make_map(CUtensorMap* m, const float* base, int64_t rows, int K, int64_t ld, int box_rows);
 int* tc_err_flag();
+// Kern<<<grid, threads, smem, st>>>(args...).  The first launch of each kernel on a device raises its dynamic shared-memory
+// limit to what the device allows next to the kernel's static shared memory, so the byte count computed at the launch site
+// is the only one written down.
+template <auto Kern, typename... A>
+int tc_launch(int grid, int threads, size_t smem, cudaStream_t st, const A&... args) {
+  static PerDeviceOnce once;
+  const int rc = once.run([]() -> int {
+    int dev = 0, optin = 0;
+    cudaFuncAttributes fa;
+    SAPCU_CUDA_CHECK(cudaGetDevice(&dev));
+    SAPCU_CUDA_CHECK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    SAPCU_CUDA_CHECK(cudaFuncGetAttributes(&fa, Kern));
+    SAPCU_CUDA_CHECK(cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)fa.sharedSizeBytes));
+    return 0;
+  });
+  if (rc) return rc;
+  Kern<<<grid, threads, smem, st>>>(args...);
+  SAPCU_LAUNCH_CHECK();
+  return 0;
+}
 // 2-D fp16 row-major [rows, K] -> boxes of [box_rows, 64 halfs] with 128B swizzle
 int tc_make_map_f16(CUtensorMap* m, const void* base, int64_t rows, int K, int box_rows);
 // rows a tile advances by in the fused attention epilogue (EXTRA == 3): the whole points that fit in the 256-row MMA tile
@@ -333,6 +346,12 @@ int tc_make_map_f16(CUtensorMap* m, const void* base, int64_t rows, int K, int b
 inline int tc_fused_tile_rows(int kk) {
   if (kk == 12 || kk == 18 || kk == 24) return (256 / kk) * kk;
   return 0;
+}
+// f(std::integral_constant<int, kk>{}) for the neighbour counts of tc_fused_tile_rows: the fused attention tail's instantiations
+template <class F> int with_kk(int kk, F&& f) {
+  if (kk == 12) return f(std::integral_constant<int, 12>{});
+  if (kk == 18) return f(std::integral_constant<int, 18>{});
+  return f(std::integral_constant<int, 24>{});
 }
 inline bool tc_fuse_attn_out_enabled() { return settings().fuse_attnout; }
 
