@@ -4,6 +4,7 @@
 torch is plumbing here: parameter containers, device memory for inputs/outputs/workspace, the stream.
 """
 import ctypes
+import threading
 
 import torch
 import torch.nn as nn
@@ -18,9 +19,11 @@ class NativeModel(nn.Module):
 
     def __init__(self):
         super().__init__()
-        self._handle = None
-        self._handle_version = None
-        self._ws = None
+        self._owner = None          # DataParallel replicas: the module whose handles and workspaces they use
+        self._handles = {}          # device index -> (state version, native handle), built from this module's parameters
+        self._workspaces = {}       # (device index, cudaStream_t) -> uint8 workspace tensor
+        self._lock = threading.Lock()
+        self._ws_last = None
         self.mode = N.MODE_FP32
 
     # ------------------------------------------------------------------ handle management
@@ -31,14 +34,31 @@ class NativeModel(nn.Module):
         # parameters/buffers are re-uploaded when any of them was modified in place or replaced
         return tuple((k, v.data_ptr(), v._version) for k, v in self.state_dict(keep_vars=True).items())
 
+    def _root(self):
+        return self if self._owner is None else self._owner
+
     def _ensure_handle(self, device=None):
-        """The native handle for the module's current parameters on `device` (the weights are uploaded to the CUDA device
-        that is current at finalize time, so the device is part of the version key; callers hold torch.cuda.device(device))."""
-        dev_index = torch.device(device).index if device is not None else (torch.cuda.current_device() if torch.cuda.is_available() else -1)
-        ver = (dev_index,) + self._state_version()
-        if self._handle is not None and ver == self._handle_version:
-            return self._handle
-        self._drop_handle()
+        """The native handle for the module's current parameters on `device` (default: the current CUDA device).  The weights
+        are uploaded to the device that is current at finalize time and the handle only runs there, so callers hold
+        torch.cuda.device(device).  One handle per device, built once per parameter version; a DataParallel replica gets
+        its owner's handle, built from the owner's parameters."""
+        owner = self._root()
+        dev_index = torch.device(device).index if device is not None else None
+        if dev_index is None:
+            dev_index = torch.cuda.current_device() if torch.cuda.is_available() else -1
+        ver = owner._state_version()
+        with owner._lock:
+            cur = owner._handles.get(dev_index)
+            if cur is not None and cur[0] == ver:
+                return cur[1]
+            if cur is not None:
+                del owner._handles[dev_index]
+                N.lib().sapcu_model_destroy(cur[1])
+            h = owner._build_handle()
+            owner._handles[dev_index] = (ver, h)
+            return h
+
+    def _build_handle(self):
         L = N.lib()
         cfg = (ctypes.c_int32 * len(self._cfg_ints()))(*self._cfg_ints())
         h = L.sapcu_model_create(self.KIND, cfg, len(cfg))
@@ -54,19 +74,34 @@ class NativeModel(nn.Module):
         except Exception:
             L.sapcu_model_destroy(h)
             raise
-        self._handle, self._handle_version = h, ver
         return h
 
-    def _drop_handle(self):
-        if self._handle is not None:
-            N.lib().sapcu_model_destroy(self._handle)
-            self._handle = None
-
     def __del__(self):
+        if self.__dict__.get("_owner") is not None or not self.__dict__.get("_handles"):
+            return                  # a replica owns nothing
         try:
-            self._drop_handle()
+            handles, self._handles = self._handles, {}
+            L = N.lib()
+            for _, h in handles.values():
+                L.sapcu_model_destroy(h)
         except Exception:
             pass
+
+    def _replicate_for_data_parallel(self):
+        replica = super()._replicate_for_data_parallel()
+        replica.__dict__["_owner"] = self._root()       # plain attribute: not a registered submodule
+        replica.__dict__["_ws_last"] = None
+        return replica
+
+    def __getstate__(self):
+        # copies (copy.deepcopy, pickle) start without native state: a handle belongs to exactly one module
+        state = self.__dict__.copy()
+        state.update(_owner=None, _handles={}, _workspaces={}, _lock=None, _ws_last=None)
+        return state
+
+    def __setstate__(self, state):
+        super().__setstate__(state)
+        self._lock = threading.Lock()
 
     # ------------------------------------------------------------------ reference API surface
     def reset_states(self):
@@ -86,16 +121,37 @@ class NativeModel(nn.Module):
         return self
 
     # ------------------------------------------------------------------ helpers for subclasses
+    @property
+    def _ws(self):
+        """The workspace of the most recent forward on this module (what tap() reads).  Setting it to None also releases
+        the cached workspaces, so that the next forward allocates under the current WORKSPACE_CAP."""
+        return self._ws_last
+
+    @_ws.setter
+    def _ws(self, value):
+        if value is None:
+            self._root()._workspaces.clear()
+        self._ws_last = value
+
     def _workspace(self, S, M, device):
+        """(workspace tensor, bytes to pass to the forward).  Workspaces are cached per (device, stream): calls on one stream
+        run in order and may share one, calls on two streams never do.  The byte count is max(one patch, min(need,
+        WORKSPACE_CAP)) whatever the cached tensor's size, so WORKSPACE_CAP alone decides the chunking."""
         L = N.lib()
         h = self._ensure_handle(device)
         need = L.sapcu_model_workspace_bytes(h, S, M)
         one = L.sapcu_model_workspace_bytes(h, 1, M)
         want = max(one, min(need, self.WORKSPACE_CAP))
-        if self._ws is None or self._ws.numel() < want or self._ws.device != device:
-            self._ws = None
-            self._ws = torch.empty(want, dtype=torch.uint8, device=device)
-        return self._ws
+        owner = self._root()
+        key = (device.index, torch.cuda.current_stream(device).cuda_stream)
+        with owner._lock:
+            ws = owner._workspaces.get(key)
+            if ws is None or ws.numel() < want:
+                owner._workspaces.pop(key, None)
+                ws = torch.empty(want, dtype=torch.uint8, device=device)
+                owner._workspaces[key] = ws
+        self._ws_last = ws
+        return ws, want
 
     def _prep_input(self, x):
         if not x.is_cuda:

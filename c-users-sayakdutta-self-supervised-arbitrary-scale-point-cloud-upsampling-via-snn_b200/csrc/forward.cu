@@ -516,6 +516,12 @@ int check_common(const sapcu_model* m, int kind, const float* patches, int64_t S
   SAPCU_REQUIRE(m, "forward: null model");
   SAPCU_REQUIRE(m->kind == kind, "forward: model kind %d used with the wrong entry point", m->kind);
   if (!m->finalized) { set_error("forward: model not finalized"); return SAPCU_ESTATE; }
+  int cur = -1;
+  SAPCU_CUDA_CHECK(cudaGetDevice(&cur));
+  if (cur != m->device) {     // the weights are another GPU's memory: refuse before any launch
+    set_error("forward: model handle was finalized on CUDA device %d, but device %d is current", m->device, cur);
+    return SAPCU_ESTATE;
+  }
   SAPCU_REQUIRE(S >= 0 && M >= 1 && M <= 128, "forward: need S >= 0 and 1 <= M <= 128 (got S=%lld M=%d)", (long long)S, M);
   SAPCU_REQUIRE(S == 0 || (patches && out && ws), "forward: null pointer");
   const int amode = mode & 0xFF;

@@ -324,6 +324,7 @@ int sapcu_model_finalize(sapcu_model* m) {
     set_error("model_finalize: no CUDA device (this library has no CPU fallback)");
     return SAPCU_ECUDA;
   }
+  SAPCU_CUDA_CHECK(cudaGetDevice(&m->device));
   const size_t n = (B.blob.size() + 63) / 64 * 64;
   B.blob.resize(n);
   SAPCU_CUDA_CHECK(cudaMalloc(&m->dev, n * sizeof(float)));
@@ -337,7 +338,13 @@ int sapcu_model_finalize(sapcu_model* m) {
 
 void sapcu_model_destroy(sapcu_model* m) {
   if (!m) return;
-  if (m->dev) cudaFree(m->dev);
+  if (m->dev) {
+    // free on the device the weights live on, whichever device the caller has current, and leave the caller's device as it was
+    int cur = -1;
+    const bool other = cudaGetDevice(&cur) == cudaSuccess && cur != m->device && cudaSetDevice(m->device) == cudaSuccess;
+    cudaFree(m->dev);
+    if (other) cudaSetDevice(cur);
+  }
   delete m;
 }
 

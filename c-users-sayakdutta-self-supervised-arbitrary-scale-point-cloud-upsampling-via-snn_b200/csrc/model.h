@@ -51,6 +51,7 @@ struct sapcu_model {
   std::vector<int> cfg;
   std::map<std::string, std::vector<float>> host;   // raw state_dict tensors (host fp32)
   bool finalized = false;
+  int device = -1;                                   // CUDA device current at finalize: the one `dev` lives on
   float* dev = nullptr;                              // one device allocation holding every derived array
   size_t dev_floats = 0;
   sapcu::FnNet fn;

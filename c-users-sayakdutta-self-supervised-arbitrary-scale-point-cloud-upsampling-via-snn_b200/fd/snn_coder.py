@@ -116,9 +116,9 @@ class EnhancedSNNDistanceEstimation(NativeModel):
         if S:
             with torch.cuda.device(x.device):        # weights, workspace, stream and launches all on the input's device
                 h = self._ensure_handle(x.device)
-                ws = self._workspace(S, M, x.device)
+                ws, ws_bytes = self._workspace(S, M, x.device)
                 if forced_idx is not None:
                     forced_idx = forced_idx.to(device=x.device, dtype=torch.int32).contiguous()
-                N.check(N.lib().sapcu_fd_forward(h, N.ptr(x), S, M, N.ptr(out), N.ptr(forced_idx), N.ptr(ws), ws.numel(),
+                N.check(N.lib().sapcu_fd_forward(h, N.ptr(x), S, M, N.ptr(out), N.ptr(forced_idx), N.ptr(ws), ws_bytes,
                                                  self.mode, N.stream_ptr(x.device)), "sapcu_fd_forward")
         return out.view(*lead) if lead else out

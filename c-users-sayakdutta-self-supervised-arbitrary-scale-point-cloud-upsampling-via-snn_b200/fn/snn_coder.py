@@ -119,7 +119,7 @@ class ImprovedSNNNormalEstimation(NativeModel):
         if S:
             with torch.cuda.device(x.device):        # weights, workspace, stream and launches all on the input's device
                 h = self._ensure_handle(x.device)
-                ws = self._workspace(S, M, x.device)
-                N.check(N.lib().sapcu_fn_forward(h, N.ptr(x), S, M, N.ptr(out), N.ptr(ws), ws.numel(), self.mode | (int(_stop_after_block) << 8),
+                ws, ws_bytes = self._workspace(S, M, x.device)
+                N.check(N.lib().sapcu_fn_forward(h, N.ptr(x), S, M, N.ptr(out), N.ptr(ws), ws_bytes, self.mode | (int(_stop_after_block) << 8),
                                                  N.stream_ptr(x.device)), "sapcu_fn_forward")
         return out.view(*lead, 3) if lead else out

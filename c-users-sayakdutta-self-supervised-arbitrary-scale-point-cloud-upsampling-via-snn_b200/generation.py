@@ -10,13 +10,19 @@ second KDTree query, per-seed Rodrigues python loop, fd forward, `seed + n*d`) b
 The kNN is computed once (the reference queries the same tree twice with identical results) and nothing
 round-trips through the host between stages.  Seeds come from `./dense` exactly as in the reference unless the
 caller injects them with `seeds=` (needed for synthetic benchmarks; SURVEY.md section 8b).
+
+`device` may also be a sequence of devices: the flat seed list is then split with `sharding.shard_bounds` (the split of the
+torch.distributed path), every shard runs the same pipeline on its device in a host thread of its own, and the results are
+gathered in shard order.  A repeated device is one more worker on that device, with its own stream.
 """
 import os
+import threading
 
 import numpy as np
 import torch
 
 from . import _native as N
+from .sharding import shard_batch_offsets, shard_bounds
 
 
 def rotation_matrix_from_vectors(vec1, vec2):
@@ -65,7 +71,10 @@ class Generator3D6(object):
     def __init__(self, model1, model2, device, k_neighbors=100, dense_spacing=0.004,
                  outlier_threshold=1.5, batch_size=400, seeds_per_pass=None, remove_outliers=True, seed_source="gpu"):
         self.model1, self.model2 = model1, model2          # fn (normals), fd (distances)
-        self.device = torch.device(device)
+        self.devices = [torch.device(d) for d in ([device] if isinstance(device, (str, int, torch.device)) else device)]
+        if not self.devices:
+            raise ValueError("Generator3D6: empty device list")
+        self.device = self.devices[0]                      # primary device: seeds, outlier filter, gathered results
         self.k_neighbors = k_neighbors
         self.dense_spacing = dense_spacing
         self.outlier_threshold = outlier_threshold
@@ -77,6 +86,7 @@ class Generator3D6(object):
         self.model1.eval()
         self.model2.eval()
         self._bufs = {}
+        self._streams = {}                                 # worker index -> its stream (several devices only)
 
     # ------------------------------------------------------------------ reference API
     def upsample(self, data, seeds=None):
@@ -113,6 +123,8 @@ class Generator3D6(object):
         h_cloud.copy_(torch.from_numpy(np.ascontiguousarray(cloud)))
         h_seeds = self._pinned("seeds", seeds.shape, torch.float64)
         h_seeds.copy_(torch.from_numpy(seeds))
+        if len(self.devices) > 1 and seeds.shape[0]:
+            return self._displace_host_sharded(h_cloud, h_seeds, batch)
         d_cloud = h_cloud.to(self.device, non_blocking=True)
         d_seeds = h_seeds.to(self.device, non_blocking=True)
         d_out = self.displace_device(d_cloud, d_seeds, batch=batch)
@@ -127,7 +139,14 @@ class Generator3D6(object):
     def displace_device(self, d_cloud, d_seeds, return_parts=False, batch=None, sort=True):
         """Device-resident pipeline: cloud [N,3] f64, seeds [S,3] f64 (cuda) -> [S,3] f64 (cuda).
         batch = (cloud_off, seed_off): host prefix tables ([B+1] ints) when d_cloud / d_seeds are the concatenation of
-        B independent (cloud, seed set) problems -- one batched kNN launch, then the same per-seed pipeline."""
+        B independent (cloud, seed set) problems -- one batched kNN launch, then the same per-seed pipeline.
+        With several devices the seeds are sharded over them and the results (with return_parts: also idx, normals, dist)
+        are gathered on the primary device; with one device everything stays on the inputs' device."""
+        if len(self.devices) > 1 and d_seeds.shape[0]:
+            return self._displace_device_sharded(d_cloud, d_seeds, return_parts, batch, sort)
+        return self._displace_local(d_cloud, d_seeds, return_parts, batch, sort)
+
+    def _displace_local(self, d_cloud, d_seeds, return_parts=False, batch=None, sort=True):
         L = N.lib()
         K = self.k_neighbors
         Ncl, S = d_cloud.shape[0], d_seeds.shape[0]
@@ -136,7 +155,7 @@ class Generator3D6(object):
             # large clouds: visit the seeds along a Morton curve (results are per-seed, so only the order of the work changes)
             with torch.cuda.device(dev):
                 perm = morton_order(d_seeds)
-                res = self.displace_device(d_cloud, d_seeds[perm].contiguous(), sort=False)
+                res = self._displace_local(d_cloud, d_seeds[perm].contiguous(), sort=False)
                 out = torch.empty_like(res)
                 out[perm] = res
             return out
@@ -176,6 +195,83 @@ class Generator3D6(object):
         if return_parts:
             return out, idx, normals, dist
         return out
+
+    # ------------------------------------------------------------------ several devices in one process
+    def _run_shards(self, S, work, after=None):
+        """work(device, lo, hi) for every entry of self.devices and its seed range shard_bounds(S, n)[i], each in a host thread of
+        its own (created here, always joined) with its device current and its own stream as the current stream.  `after`: an
+        event every worker stream waits for before its first launch.  Returns (results in shard order, streams); an exception in
+        a worker is raised here once every worker has finished."""
+        n = len(self.devices)
+        for d in self.devices:
+            if d.type != "cuda":
+                raise N.SapcuError("Generator3D6 needs CUDA devices (no CPU fallback); got %s" % d)
+        for i in range(n):
+            if i not in self._streams:
+                self._streams[i] = torch.cuda.Stream(device=self.devices[i])
+        streams = [self._streams[i] for i in range(n)]
+        results, errors = [None] * n, [None] * n
+
+        def run(i, lo, hi):
+            try:
+                with torch.no_grad(), torch.cuda.device(streams[i].device), torch.cuda.stream(streams[i]):
+                    if after is not None:
+                        streams[i].wait_event(after)
+                    results[i] = work(streams[i].device, lo, hi) if hi > lo else None
+            except BaseException as e:      # noqa: BLE001 -- re-raised in the caller below
+                errors[i] = e
+
+        threads = [threading.Thread(target=run, args=(i, lo, hi), name="Generator3D6-%d" % i)
+                   for i, (lo, hi) in enumerate(shard_bounds(S, n))]
+        for t in threads:
+            t.start()
+        for t in threads:
+            t.join()
+        for e in errors:
+            if e is not None:
+                raise e
+        return results, streams
+
+    def _displace_device_sharded(self, d_cloud, d_seeds, return_parts, batch, sort):
+        def work(dev, lo, hi):
+            b = None if batch is None else (batch[0], shard_batch_offsets(batch[1], lo, hi))
+            c = d_cloud.to(dev, non_blocking=True)                     # the cloud is replicated to every device
+            s = d_seeds[lo:hi].to(dev, non_blocking=True).contiguous()
+            res = self._displace_local(c, s, return_parts, b, sort)
+            return res if return_parts else (res,)
+
+        ready = torch.cuda.Event()
+        ready.record(torch.cuda.current_stream(d_seeds.device))            # the inputs are complete on the caller's stream
+        parts, streams = self._run_shards(d_seeds.shape[0], work, after=ready)
+        parts = [p for p in parts if p is not None]
+        home = torch.cuda.current_stream(self.device)
+        for st in streams:
+            home.wait_stream(st)
+        for p in parts:
+            for t in p:      # made on a worker stream, read by the gather on the caller's stream of its device
+                t.record_stream(torch.cuda.current_stream(t.device))
+        with torch.cuda.device(self.device):
+            out = tuple(torch.cat([p[j].to(self.device, non_blocking=True) for p in parts]) for j in range(len(parts[0])))
+        return out if return_parts else out[0]
+
+    def _displace_host_sharded(self, h_cloud, h_seeds, batch):
+        """displace_host over several devices: every worker copies the pinned cloud and its seed rows to its device, runs the
+        pipeline, copies its points into its rows of one pinned output and synchronises its stream.  Only this (calling)
+        thread allocates and fills the pinned buffers, so the workers never race on them."""
+        h_out = self._pinned("out", tuple(h_seeds.shape), torch.float64)
+
+        def work(dev, lo, hi):
+            b = None if batch is None else (batch[0], shard_batch_offsets(batch[1], lo, hi))
+            c = h_cloud.to(dev, non_blocking=True)
+            s = h_seeds[lo:hi].to(dev, non_blocking=True)
+            h_out[lo:hi].copy_(self._displace_local(c, s, batch=b), non_blocking=True)
+            torch.cuda.current_stream(dev).synchronize()
+
+        _, streams = self._run_shards(h_seeds.shape[0], work)
+        for d in dict.fromkeys(st.device for st in streams):
+            with torch.cuda.device(d):
+                N.check_device("displace_host")
+        return h_out.numpy().copy()
 
     def upsample_batch(self, clouds, seeds):
         """A batch of independent clouds in one device pipeline (the per-file loop of the reference's generate.py:135-160

@@ -32,7 +32,7 @@ extern "C" {
 #define SAPCU_EINVAL       -1   /* bad argument (shape, null pointer, unsupported size) */
 #define SAPCU_ECUDA        -2   /* a CUDA runtime call or kernel launch failed */
 #define SAPCU_EWORKSPACE   -3   /* workspace too small for even one patch */
-#define SAPCU_ESTATE       -4   /* model not finalized / missing tensor */
+#define SAPCU_ESTATE       -4   /* model not finalized / missing tensor / handle used on another device */
 
 #define SAPCU_MODEL_FN      0   /* ImprovedSNNNormalEstimation   (fn/snn_coder.py:627) */
 #define SAPCU_MODEL_FD      1   /* EnhancedSNNDistanceEstimation (fd/snn_coder.py:805) */
@@ -158,7 +158,10 @@ int sapcu_fps(const float* d_xyz, int64_t N, int64_t npoint, int64_t start, int3
  * After finalize the handle is immutable (weights, folded parameters, LIF tables) and may be used from several host
  * threads / streams concurrently, each call with its own workspace; per-device kernel attributes and the watchdog flag are
  * set up under a lock on first use of a device, the A/B environment switches are read once per process.  A handle's
- * weights live on the CUDA device that was current at finalize.
+ * weights live on the CUDA device that was current at finalize, and the handle records that device:
+ * sapcu_fn_forward / sapcu_fd_forward return SAPCU_ESTATE, before any launch, when another device is current, and
+ * sapcu_model_destroy frees on the recorded device and leaves the caller's current device unchanged.  One handle per
+ * device: finalize a separate handle for every GPU that runs the model.
  * ---------------------------------------------------------------------------------- */
 typedef struct sapcu_model sapcu_model;
 
