@@ -99,7 +99,8 @@ struct G {
   int mode; cudaStream_t st;
   mutable const char* lab = nullptr;                       // profiler label of the next launch: g.L("fn.fc1").layer(...)
   const G& L(const char* l) const { lab = l; return *this; }
-  int run(GemmArgs& g, int amode) const {
+  int passes() const { return mode == SAPCU_MODE_TF32 || mode == SAPCU_MODE_FAST ? 1 : 3; }   // tensor-core products per MAC
+  int run(GemmArgs g, int amode) const {
     if (lab) { g.label = lab; lab = nullptr; }
     int slot = -1;
     ProfWork w;
@@ -113,7 +114,7 @@ struct G {
     }
     const bool prof = prof_begin(st, g.label, w, &slot);
     int rc;
-    g.tc_passes = (mode == SAPCU_MODE_TF32 || mode == SAPCU_MODE_FAST) ? 1 : 3;
+    g.tc_passes = passes();
     // fast mode, plain point-level contractions: single-pass TF32 needs no operand split -> the compact-stage flavour
     if (mode == SAPCU_MODE_FAST && amode == A_PLAIN && g.act == ACT_NONE && !g.residual && !g.at_pos && !g.pool && !g.x_h2 && !g.out_h2 && !g.edge_bias) g.fast = true;
     if (mode != SAPCU_MODE_FP32 && gemm_tc2_supported(g, amode)) rc = launch_gemm_tc2(g, st);
@@ -129,7 +130,7 @@ struct G {
     g.A = X; g.lda = lda; g.R = R; g.K = L.K; g.W = L.W; g.Whi = L.Whi; g.Wlo = L.Wlo; g.N = L.N; g.bias = L.bias; g.scale = L.scale; g.shift = L.shift;
     g.Wh = L.Wh; g.Wl = L.Wl; g.winv = L.winv; g.x_unit = x_unit;
     g.act = act; g.T = T; g.nparams = nr ? nr->np : nullptr; g.residual = res; g.ldr = ldr; g.Y = Y; g.ldc = ldc;
-    g.tc_passes = (mode == SAPCU_MODE_TF32 || mode == SAPCU_MODE_FAST) ? 1 : 3;
+    g.tc_passes = passes();
     if (mode == SAPCU_MODE_FAST && act == ACT_LIF && nr) {     // point-level LIF layers: compact single-pass TF32 stages + the layer's LIF table
       g.fast = true;
       if (settings().fast_tables && nr->tab_ok && nr->tab_T == T) { g.lif_tab = nr->tab; g.lif_tab_stride = nr->tab_stride; }
@@ -143,15 +144,27 @@ struct G {
   }
 };
 
-// The storage format of the tapped spike tensors (0 fp32, 1 fp16 (hi, lo) planes, 2 one fp16 plane) is recorded in the
-// handle by every forward (sapcu_model::tap_*): debug information for the parity tests, relaxed atomics.
+// The storage format of the tapped spike tensors (0 fp32, 1 fp16 (hi, lo) planes of x * 2^13, 2 one fp16 plane) is recorded
+// in the handle by every forward (sapcu_model::tap_*): debug information for the parity tests, relaxed atomics.
 
 #define SAPCU_TRY(expr) do { int _rc = (expr); if (_rc) return _rc; } while (0)
 
+// One fn block's hand-over formats, in the tap codes above, and the LIF tables and fusions that go with them. plan() in
+// fn_chunk fills it before the block's first launch; the launch sequence reads nothing else.
+struct BlockPlan {
+  int x_planes = 0;      // fc1 -> q/k/v
+  int delta = 0;         // pos-enc layer 1 -> fc_delta2
+  int pos = 0;           // pos (fc_delta2's spikes) -> fc_gamma and the attention tail
+  bool pos32 = false;    // fc_delta2 also writes pos in fp32 (E3), and the attention tail reads that copy
+  int gamma = 0;         // fc_gamma -> fc_gamma2
+  // LIF chains read from the layer's table (in the fast mode fc1 and q/k/v take theirs in G::args, as every point-level layer)
+  bool tab_fc1 = false, tab_qkv = false, tab_delta = false, tab_delta2 = false, tab_gamma = false;
+  bool attn_in = false;  // factorised attention input: [W q | W k] per point + fc_gamma's edge-bias epilogue
+  bool attn_out = false; // fc_gamma2 with the fused softmax + weighted-sum tail
+};
+
 int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* normals, const FnPlan& p, int mode, int stop_block, cudaStream_t st) {
   const FnNet& f = mdl->fn;
-  int g_tap_gamma_h2 = 0, g_tap_delta2_h2 = 0, g_tap_snn1_h2 = 0;
-  struct TapPublish { const sapcu_model* m; int* g; int* d; int* x; ~TapPublish() { m->tap_gamma.store(*g, std::memory_order_relaxed); m->tap_delta2.store(*d, std::memory_order_relaxed); m->tap_snn1.store(*x, std::memory_order_relaxed); } } tap_publish{mdl, &g_tap_gamma_h2, &g_tap_delta2_h2, &g_tap_snn1_h2};
   const int64_t P = s * M;
   const bool precise = mode == SAPCU_MODE_FP32;
   const G g{mode, st};
@@ -161,49 +174,9 @@ int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
   { ProfWork w; w.elsteps = (double)P * 64 * f.T_enc; w.bytes = (double)P * (12 + 256);
     SAPCU_PROF(st, "fn.conv1+lif", w, launch_pointwise3_lif(false, precise, xyz, nullptr, 0, 0, M, P, 64, f.conv1.W, f.conv1.bias, f.conv1.scale,
                                   f.conv1.shift, f.snn_init.np, f.T_enc, p.F0, st)); }
-  // ---- tensor-core schedule helpers ------------------------------------------------------------------------------
-  // fc_gamma's first layer is linear, so W(q_i - k_j + pos_ij) = W q_i - W k_j + W pos_ij: the edge contraction runs on
-  // pos (E2) alone and its epilogue adds the two per-POINT products [W q | W k] (QK, [P, 2D]) gathered through the graph
-  // before BN + LIF; fc_gamma2's epilogue does the softmax over k and the weighted sum.  Neither the attention input nor
-  // the logits are materialised.
-  auto gamma_args = [&](int b, const float* pos, float* out, float* QK) {
-    const FnBlock& k = f.blk[b];
-    const int D = k.D, kk = k.k < M ? k.k : M;
-    GemmArgs a;
-    const Layer& L = k.fc_gamma;
-    a.A = pos; a.lda = D; a.R = P * kk; a.K = D; a.W = L.W; a.Whi = L.Whi; a.Wlo = L.Wlo; a.N = D;
-    a.bias = L.bias; a.scale = L.scale; a.shift = L.shift; a.act = ACT_LIF; a.T = 4; a.nparams = k.snn_gamma.np;
-    a.Y = out; a.ldc = D;
-    a.Q = QK; a.Kf = QK + D; a.ldq = 2 * D; a.idx = p.idx; a.ldi = p.kmax; a.kk = kk; a.Mpts = M; a.edge_bias = true;
-    a.Wh = L.Wh; a.Wl = L.Wl; a.winv = L.winv; a.x_unit = true;                     // pos is a LIF output
-    return a;
-  };
-  auto gamma2_args = [&](int b, const float* in, const float* pos) {
-    const FnBlock& k = f.blk[b];
-    const int D = k.D, kk = k.k < M ? k.k : M;
-    GemmArgs a;
-    const Layer& L = k.fc_gamma2;
-    a.A = in; a.lda = D; a.R = P * kk; a.K = D; a.W = L.W; a.Whi = L.Whi; a.Wlo = L.Wlo; a.N = D;
-    a.bias = L.bias; a.scale = L.scale; a.shift = L.shift; a.act = ACT_NONE;
-    a.idx = p.idx; a.ldi = p.kmax; a.kk = kk; a.Mpts = M;
-    a.idx8 = mode != SAPCU_MODE_FP32 ? p.idx8 : nullptr; a.ldi8w = (p.kmax + 3) / 4;
-    a.at_pos = pos; a.at_v = p.QKV + 2 * D; a.at_ldv = 3 * D; a.at_sqrt = sqrtf((float)(D / f.heads));   // torch divides by the python scalar sqrt(head_dim)
-    a.Y = p.RES; a.ldc = D;
-    a.Wh = L.Wh; a.Wl = L.Wl; a.winv = L.winv; a.x_unit = true;                     // fc_gamma's LIF output
-    a.tc_passes = (mode == SAPCU_MODE_TF32 || mode == SAPCU_MODE_FAST) ? 1 : 3;
-    return a;
-  };
-  auto edge_pos = [&](int b, float* out, cudaStream_t s_, int nsplit, bool h2) {
-    const FnBlock& k = f.blk[b];
-    const int kk = k.k < M ? k.k : M;
-    ProfWork w; w.elsteps = (double)P * kk * k.D * 4; w.bytes = (double)P * kk * k.D * 4.0;
-    SAPCU_PROF(s_, "fn.fc_delta(K=3)+lif (edge_pos_lif)", w,
-               launch_pointwise3_lif(true, precise, xyz, p.idx, kk, p.kmax, M, P * kk, k.D, k.fc_delta.W, k.fc_delta.bias,
-                                     k.fc_delta.scale, k.fc_delta.shift, k.snn_delta.np, 4, out, s_, nsplit, h2));
-    return 0;
-  };
-  const bool factorise = settings().factor_attnin;
   const bool use_tables = settings().fast_tables;       // 0: reduced-MUFU chains (A/B)
+  auto fits = [](const Neuron& n, uint32_t budget) { return n.tab_ok && n.tab_T == 4 && n.tab_stride <= budget; };
+  auto sup2 = [](const GemmArgs& a) { return gemm_tc2_supported(a, A_PLAIN); };
   for (int b = 0; b < 3; ++b) {
     if (stop_block && b >= stop_block) return 0;            // debug: leave block `stop_block`'s intermediates in the workspace
     const FnBlock& k = f.blk[b];
@@ -211,171 +184,150 @@ int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
     const float* fin = b == 0 ? p.F0 : p.FCAT + 64 * (b - 1);
     const int64_t ldin = b == 0 ? 64 : 192;
     const int64_t E = P * kk;
-    float* Xb = p.E1;                                             // this block's edge buffer (pos-enc layer 1, then fc_gamma's output)
-    bool xb_h2 = false, e2_h2 = false, pos32 = false;             // fc_gamma's output / pos stored as fp16 planes (see below); + fp32 copy of pos
-    {
-      // Parity-grade mode, wide blocks: fc1's spikes have ONE reader, the q/k/v contraction -> handed over as fp16 (hi, lo)
-      // planes in the bytes of the fp32 tensor; q/k/v then runs fp16x3 products (the 22-bit products of 3xTF32 at twice the
-      // tensor rate, no splitter pass) and reads its LIF^T chains from the layer's table when it fits next to two stages.
-      GemmArgs a1 = g.args(k.fc1, fin, ldin, P, p.X, D, ACT_LIF, &k.snn1, 4);
-      GemmArgs a2 = g.args(k.qkv, p.X, D, P, p.QKV, 3 * D, ACT_LIF, &k.snn_qkv, 4);
-      bool x_planes = false;
+    const float sq = sqrtf((float)(D / f.heads));           // torch divides the logits by the python scalar sqrt(head_dim)
+    // ---- the contractions whose operand formats the plan chooses: one builder each, used to probe and to launch
+    auto fc1_args = [&](const BlockPlan& q) {
+      GemmArgs a = g.args(k.fc1, fin, ldin, P, p.X, D, ACT_LIF, &k.snn1, 4);
+      a.out_h2 = a.tc2_any_rows = q.x_planes != 0;
+      if (q.tab_fc1) { a.lif_tab = k.snn1.tab; a.lif_tab_stride = k.snn1.tab_stride; }
+      return a;
+    };
+    auto qkv_args = [&](const BlockPlan& q) {
+      GemmArgs a = g.args(k.qkv, p.X, D, P, p.QKV, 3 * D, ACT_LIF, &k.snn_qkv, 4, nullptr, 0, q.x_planes != 0);
+      a.x_h2 = a.tc2_any_rows = q.x_planes != 0;
+      if (q.tab_qkv) { a.lif_tab = k.snn_qkv.tab; a.lif_tab_stride = k.snn_qkv.tab_stride; }
+      return a;
+    };
+    // per-edge contractions on LIF outputs: input format `in` (2 = the fast mode's single-product path), LIF output format `out`
+    auto edge = [](GemmArgs a, int in, int out, const Neuron* n, bool tab) {
+      a.x_h2 = in != 0; a.out_h2 = out != 0; a.fast = in == 2;
+      a.lif_tab = tab ? n->tab : nullptr; a.lif_tab_stride = tab ? n->tab_stride : 0;
+      return a;
+    };
+    auto delta2_args = [&](const BlockPlan& q) {
+      GemmArgs a = edge(g.args(k.fc_delta2, p.E1, D, E, p.E2, D, ACT_LIF, &k.snn_delta2, 4, nullptr, 0, true), q.delta, q.pos,
+                        &k.snn_delta2, q.tab_delta2);
+      a.Y2 = q.pos32 ? p.E3 : nullptr;
+      return a;
+    };
+    // fc_gamma's first layer is linear, so W(q_i - k_j + pos_ij) = W q_i - W k_j + W pos_ij: the edge contraction runs on
+    // pos (E2) alone and its epilogue adds the two per-POINT products [W q | W k] (QK, [P, 2D]) gathered through the graph
+    // before BN + LIF; fc_gamma2's epilogue does the softmax over k and the weighted sum.  Neither the attention input nor
+    // the logits are materialised.
+    auto gamma_args = [&](const BlockPlan& q) {
+      GemmArgs a = edge(g.args(k.fc_gamma, p.E2, D, E, p.E1, D, ACT_LIF, &k.snn_gamma, 4, nullptr, 0, true), q.pos, q.gamma,
+                        &k.snn_gamma, q.tab_gamma);
+      a.Q = p.QK; a.Kf = p.QK + D; a.ldq = 2 * D; a.idx = p.idx; a.ldi = p.kmax; a.kk = kk; a.Mpts = M; a.edge_bias = true;
+      return a;
+    };
+    auto gamma2_args = [&](const BlockPlan& q) {
+      GemmArgs a = edge(g.args(k.fc_gamma2, p.E1, D, E, p.RES, D, ACT_NONE, nullptr, 0, nullptr, 0, true), q.gamma, 0, nullptr, false);
+      a.idx = p.idx; a.ldi = p.kmax; a.kk = kk; a.Mpts = M; a.idx8 = p.idx8; a.ldi8w = (p.kmax + 3) / 4;
+      a.at_pos = q.pos32 ? p.E3 : p.E2; a.pos_h2 = q.pos != 0 && !q.pos32;
+      a.at_v = p.QKV + 2 * D; a.at_ldv = 3 * D; a.at_sqrt = sq;
+      return a;
+    };
+    // ---- the plan: asks the engines, in dependency order, which formats each producer / consumer pair takes; launches nothing
+    auto plan = [&]() {
+      BlockPlan q;
+      if (mode == SAPCU_MODE_FP32) return q;
       if (mode == SAPCU_MODE_TC) {
-        GemmArgs t1 = a1, t2 = a2;
-        t1.out_h2 = true; t2.x_h2 = true; t2.x_unit = true; t1.tc2_any_rows = t2.tc2_any_rows = true;
-        x_planes = D % 256 == 0 && gemm_tc2_supported(t1, A_PLAIN) && gemm_tc2_supported(t2, A_PLAIN) && gemm_tc2_fp16x3(t2);
-        if (x_planes) {
-          a1 = t1; a2 = t2;
-          if (k.snn_qkv.tab_ok && k.snn_qkv.tab_T == 4 && k.snn_qkv.tab_stride <= LT_SMEM_BUDGET_TC) {
-            a2.lif_tab = k.snn_qkv.tab; a2.lif_tab_stride = k.snn_qkv.tab_stride;
-          }
-          // fc1 itself keeps 3xTF32 products (its input is not a spike tensor) and reads its chain from the table as well
-          if (k.snn1.tab_ok && k.snn1.tab_T == 4 && k.snn1.tab_stride <= LT_SMEM_BUDGET_TC) {
-            a1.lif_tab = k.snn1.tab; a1.lif_tab_stride = k.snn1.tab_stride;
-          }
-        }
+        // Parity-grade mode, wide blocks: fc1's spikes have ONE reader, the q/k/v contraction -> handed over as fp16 (hi, lo)
+        // planes in the bytes of the fp32 tensor; q/k/v then runs fp16x3 products (the 22-bit products of 3xTF32 at twice the
+        // tensor rate, no splitter pass) and reads its LIF^T chains from the layer's table when it fits next to two stages.
+        // fc1 itself keeps 3xTF32 products (its input is not a spike tensor) and reads its chain from the table as well.
+        q.x_planes = 1;
+        const GemmArgs a1 = fc1_args(q), a2 = qkv_args(q);
+        q.x_planes = D % 256 == 0 && sup2(a1) && sup2(a2) && gemm_tc2_fp16x3(a2);
+        q.tab_fc1 = q.x_planes && fits(k.snn1, LT_SMEM_BUDGET_TC);
+        q.tab_qkv = q.x_planes && fits(k.snn_qkv, LT_SMEM_BUDGET_TC);
       }
-      g_tap_snn1_h2 = x_planes ? 1 : 0;
-      SAPCU_TRY(g.L("fn.fc1+lif").run(a1, A_PLAIN));
-      SAPCU_TRY(g.L("fn.qkv+lif").run(a2, A_PLAIN));
+      const bool factorise = settings().factor_attnin && kk >= 2;
+      if (mode == SAPCU_MODE_FAST && factorise) {
+        // Fast schedule: every per-edge spike tensor of the block is ONE fp16 plane of x * 2^13, every edge contraction one fp16
+        // product per MAC (2-CTA kernel, HM = 3), every LIF^T chain a table lookup where the layer's table fits shared memory.
+        BlockPlan t = q;
+        t.delta = t.pos = t.gamma = 2;
+        t.attn_in = t.attn_out = true;
+        t.tab_delta = use_tables && fits(k.snn_delta, LT_SMEM_BUDGET);
+        t.tab_delta2 = use_tables && fits(k.snn_delta2, LT_SMEM_BUDGET);
+        t.tab_gamma = use_tables && fits(k.snn_gamma, LT_SMEM_BUDGET);
+        const GemmArgs a = delta2_args(t), a1 = gamma_args(t), a2 = gamma2_args(t);
+        if (sup2(a) && gemm_tc2_fast(a) && sup2(a1) && gemm_tc2_fast(a1) && sup2(a2) && gemm_tc2_fast(a2)) return t;
+      }
+      // Parity-grade mode with tabulated LIF^T chains: the three per-edge LIF layers of a block whose tables fit next to two
+      // pipeline stages read their chains from the tables (lif_table.cuh, |error| <= 4e-5, far inside the spike tolerance); all
+      // three edge tensors are then handed over as fp16 (hi, lo) planes.  Without the tables pos stays fp32 (measured slower as
+      // planes: the attention tail then issues two 2-byte loads per operand instead of one 4-byte load).
+      const bool blk_tab = mode == SAPCU_MODE_TC && factorise && fits(k.snn_delta, LT_SMEM_BUDGET) &&
+                           fits(k.snn_delta2, LT_SMEM_BUDGET_TC) && fits(k.snn_gamma, LT_SMEM_BUDGET_TC);
+      // fc_delta2 on the pos-enc layer-1 spikes: planes of x * 2^13 (same bytes as fp32) when it runs on the fp16x3 path,
+      // which loads them without converting (128-channel layers run on the 2-CTA engine only from planes)
+      q.delta = 1;
+      const GemmArgs a = delta2_args(q);
+      q.delta = sup2(a) && gemm_tc2_fp16x3(a);
+      // pos has two readers, fc_gamma's contraction and the fused attention tail: planes when both take them
+      q.pos = q.gamma = 1;
+      const GemmArgs a1 = gamma_args(q), a2 = gamma2_args(q);
+      q.pos = blk_tab && q.delta && sup2(a1) && gemm_tc2_fp16x3(a1) && sup2(a2) && gemm_tc2_fp16x3(a2);
+      // the whole chain of plane hand-overs is in place: its producers read their tables, and the attention tail, which gathers
+      // pos per edge, prefers one 4-byte load over two 2-byte loads -- with the table-driven (ALU-bound) epilogue the extra
+      // fp32 store is free
+      q.pos32 = q.tab_delta = q.tab_delta2 = q.pos;
+      // fc_gamma's spikes go to fc_gamma2 only: planes when both run on the 2-CTA fp16x3 path
+      const GemmArgs b1 = gamma_args(q), b2 = gamma2_args(q);
+      q.gamma = factorise && sup2(b1) && sup2(b2) && gemm_tc2_fp16x3(b2);
+      q.tab_gamma = blk_tab && q.pos && q.gamma;
+      const GemmArgs c1 = gamma_args(q), c2 = gamma2_args(q);
+      q.attn_in = factorise && (sup2(c1) || gemm_tc_supported(c1, A_PLAIN));
+      q.attn_out = sup2(c2) || gemm_tc_supported(c2, A_PLAIN);
+      return q;
+    };
+    const BlockPlan q = plan();
+    mdl->tap_snn1.store(q.x_planes, std::memory_order_relaxed);
+    mdl->tap_delta2.store(q.pos, std::memory_order_relaxed);
+    mdl->tap_gamma.store(q.gamma, std::memory_order_relaxed);
+    // ---- the block's launches
+    SAPCU_TRY(g.L("fn.fc1+lif").run(fc1_args(q), A_PLAIN));
+    SAPCU_TRY(g.L("fn.qkv+lif").run(qkv_args(q), A_PLAIN));
+    {   // pos-enc layer 1 (fc_delta, K = 3) into E1: edge_pos_lif_fast writes one plane, or (hi, lo) planes from the table
+      const Neuron& n = k.snn_delta;
+      ProfWork w; w.elsteps = (double)E * D * 4; w.bytes = (double)E * D * (q.delta == 2 ? 2.0 : 4.0);
+      SAPCU_PROF(st, "fn.fc_delta(K=3)+lif (edge_pos_lif)", w, q.delta == 2 || q.tab_delta
+          ? launch_edge_pos_lif_fast(xyz, p.idx, kk, p.kmax, M, E, D, k.fc_delta.W, k.fc_delta.bias, k.fc_delta.scale, k.fc_delta.shift,
+                                     n.np, 4, p.E1, q.tab_delta ? n.tab : nullptr, q.tab_delta ? n.tab_stride : 0, st, q.delta == 1)
+          : launch_pointwise3_lif(true, precise, xyz, p.idx, kk, p.kmax, M, E, D, k.fc_delta.W, k.fc_delta.bias, k.fc_delta.scale,
+                                  k.fc_delta.shift, n.np, 4, p.E1, st, 1, q.delta == 1));
     }
-    if (mode == SAPCU_MODE_FP32) { g_tap_gamma_h2 = 0; g_tap_delta2_h2 = 0; SAPCU_TRY(edge_pos(b, Xb, st, 1, false)); }
-    if (mode == SAPCU_MODE_FAST) {
-      // Fast schedule: every per-edge spike tensor of the block is ONE fp16 plane of x * 2^13, every edge contraction one fp16
-      // product per MAC (2-CTA kernel, HM = 3), every LIF^T chain a table lookup where the layer's table fits shared memory.
-      GemmArgs a;
-      {
-        const Layer& L = k.fc_delta2;
-        a.A = Xb; a.lda = D; a.R = E; a.K = D; a.W = L.W; a.Whi = L.Whi; a.Wlo = L.Wlo; a.N = D;
-        a.bias = L.bias; a.scale = L.scale; a.shift = L.shift; a.act = ACT_LIF; a.T = 4; a.nparams = k.snn_delta2.np;
-        a.Y = p.E2; a.ldc = D; a.Wh = L.Wh; a.Wl = L.Wl; a.winv = L.winv; a.x_unit = true; a.tc_passes = 1;
-        a.fast = true; a.x_h2 = true; a.out_h2 = true;
-        if (use_tables && k.snn_delta2.tab_ok) { a.lif_tab = k.snn_delta2.tab; a.lif_tab_stride = k.snn_delta2.tab_stride; }
-      }
-      GemmArgs a1 = gamma_args(b, p.E2, Xb, p.QK), a2 = gamma2_args(b, Xb, p.E2);
-      a1.tc_passes = a2.tc_passes = 1;
-      a1.fast = true; a1.x_h2 = true; a1.out_h2 = true;
-      if (use_tables && k.snn_gamma.tab_ok) { a1.lif_tab = k.snn_gamma.tab; a1.lif_tab_stride = k.snn_gamma.tab_stride; }
-      a2.fast = true; a2.x_h2 = true; a2.pos_h2 = true;
-      const bool blk_fast = factorise && kk >= 2 && gemm_tc2_supported(a, A_PLAIN) && gemm_tc2_fast(a) &&
-                            gemm_tc2_supported(a1, A_PLAIN) && gemm_tc2_fast(a1) && gemm_tc2_supported(a2, A_PLAIN) && gemm_tc2_fast(a2);
-      if (blk_fast) {
-        g_tap_gamma_h2 = 2; g_tap_delta2_h2 = 2;
-        {
-          ProfWork w; w.elsteps = (double)E * D * 4; w.bytes = (double)E * D * 2.0;
-          const bool lt = use_tables && k.snn_delta.tab_ok;
-          SAPCU_PROF(st, "fn.fc_delta(K=3)+lif (edge_pos_lif)", w,
-                     launch_edge_pos_lif_fast(xyz, p.idx, kk, p.kmax, M, E, D, k.fc_delta.W, k.fc_delta.bias, k.fc_delta.scale,
-                                              k.fc_delta.shift, k.snn_delta.np, 4, Xb, lt ? k.snn_delta.tab : nullptr,
-                                              lt ? k.snn_delta.tab_stride : 0, st));
-        }
-        SAPCU_TRY(g.L("fn.fc_delta2+lif").run(a, A_PLAIN));
-        Layer Lw = k.fc_gamma;
-        Lw.bias = nullptr; Lw.scale = nullptr; Lw.shift = nullptr;
-        SAPCU_TRY(g.L("fn.fc_gamma(Wq|Wk per point)").layer(Lw, p.QKV, 3 * D, P, p.QK, 2 * D, ACT_NONE));
-        SAPCU_TRY(g.L("fn.fc_gamma(Wq|Wk per point)").layer(Lw, p.QKV + D, 3 * D, P, p.QK + D, 2 * D, ACT_NONE));
-        SAPCU_TRY(g.L("fn.fc_gamma+edge_bias+lif").run(a1, A_PLAIN));
-        SAPCU_TRY(g.L("fn.fc_gamma2+softmax+sum(attention tail)").run(a2, A_PLAIN));
-        SAPCU_TRY(g.L("fn.out_proj").layer(k.out_proj, p.RES, D, P, p.R1, D, ACT_NONE));
-        SAPCU_TRY(g.L("fn.fc2+residual").layer(k.fc2, p.R1, D, P, p.FCAT + 64 * b, 192, ACT_NONE, nullptr, 0, fin, ldin));
-        continue;
-      }
-    }
-    // Parity-grade mode with tabulated LIF^T chains: the three per-edge LIF layers of a block whose tables fit next to two
-    // pipeline stages read their chains from the tables (lif_table.cuh, |error| <= 4e-5, far inside the spike tolerance); all
-    // three edge tensors are then handed over as fp16 (hi, lo) planes.  Without the tables pos stays fp32 (measured slower as
-    // planes: the attention tail then issues two 2-byte loads per operand instead of one 4-byte load).
-    const bool blk_tab = mode == SAPCU_MODE_TC && factorise && kk >= 2 &&
-                         k.snn_delta.tab_ok && k.snn_delta2.tab_ok && k.snn_gamma.tab_ok && k.snn_delta.tab_stride <= LT_SMEM_BUDGET &&
-                         k.snn_delta2.tab_stride <= LT_SMEM_BUDGET_TC && k.snn_gamma.tab_stride <= LT_SMEM_BUDGET_TC;
-    if (mode != SAPCU_MODE_FP32) {
-      // fc_delta2 on the pos-enc layer-1 spikes.  When it runs on the fp16x3 path, edge_pos_lif hands the spikes over as
-      // fp16 (hi, lo) planes of x * 2^13 (same bytes as fp32) and the contraction loads them without converting.
-      {
-        GemmArgs a;
-        const Layer& L = k.fc_delta2;
-        a.A = Xb; a.lda = D; a.R = E; a.K = D; a.W = L.W; a.Whi = L.Whi; a.Wlo = L.Wlo; a.N = D;
-        a.bias = L.bias; a.scale = L.scale; a.shift = L.shift; a.act = ACT_LIF; a.T = 4; a.nparams = k.snn_delta2.np;
-        a.Y = p.E2; a.ldc = D; a.Wh = L.Wh; a.Wl = L.Wl; a.winv = L.winv; a.x_unit = true;   // input: LIF output
-        a.tc_passes = (mode == SAPCU_MODE_TF32 || mode == SAPCU_MODE_FAST) ? 1 : 3;
-        a.x_h2 = true;                                              // tentatively: 128-channel layers run on the 2-CTA engine only from planes
-        a.x_h2 = gemm_tc2_supported(a, A_PLAIN) && gemm_tc2_fp16x3(a);
-        {   // pos (E2) has two readers, fc_gamma's contraction and the fused attention tail: planes when both take them
-          GemmArgs a1 = gamma_args(b, p.E2, Xb, p.QK), a2 = gamma2_args(b, Xb, p.E2);
-          a1.tc_passes = a2.tc_passes = a.tc_passes;
-          a1.x_h2 = a2.x_h2 = a2.pos_h2 = true;                    // the formats this hand-over would give them
-          e2_h2 = blk_tab && a.x_h2 && factorise && kk >= 2 && gemm_tc2_supported(a, A_PLAIN) && gemm_tc2_supported(a1, A_PLAIN) &&
-                  gemm_tc2_fp16x3(a1) && gemm_tc2_supported(a2, A_PLAIN) && gemm_tc2_fp16x3(a2);
-        }
-        a.out_h2 = e2_h2;
-        g_tap_delta2_h2 = e2_h2 ? 1 : 0;
-        const bool tab_on = blk_tab && a.x_h2 && e2_h2;           // the whole chain of plane hand-overs is in place
-        // pos has two readers: fc_gamma's contraction takes the planes, the attention tail gathers it per edge and prefers one
-        // 4-byte load over two 2-byte loads -- with the table-driven (ALU-bound) epilogue the extra fp32 store is free
-        pos32 = tab_on;
-        if (pos32) a.Y2 = p.E3;
-        if (tab_on) {
-          ProfWork w; w.elsteps = (double)E * D * 4; w.bytes = (double)E * D * 4.0;
-          SAPCU_PROF(st, "fn.fc_delta(K=3)+lif (edge_pos_lif)", w,
-                     launch_edge_pos_lif_fast(xyz, p.idx, kk, p.kmax, M, E, D, k.fc_delta.W, k.fc_delta.bias, k.fc_delta.scale,
-                                              k.fc_delta.shift, k.snn_delta.np, 4, Xb, k.snn_delta.tab, k.snn_delta.tab_stride, st, true));
-          a.lif_tab = k.snn_delta2.tab; a.lif_tab_stride = k.snn_delta2.tab_stride;
-        } else {
-          SAPCU_TRY(edge_pos(b, Xb, st, 1, a.x_h2));
-        }
-        SAPCU_TRY(g.L("fn.fc_delta2+lif").run(a, A_PLAIN));
-      }
-      {
-        float* QK = p.QK;                                          // [W q | W k], [P, 2D]
-        GemmArgs a = gamma_args(b, p.E2, Xb, QK);
-        a.tc_passes = (mode == SAPCU_MODE_TF32 || mode == SAPCU_MODE_FAST) ? 1 : 3;
-        {   // fc_gamma's spikes go to fc_gamma2 only: hand them over as fp16 planes when both run on the 2-CTA fp16x3 path
-          GemmArgs a2 = gamma2_args(b, Xb, p.E2);
-          a2.x_h2 = true; a2.pos_h2 = e2_h2;
-          GemmArgs at = a; at.x_h2 = e2_h2;
-          xb_h2 = factorise && kk >= 2 && gemm_tc2_supported(at, A_PLAIN) && gemm_tc2_supported(a2, A_PLAIN) && gemm_tc2_fp16x3(a2);
-        }
-        a.out_h2 = xb_h2; a.x_h2 = e2_h2;
-        g_tap_gamma_h2 = xb_h2 ? 1 : 0;
-        if (blk_tab && e2_h2 && xb_h2) { a.lif_tab = k.snn_gamma.tab; a.lif_tab_stride = k.snn_gamma.tab_stride; }
-        if (factorise && kk >= 2 && (gemm_tc2_supported(a, A_PLAIN) || gemm_tc_supported(a, A_PLAIN))) {
-          Layer Lw = k.fc_gamma;
-          Lw.bias = nullptr; Lw.scale = nullptr; Lw.shift = nullptr;
-          SAPCU_TRY(g.L("fn.fc_gamma(Wq|Wk per point)").layer(Lw, p.QKV, 3 * D, P, QK, 2 * D, ACT_NONE));
-          SAPCU_TRY(g.L("fn.fc_gamma(Wq|Wk per point)").layer(Lw, p.QKV + D, 3 * D, P, QK + D, 2 * D, ACT_NONE));
-          SAPCU_TRY(g.L("fn.fc_gamma+edge_bias+lif").run(a, A_PLAIN));
-        } else {
-          SAPCU_TRY(launch_attn_in(p.QKV, p.QKV + D, 3 * D, p.E2, p.idx, p.kmax, kk, M, E, D, p.E3, st));
-          SAPCU_TRY(g.L("fn.fc_gamma+lif").layer(k.fc_gamma, p.E3, D, E, p.E1, D, ACT_LIF, &k.snn_gamma, 4));
-        }
-      }
-      {
-        GemmArgs a = gamma2_args(b, Xb, pos32 ? p.E3 : p.E2);
-        a.x_h2 = xb_h2; a.pos_h2 = e2_h2 && !pos32;
-        if (gemm_tc2_supported(a, A_PLAIN) || gemm_tc_supported(a, A_PLAIN)) {
-          SAPCU_TRY(g.L("fn.fc_gamma2+softmax+sum(attention tail)").run(a, A_PLAIN));
-        } else {
-          SAPCU_TRY(g.L("fn.fc_gamma2").layer(k.fc_gamma2, p.E1, D, E, p.E3, D, ACT_NONE));
-          SAPCU_TRY(launch_attn_out(precise, p.E3, p.E2, p.QKV + 2 * D, 3 * D, p.idx, p.kmax, kk, M, P, D, a.at_sqrt, p.RES, st));
-        }
-      }
-      SAPCU_TRY(g.L("fn.out_proj").layer(k.out_proj, p.RES, D, P, p.R1, D, ACT_NONE));
-      SAPCU_TRY(g.L("fn.fc2+residual").layer(k.fc2, p.R1, D, P, p.FCAT + 64 * b, 192, ACT_NONE, nullptr, 0, fin, ldin));
-      continue;
-    }
-    SAPCU_TRY(g.L("fn.fc_delta2+lif").layer(k.fc_delta2, p.E1, D, E, p.E2, D, ACT_LIF, &k.snn_delta2, 4));
-    {
+    if (mode == SAPCU_MODE_FP32) {   // the literal schedule: attention input and logits materialised
+      SAPCU_TRY(g.L("fn.fc_delta2+lif").layer(k.fc_delta2, p.E1, D, E, p.E2, D, ACT_LIF, &k.snn_delta2, 4));
       GemmArgs a;
       a.A = p.E2; a.lda = D; a.R = E; a.K = D; a.idx = p.idx; a.ldi = p.kmax; a.kk = kk; a.Mpts = M;
       a.Q = p.QKV; a.Kf = p.QKV + D; a.ldq = 3 * D;
       a.W = k.fc_gamma.W; a.N = D; a.bias = k.fc_gamma.bias; a.scale = k.fc_gamma.scale; a.shift = k.fc_gamma.shift;
       a.act = ACT_LIF; a.T = 4; a.nparams = k.snn_gamma.np; a.Y = p.E3; a.ldc = D;
       SAPCU_TRY(g.L("fn.fc_gamma+lif").run(a, A_ATTNIN));
+      SAPCU_TRY(g.L("fn.fc_gamma2").layer(k.fc_gamma2, p.E3, D, E, p.E1, D, ACT_NONE));
+      SAPCU_TRY(launch_attn_out(precise, p.E1, p.E2, p.QKV + 2 * D, 3 * D, p.idx, p.kmax, kk, M, P, D, sq, p.RES, st));
+    } else {
+      SAPCU_TRY(g.L("fn.fc_delta2+lif").run(delta2_args(q), A_PLAIN));
+      if (q.attn_in) {
+        Layer Lw = k.fc_gamma;
+        Lw.bias = nullptr; Lw.scale = nullptr; Lw.shift = nullptr;
+        for (int h = 0; h < 2; ++h)   // [W q | W k], [P, 2D]
+          SAPCU_TRY(g.L("fn.fc_gamma(Wq|Wk per point)").layer(Lw, p.QKV + h * D, 3 * D, P, p.QK + h * D, 2 * D, ACT_NONE));
+        SAPCU_TRY(g.L("fn.fc_gamma+edge_bias+lif").run(gamma_args(q), A_PLAIN));
+      } else {
+        SAPCU_TRY(launch_attn_in(p.QKV, p.QKV + D, 3 * D, p.E2, p.idx, p.kmax, kk, M, E, D, p.E3, st));
+        SAPCU_TRY(g.L("fn.fc_gamma+lif").layer(k.fc_gamma, p.E3, D, E, p.E1, D, ACT_LIF, &k.snn_gamma, 4));
+      }
+      if (q.attn_out) {
+        SAPCU_TRY(g.L("fn.fc_gamma2+softmax+sum(attention tail)").run(gamma2_args(q), A_PLAIN));
+      } else {
+        SAPCU_TRY(g.L("fn.fc_gamma2").layer(k.fc_gamma2, p.E1, D, E, p.E3, D, ACT_NONE));
+        SAPCU_TRY(launch_attn_out(precise, p.E3, p.E2, p.QKV + 2 * D, 3 * D, p.idx, p.kmax, kk, M, P, D, sq, p.RES, st));
+      }
     }
-    SAPCU_TRY(g.L("fn.fc_gamma2").layer(k.fc_gamma2, p.E3, D, E, p.E1, D, ACT_NONE));
-    // torch (CPU) divides the logits by the python scalar sqrt(head_dim)
-    const float sq = sqrtf((float)(D / f.heads));
-    SAPCU_TRY(launch_attn_out(precise, p.E1, p.E2, p.QKV + 2 * D, 3 * D, p.idx, p.kmax, kk, M, P, D, sq, p.RES, st));
     SAPCU_TRY(g.L("fn.out_proj").layer(k.out_proj, p.RES, D, P, p.R1, D, ACT_NONE));
     SAPCU_TRY(g.L("fn.fc2+residual").layer(k.fc2, p.R1, D, P, p.FCAT + 64 * b, 192, ACT_NONE, nullptr, 0, fin, ldin));
   }
@@ -393,8 +345,6 @@ int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
 int fd_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* dist, const int32_t* const forced[3],
              const FdPlan& p, int mode, cudaStream_t st) {
   const FdNet& f = mdl->fd;
-  int g_tap_spk_h2 = 0;
-  struct TapPublish { const sapcu_model* m; int* g; ~TapPublish() { m->tap_spk.store(*g, std::memory_order_relaxed); } } tap_publish{mdl, &g_tap_spk_h2};
   const int64_t P = s * M;
   const bool precise = mode == SAPCU_MODE_FP32;
   const G g{mode, st};
@@ -412,25 +362,22 @@ int fd_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
   SAPCU_TRY(g.L("fd.scale_fusion").layer(f.fusion, p.F0, 64 * f.nscales, P, p.U0, 64, ACT_LEAKY));
   const int64_t ldspk = (int64_t)T * 960;
   // conv5 (multi-scale fusion) + LeakyReLU + max over the patch's points: in the tensor-core modes the 2-CTA kernel
-  // reduces in its epilogue (per-thread running maxima, then float atomic max) and AGG is never written
-  GemmArgs c5;
-  {
-    const Layer& L = f.msc;
-    c5.A = p.SPK; c5.lda = 960; c5.R = P * T; c5.K = L.K; c5.W = L.W; c5.Whi = L.Whi; c5.Wlo = L.Wlo; c5.N = L.N;
-    c5.bias = L.bias; c5.scale = L.scale; c5.shift = L.shift; c5.act = ACT_LEAKY; c5.Y = p.AGG; c5.ldc = f.emb;
-    c5.pool = p.POOL; c5.pool_T = T; c5.pool_M = M;
-    c5.Wh = L.Wh; c5.Wl = L.Wl; c5.winv = L.winv; c5.x_unit = true;                   // the spike tensor
-    c5.tc_passes = (mode == SAPCU_MODE_TF32 || mode == SAPCU_MODE_FAST) ? 1 : 3;
-  }
-  const bool pooled = mode != SAPCU_MODE_FP32 && settings().fuse_pool && gemm_tc2_supported(c5, A_PLAIN);
-  // When conv5 runs on the fp16x3 path the spike tensor is stored as fp16 (hi, lo) planes of s * 2^13 (rows = point*T + t)
-  // that it loads without converting; the step-0 spikes, which the graphs and EdgeConvs of the next block read, are
-  // also kept in fp32 (SPK0, [P, 960]).
-  bool spk_fast = false;
-  if (mode == SAPCU_MODE_FAST && pooled) { c5.fast = true; c5.x_h2 = true; spk_fast = gemm_tc2_fast(c5); c5.fast = spk_fast; c5.x_h2 = false; }
-  const bool spk_h2 = pooled && (spk_fast || gemm_tc2_fp16x3(c5));
-  g_tap_spk_h2 = spk_fast ? 2 : (spk_h2 ? 1 : 0);
-  const int64_t plane = spk_fast ? 0 : P * T * 960;         // fast mode: hi plane only
+  // reduces in its epilogue (per-thread running maxima, then float atomic max) and AGG is never written.  `spk` is the
+  // spike tensor's format (tap code): conv5 loads it as it is stored.
+  auto c5_args = [&](int spk, bool pooled) {
+    GemmArgs a = g.args(f.msc, p.SPK, 960, P * T, p.AGG, f.emb, ACT_LEAKY, nullptr, 0, nullptr, 0, true);   // the spike tensor
+    a.pool = pooled ? p.POOL : nullptr; a.pool_T = T; a.pool_M = M;
+    a.x_h2 = spk != 0; a.fast = spk == 2;
+    return a;
+  };
+  const bool pooled = mode != SAPCU_MODE_FP32 && settings().fuse_pool && gemm_tc2_supported(c5_args(0, true), A_PLAIN);
+  // When conv5 runs on the fast or the fp16x3 path the spike tensor is stored as one fp16 plane or as fp16 (hi, lo) planes
+  // of s * 2^13 (rows = point*T + t); the step-0 spikes, which the graphs and EdgeConvs of the next block read, are also
+  // kept in fp32 (SPK0, [P, 960]).
+  const int spk = !pooled ? 0 : (mode == SAPCU_MODE_FAST && gemm_tc2_fast(c5_args(2, true))) ? 2 : gemm_tc2_fp16x3(c5_args(1, true)) ? 1 : 0;
+  mdl->tap_spk.store(spk, std::memory_order_relaxed);
+  const bool spk_h2 = spk != 0;
+  const int64_t plane = spk == 2 ? 0 : P * T * 960;         // fast mode: hi plane only
   const float* S0 = spk_h2 ? p.SPK0 : p.SPK;                     // step-0 spikes: row stride ld0
   const int64_t ld0 = spk_h2 ? 960 : ldspk;
   if (spk_h2) SAPCU_TRY(launch_neuron_unroll(true, precise, p.U0, 64, P, 64, T, f.blk[0].np, f.blk[0].ep, 1, p.SPK, 960, st, true, p.SPK0, plane, 0));
@@ -481,12 +428,10 @@ int fd_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
                                    p.SPK + off_out[b], 960, st));
   }
   if (pooled) {
-    c5.x_h2 = spk_h2;
     SAPCU_TRY(launch_fill(p.POOL, s * T * f.emb, -INFINITY, st));
-    SAPCU_TRY(g.L("fd.conv5+maxpool").run(c5, A_PLAIN));
+    SAPCU_TRY(g.L("fd.conv5+maxpool").run(c5_args(spk, true), A_PLAIN));
   } else {
-    c5.pool = nullptr;
-    SAPCU_TRY(g.L("fd.conv5").run(c5, A_PLAIN));
+    SAPCU_TRY(g.L("fd.conv5").run(c5_args(0, false), A_PLAIN));
     SAPCU_TRY(launch_group_max(p.AGG, s, M, T, f.emb, p.POOL, st));
   }
   SAPCU_TRY(launch_temporal_lif(precise, p.POOL, s, T, f.emb, f.tw, f.snn_fc.np, p.Z, st));
