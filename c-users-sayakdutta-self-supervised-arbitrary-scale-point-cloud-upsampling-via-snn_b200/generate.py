@@ -4,6 +4,7 @@
   farthest_point_sample     generate.py:56-74   one cooperative CUDA kernel (csrc/post_ops.cu) instead of `npoint` torch
                                                  round trips; same fp32 arithmetic, start index N // 2, lowest-index ties
   process_file              generate.py:81-101  load .xyz -> normalise -> upsample -> denormalise -> FPS -> save
+                                                 (with_normals=True: six columns, point and oriented normal)
 """
 import numpy as np
 import torch
@@ -33,11 +34,19 @@ def farthest_point_sample(xyz, npoint, device="cuda"):
     return out.cpu().numpy().astype(np.int64)
 
 
-def process_file(input_path, output_path, generator, target_points):
+def process_file(input_path, output_path, generator, target_points, with_normals=False):
+    """with_normals: six columns per row, the point and its oriented normal (Generator3D6.upsample(return_normals=True));
+    the uniform scale and translation of the denormalisation leave normals unchanged."""
     cloud = np.loadtxt(input_path)[:, :3]
     cloud, loc, scale = normalize_pointcloud(cloud)
-    upsampled = np.array(generator.upsample(np.expand_dims(cloud, 0)))
+    if with_normals:
+        upsampled, normals = generator.upsample(np.expand_dims(cloud, 0), return_normals=True)
+    else:
+        upsampled = np.array(generator.upsample(np.expand_dims(cloud, 0)))
     upsampled = upsampled * scale + loc
     assert upsampled.shape[0] >= target_points, f"Generated {upsampled.shape[0]} points, expected >= {target_points}"
     indices = farthest_point_sample(upsampled, target_points, device=generator.device)
-    np.savetxt(output_path, upsampled[indices], fmt="%.6f")
+    rows = upsampled[indices]
+    if with_normals:
+        rows = np.concatenate([rows, normals[indices]], axis=1)
+    np.savetxt(output_path, rows, fmt="%.6f")

@@ -11,6 +11,9 @@ The kNN is computed once (the reference queries the same tree twice with identic
 round-trips through the host between stages.  Seeds come from `./dense` exactly as in the reference unless the
 caller injects them with `seeds=` (needed for synthetic benchmarks; SURVEY.md section 8b).
 
+`upsample(..., return_normals=True)` also returns the fn normals of the output points, oriented consistently on the device
+(`orient_normals`: self-kNN + sapcu_orient_normals); without it every path and result is the reference contract above.
+
 `device` may also be a sequence of devices: the flat seed list is then split with `sharding.shard_bounds` (the split of the
 torch.distributed path), every shard runs the same pipeline on its device in a host thread of its own, and the results are
 gathered in shard order.  A repeated device is one more worker on that device, with its own stream.
@@ -53,6 +56,37 @@ def morton_order(d_pts, bits=10):
     return torch.argsort(key)
 
 
+@torch.no_grad()
+def orient_normals(d_points, d_normals, k=10):
+    """Consistently oriented copy of unit normals [S,3] f32 at points [S,3] f64 (both cuda): the self-kNN (sapcu_knn,
+    K = min(k + 1, S), the +1 for the point itself) and the spanning-forest propagation of sapcu_orient_normals.  Every row
+    of the result is bitwise its input or its negation; per connected component of the kNN graph the topmost point's normal
+    points up (include/sapcu_b200.h gives the exact rule)."""
+    S = d_points.shape[0]
+    if d_points.shape != (S, 3) or d_normals.shape != (S, 3) or d_points.dtype != torch.float64 or d_normals.dtype != torch.float32:
+        raise ValueError("orient_normals: points [S,3] float64 and normals [S,3] float32 expected")
+    if d_points.device.type != "cuda" or d_normals.device != d_points.device:
+        raise N.SapcuError("orient_normals needs both tensors on one CUDA device (no CPU fallback)")
+    if k < 1:
+        raise ValueError("orient_normals: k must be at least 1")
+    out = d_normals.clone(memory_format=torch.contiguous_format)
+    if S == 0:
+        return out
+    L = N.lib()
+    dev = d_points.device
+    K = min(k + 1, S)
+    with torch.cuda.device(dev):
+        st = N.stream_ptr(dev)
+        pts = d_points.contiguous()
+        idx = torch.empty(S, K, dtype=torch.int32, device=dev)
+        kws = torch.empty(L.sapcu_knn_workspace_bytes(S), dtype=torch.uint8, device=dev)
+        N.check(L.sapcu_knn(N.ptr(pts), S, N.ptr(pts), S, K, N.ptr(idx), N.ptr(kws), kws.numel(), st), "sapcu_knn(self)")
+        ws = torch.empty(L.sapcu_orient_normals_workspace_bytes(S, K), dtype=torch.uint8, device=dev)
+        N.check(L.sapcu_orient_normals(N.ptr(pts), S, N.ptr(idx), K, N.ptr(out), None, N.ptr(ws), ws.numel(), st),
+                "sapcu_orient_normals")
+    return out
+
+
 def _on_device(fn):
     """Run a Generator3D6 method with the generator's CUDA device current (launches, allocations and the stream the
     C ABI receives all belong to that device, whichever device the calling thread had selected)."""
@@ -69,7 +103,8 @@ def _on_device(fn):
 
 class Generator3D6(object):
     def __init__(self, model1, model2, device, k_neighbors=100, dense_spacing=0.004,
-                 outlier_threshold=1.5, batch_size=400, seeds_per_pass=None, remove_outliers=True, seed_source="gpu"):
+                 outlier_threshold=1.5, batch_size=400, seeds_per_pass=None, remove_outliers=True, seed_source="gpu",
+                 normal_neighbors=10):
         self.model1, self.model2 = model1, model2          # fn (normals), fd (distances)
         self.devices = [torch.device(d) for d in ([device] if isinstance(device, (str, int, torch.device)) else device)]
         if not self.devices:
@@ -83,26 +118,50 @@ class Generator3D6(object):
         self.remove_outliers = remove_outliers
         self.seed_source = seed_source                     # "gpu": sapcu_seedgen; "dense": the reference's ./dense process
         self.sort_seeds = True                             # Morton-order the seeds of large clouds (N >= 2^20) before the pipeline
+        self.normal_neighbors = normal_neighbors           # k of the graph that orients returned normals (return_normals=True)
         self.model1.eval()
         self.model2.eval()
         self._bufs = {}
         self._streams = {}                                 # worker index -> its stream (several devices only)
 
     # ------------------------------------------------------------------ reference API
-    def upsample(self, data, seeds=None):
-        return self.generateiopoint(data, seeds=seeds)
+    def upsample(self, data, seeds=None, return_normals=False):
+        return self.generateiopoint(data, seeds=seeds, return_normals=return_normals)
 
-    def generateiopoint(self, data, seeds=None):
+    def generateiopoint(self, data, seeds=None, return_normals=False):
+        """-> points [M,3] f64; with return_normals: (points, normals [M,3] f32), the fn normals of the same rows, oriented
+        consistently over the surviving points (orient_normals, k = normal_neighbors)."""
         data = np.asarray(data, dtype=np.float64)
         if data.ndim == 3:
             data = np.squeeze(data, 0)
         if seeds is None:
             seeds = self._dense_seeds(data)
         seeds = np.ascontiguousarray(np.asarray(seeds, dtype=np.float64)[:, :3])
+        if return_normals:
+            return self._points_and_normals(np.ascontiguousarray(data), seeds)[0]
         out = self.displace_host(data, seeds)
         if self.remove_outliers:
             out = self._outlier_filter(out)
         return out
+
+    @_on_device
+    def _points_and_normals(self, cloud, seeds, batch=None):
+        """The pipeline with its normals kept, per problem of `batch` (one problem without): the outlier mask selects points
+        and normals alike, then the normals are oriented on the surviving points, on the primary device.  Returns a list of
+        (points [M_b,3] f64, normals [M_b,3] f32) host arrays."""
+        d_out, _, d_normals, _ = self.displace_device(torch.from_numpy(cloud).to(self.device),
+                                                      torch.from_numpy(seeds).to(self.device), return_parts=True, batch=batch)
+        so = (0, seeds.shape[0]) if batch is None else batch[1]
+        res = []
+        for b in range(len(so) - 1):
+            pts, nrm = d_out[so[b]:so[b + 1]], d_normals[so[b]:so[b + 1]]
+            if self.remove_outliers:
+                keep = self._outlier_keep(pts).bool()
+                pts, nrm = pts[keep], nrm[keep]
+            nrm = orient_normals(pts, nrm, self.normal_neighbors)
+            res.append((pts.cpu().numpy(), nrm.cpu().numpy()))
+        N.check_device("upsample(return_normals=True)")
+        return res
 
     # ------------------------------------------------------------------ host <-> device pipeline
     def _pinned(self, key, shape, dtype):
@@ -273,16 +332,19 @@ class Generator3D6(object):
                 N.check_device("displace_host")
         return h_out.numpy().copy()
 
-    def upsample_batch(self, clouds, seeds):
+    def upsample_batch(self, clouds, seeds, return_normals=False):
         """A batch of independent clouds in one device pipeline (the per-file loop of the reference's generate.py:135-160
         as ONE call): clouds / seeds are lists of [N_b,3] / [S_b,3] arrays; returns the list of displaced [S_b,3] f64
-        arrays (outlier-filtered per cloud when remove_outliers is set)."""
+        arrays (outlier-filtered per cloud when remove_outliers is set).  return_normals: a list of (points, normals) pairs,
+        each cloud's normals oriented on its own points as in upsample."""
         clouds = [np.ascontiguousarray(np.asarray(c, dtype=np.float64).reshape(-1, 3)) for c in clouds]
         seeds = [np.ascontiguousarray(np.asarray(s, dtype=np.float64)[:, :3]) for s in seeds]
         if len(clouds) != len(seeds):
             raise ValueError("upsample_batch: one seed array per cloud")
         co = np.concatenate([[0], np.cumsum([c.shape[0] for c in clouds])]).astype(np.int64)
         so = np.concatenate([[0], np.cumsum([s.shape[0] for s in seeds])]).astype(np.int64)
+        if return_normals:
+            return self._points_and_normals(np.concatenate(clouds, 0), np.concatenate(seeds, 0), batch=(co, so))
         out = self.displace_host(np.concatenate(clouds, 0), np.concatenate(seeds, 0), batch=(co, so))
         res = [out[so[b]:so[b + 1]] for b in range(len(clouds))]
         if self.remove_outliers:
@@ -322,12 +384,17 @@ class Generator3D6(object):
     def _outlier_filter(self, xyz):
         """generation.py:176-183 on the device: self-kNN (k = 30) with sapcu_knn, mean neighbour distance per point,
         keep the points below outlier_threshold x the global mean."""
+        d_pts = torch.from_numpy(np.ascontiguousarray(xyz, dtype=np.float64)).to(self.device)
+        return xyz[self._outlier_keep(d_pts).cpu().numpy().astype(bool), :]
+
+    def _outlier_keep(self, d_pts):
+        """uint8 [S] keep mask of the outlier filter for points [S,3] f64 on self.device (which must be current)."""
         L = N.lib()
-        S = xyz.shape[0]
+        S = d_pts.shape[0]
         if S < 30:
             raise ValueError("k must be less than or equal to the number of training points")   # as sklearn does
         st = N.stream_ptr(self.device)
-        d_pts = torch.from_numpy(np.ascontiguousarray(xyz, dtype=np.float64)).to(self.device)
+        d_pts = d_pts.contiguous()
         idx = torch.empty(S, 30, dtype=torch.int32, device=self.device)
         kws = torch.empty(L.sapcu_knn_workspace_bytes(S), dtype=torch.uint8, device=self.device)
         N.check(L.sapcu_knn(N.ptr(d_pts), S, N.ptr(d_pts), S, 30, N.ptr(idx), N.ptr(kws), kws.numel(), st), "sapcu_knn(self)")
@@ -335,7 +402,7 @@ class Generator3D6(object):
         ows = torch.empty(L.sapcu_outlier_workspace_bytes(S), dtype=torch.uint8, device=self.device)
         N.check(L.sapcu_outlier_mask(N.ptr(d_pts), S, N.ptr(idx), 30, float(self.outlier_threshold), N.ptr(keep), N.ptr(ows),
                                      ows.numel(), st), "sapcu_outlier_mask")
-        return xyz[keep.cpu().numpy().astype(bool), :]
+        return keep
 
 
 class SNNPointCloudGenerator(Generator3D6):

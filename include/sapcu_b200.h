@@ -150,6 +150,27 @@ int sapcu_fps(const float* d_xyz, int64_t N, int64_t npoint, int64_t start, int3
               void* d_ws, size_t ws_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------
+ * Normal orientation (no reference counterpart; the spanning-tree propagation of Hoppe et al., Open3D's
+ * orient_normals_consistent_tangent_plane): flips the signs of unit normals so that neighbours agree (csrc/orient.cu).
+ *   graph   undirected, edges {i, d_idx[i*k + j]} for j < k; entries equal to i are skipped (with duplicated points the
+ *           self entry is not always in column 0), and so are entries outside [0, S).  Intended input: sapcu_knn with cloud = seeds =
+ *           d_points and K = k.  1 <= k <= 128, S >= 1, S*k < 2^31, else SAPCU_EINVAL; a short workspace: SAPCU_EWORKSPACE.
+ *   edge    dot = ((nx_i*nx_j) + (ny_i*ny_j)) + nz_i*nz_j in fp64 from the fp32 components, without contraction (a numpy
+ *           restatement gives the same bits); a flip edge has dot < 0; its weight is |dot|.
+ *   forest  the maximum spanning forest under the strict order: larger |dot| first, then the smaller (min(i,j), max(i,j))
+ *           pair -- unique, independent of the launch configuration and of the order in which atomics land.
+ *   root    per connected component the point with the largest z (ties -> lowest index); it keeps its normal when
+ *           nz >= 0 and is negated when nz < 0 (outward at the topmost point of a closed surface).
+ *   others  negated when the root was negated XOR the tree path from the root holds an odd number of flip edges.
+ * d_normals: [S,3] fp32, oriented in place -- every output is bitwise its input or the exact negation of it (sign bit).
+ * d_root (nullable): int32 [S], each point's root index.  d_points: [S,3] f64 (only z is read).  Allocates nothing and
+ * does not synchronise the stream.
+ * ---------------------------------------------------------------------------------- */
+size_t sapcu_orient_normals_workspace_bytes(int64_t S, int k);   /* 0 for arguments outside the limits above */
+int sapcu_orient_normals(const double* d_points, int64_t S, const int32_t* d_idx, int k,
+                         float* d_normals, int32_t* d_root, void* d_ws, size_t ws_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------
  * Models.  A handle is built from the same hyper-parameters get_model() consumes
  * (fn/config.py:183-210, fd/config.py:89-117) and the tensors of the module's
  * state_dict (host fp32 pointers, names = state_dict keys, SURVEY.md section 8b).
