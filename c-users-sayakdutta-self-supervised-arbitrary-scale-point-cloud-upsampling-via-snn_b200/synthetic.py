@@ -3,6 +3,7 @@
   cloud(n, seed, shape)   points on a closed surface, bbox-normalised like generate.py:43-53 (fp64)
   seeds(cloud, ratio, seed)  S = ceil(ratio*N) seeds in the 0.011-0.015 band dense.cpp emits around the surface
   init_weights(model, seed, stress)  deterministic random weights for an fn/fd module (state_dict in place)
+  sphere_mesh(level)      the icosphere of radius 0.5 that cloud(shape="sphere") samples (metrics tests and benchmark)
 
 Everything is generated from numpy / torch CPU generators so the GPU box reproduces the same bits
 without the reference checkout.
@@ -56,6 +57,31 @@ def seeds(cloud_pts, ratio, seed=1):
     u /= np.linalg.norm(u, axis=1, keepdims=True)
     rho = rng.uniform(0.011, 0.015, size=(s, 1))
     return np.ascontiguousarray(cloud_pts[np.arange(s) % n] + u * rho)
+
+
+def sphere_mesh(level=3):
+    """Icosahedron subdivided `level` times (20 * 4**level faces), vertices on the sphere of radius 0.5 centred at the
+    origin -> (vertices [V,3] float64, faces [F,3] int32).  Every face is wound counter-clockwise seen from outside, so
+    (b-a)x(c-a) points outward.  cloud(n, shape="sphere") samples this sphere (up to its bounding-box normalisation, which
+    moves the points by well under 1e-2 for n >= 1000)."""
+    t = (1.0 + math.sqrt(5.0)) / 2.0
+    v = np.array([[-1, t, 0], [1, t, 0], [-1, -t, 0], [1, -t, 0], [0, -1, t], [0, 1, t], [0, -1, -t], [0, 1, -t],
+                  [t, 0, -1], [t, 0, 1], [-t, 0, -1], [-t, 0, 1]], dtype=np.float64)
+    f = np.array([[0, 11, 5], [0, 5, 1], [0, 1, 7], [0, 7, 10], [0, 10, 11], [1, 5, 9], [5, 11, 4], [11, 10, 2], [10, 7, 6],
+                  [7, 1, 8], [3, 9, 4], [3, 4, 2], [3, 2, 6], [3, 6, 8], [3, 8, 9], [4, 9, 5], [2, 4, 11], [6, 2, 10],
+                  [8, 6, 7], [9, 8, 1]], dtype=np.int64)
+    v /= np.linalg.norm(v, axis=1, keepdims=True)
+    for _ in range(level):
+        nv, nf = v.shape[0], f.shape[0]
+        e = np.concatenate([f[:, [0, 1]], f[:, [1, 2]], f[:, [2, 0]]])
+        e.sort(axis=1)
+        uniq, inv = np.unique(e[:, 0] * nv + e[:, 1], return_inverse=True)
+        mid = v[uniq // nv] + v[uniq % nv]
+        v = np.concatenate([v, mid / np.linalg.norm(mid, axis=1, keepdims=True)])
+        m01, m12, m20 = (nv + inv.reshape(3, nf))
+        a, b, c = f[:, 0], f[:, 1], f[:, 2]
+        f = np.concatenate([np.stack(x, axis=1) for x in ((a, m01, m20), (b, m12, m01), (c, m20, m12), (m01, m12, m20))])
+    return np.ascontiguousarray(0.5 * v), np.ascontiguousarray(f, dtype=np.int32)
 
 
 def _gen(seed):

@@ -171,6 +171,32 @@ int sapcu_orient_normals(const double* d_points, int64_t S, const int32_t* d_idx
                          float* d_normals, int32_t* d_root, void* d_ws, size_t ws_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------
+ * Point-to-mesh distance (no reference counterpart; the P2F metric of the upsampling literature, computed there on the
+ * host with CGAL): the exact squared distance from every query point to a triangle mesh (csrc/mesh_dist.cu).
+ *   distance  d_dist2[s] = min over faces f of D(p_s, f).  D is ((dx*dx)+(dy*dy))+(dz*dz) in fp64 without contraction,
+ *             from p_s to q, where q is the closest point on the triangle (a, b, c) = d_vertices[d_faces[f]] of the shared
+ *             routine (csrc/geom.cuh, Ericson's region test in the operation order of the reference's dense.cpp), with
+ *             two additions: when a coordinate of that point is not finite (the 0/0 of a degenerate face: two coincident
+ *             vertices, or a zero normal) q is the closest of the three segment points of ab, bc, ca, each
+ *             a + e*t with e = b - a, t = ((p-a).e)/(e.e) clamped to [0, 1] (t = 0 when e.e == 0), the first of equal
+ *             distances; and q is then clamped coordinate-wise into the face's box [min, max of the vertex coordinates]
+ *             (which holds the exact closest point, so the clamp only moves q towards it).  No input gives NaN.
+ *   face      d_face[s] (nullable): the face attaining the minimum; ties (bitwise-equal D) go to the lowest face index.
+ *             -1 (and d_dist2 = +inf) when no face is valid.
+ *   order     the result does not depend on the tree, the launch configuration or the order of the query points: it is
+ *             bitwise the brute-force minimum of (D, face index).
+ *   limits    V >= 1, 1 <= F < 2^31, S >= 0, else SAPCU_EINVAL; S == 0 is a no-op; a short workspace: SAPCU_EWORKSPACE.
+ *             Faces with an index outside [0, V) are skipped, so no input makes a kernel read outside its arrays.
+ *   method    one linear BVH per call (Karras 2012) over the faces' centroid Morton codes, built and queried on the device.
+ * d_vertices: [V,3] f64, d_faces: [F,3] int32, d_points: [S,3] f64, d_dist2: [S] f64.  Allocates nothing and does not
+ * synchronise the stream.  The workspace size is a closed form of F (about 200 bytes per face), computed without a device.
+ * ---------------------------------------------------------------------------------- */
+size_t sapcu_mesh_distance_workspace_bytes(int64_t V, int64_t F);   /* 0 for arguments outside the limits above */
+int sapcu_mesh_distance(const double* d_vertices, int64_t V, const int32_t* d_faces, int64_t F,
+                        const double* d_points, int64_t S, double* d_dist2, int32_t* d_face,
+                        void* d_ws, size_t ws_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------
  * Models.  A handle is built from the same hyper-parameters get_model() consumes
  * (fn/config.py:183-210, fd/config.py:89-117) and the tensors of the module's
  * state_dict (host fp32 pointers, names = state_dict keys, SURVEY.md section 8b).
