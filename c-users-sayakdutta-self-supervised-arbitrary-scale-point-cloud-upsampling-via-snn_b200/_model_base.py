@@ -133,14 +133,19 @@ class NativeModel(nn.Module):
             self._root()._workspaces.clear()
         self._ws_last = value
 
-    def _workspace(self, S, M, device):
+    def _workspace(self, S, M, device, ncloud=0):
         """(workspace tensor, bytes to pass to the forward).  Workspaces are cached per (device, stream): calls on one stream
         run in order and may share one, calls on two streams never do.  The byte count is max(one patch, min(need,
-        WORKSPACE_CAP)) whatever the cached tensor's size, so WORKSPACE_CAP alone decides the chunking."""
+        WORKSPACE_CAP)) whatever the cached tensor's size, so WORKSPACE_CAP alone decides the chunking.  ncloud > 0: the
+        workspace of the fn forward on patches indexed into a cloud of that many points."""
         L = N.lib()
         h = self._ensure_handle(device)
-        need = L.sapcu_model_workspace_bytes(h, S, M)
-        one = L.sapcu_model_workspace_bytes(h, 1, M)
+        if ncloud:
+            need = L.sapcu_fn_indexed_workspace_bytes(h, S, M, ncloud, self.mode)
+            one = L.sapcu_fn_indexed_workspace_bytes(h, 1, M, ncloud, self.mode)
+        else:
+            need = L.sapcu_model_workspace_bytes(h, S, M)
+            one = L.sapcu_model_workspace_bytes(h, 1, M)
         want = max(one, min(need, self.WORKSPACE_CAP))
         owner = self._root()
         key = (device.index, torch.cuda.current_stream(device).cuda_stream)

@@ -13,7 +13,7 @@ _CSRC = os.path.join(_HERE, "csrc")
 _SO = os.path.join(_HERE, "libsapcu_b200.so")
 _SOURCES = ["api.cu", "model.cu", "forward.cu", "gemm.cu", "gemm_tc.cu", "gemm_tc2.cu", "knn_seed.cu", "patch_ops.cu",
             "intra_knn.cu", "fn_kernels.cu", "fd_kernels.cu", "seedgen.cu", "post_ops.cu", "lif_table.cu", "orient.cu",
-            "mesh_dist.cu"]
+            "mesh_dist.cu", "edge_pairs.cu"]
 # per-file flags: the fp64 geometry of seedgen.cu must round like the g++ build of dense.cpp (no FMA contraction), and that
 # of mesh_dist.cu like its numpy restatement
 _FILE_FLAGS = {"seedgen.cu": ["-fmad=false"], "mesh_dist.cu": ["-fmad=false"]}
@@ -137,6 +137,15 @@ _SIGS = {
     "sapcu_fn_forward": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int,
                                         ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_int,
                                         ctypes.c_void_p]),
+    "sapcu_fn_indexed_workspace_bytes": (ctypes.c_size_t, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_int64, ctypes.c_int]),
+    "sapcu_pair_table_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_int64]),
+    "sapcu_pair_table": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
+                                        ctypes.c_int64, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_size_t,
+                                        ctypes.c_void_p, ctypes.c_void_p]),
+    "sapcu_fn_forward_indexed": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int,
+                                                ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_int64,
+                                                ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_int,
+                                                ctypes.c_void_p]),
     "sapcu_fd_forward": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int,
                                         ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t,
                                         ctypes.c_int, ctypes.c_void_p]),

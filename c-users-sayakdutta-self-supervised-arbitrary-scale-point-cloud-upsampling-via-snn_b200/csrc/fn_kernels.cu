@@ -137,6 +137,42 @@ edge_pos_lif_kernel(const float* __restrict__ xyz, const int32_t* __restrict__ i
 // offsets are expanded into shared memory, and 4 threads per channel walk the edges (lane = channel, so a warp's 32 stores
 // of a row are 64 contiguous bytes).  LTAB = 0: no usable table -- the reduced-MUFU recurrence instead.
 constexpr int EPF_THREADS = 512;
+// LIF^T chain of NV rows of one channel from x = BN(.) - theta0 (LTAB: the table at lt_desc, exact chain out of its range) or
+// from u = BN(.) (reduced-MUFU recurrence)
+template <int LTAB, int NV>
+__device__ __forceinline__ void lif_rows(float (&u)[NV], const NeuronParams& p, int T, uint32_t lt_desc) {
+  if (LTAB) {
+    float x0[NV];
+#pragma unroll
+    for (int j = 0; j < NV; ++j) x0[j] = u[j];
+    if (lif_table_eval_vec<NV>(u, lt_desc)) {
+#pragma unroll
+      for (int j = 0; j < NV; ++j) if (lif_table_oob(x0[j])) u[j] = lif_chain<false>(x0[j] + p.th0, p, T);
+    }
+  } else {
+    lif_chain_vec_fast2<NV>(u, p, T);
+  }
+}
+// fc_delta (K = 3) with BN folded into (w0, w1, w2, b0), then the LIF^T chain: the same fmaf chain for edge and pair rows
+template <int LTAB>
+__device__ __forceinline__ void pos_lif4(const float4 (&d)[4], float w0, float w1, float w2, float b0, const NeuronParams& p, int T,
+                                         uint32_t lt_desc, float (&u)[4]) {
+#pragma unroll
+  for (int j = 0; j < 4; ++j) u[j] = fmaf(w2, d[j].z, fmaf(w1, d[j].y, fmaf(w0, d[j].x, b0)));
+  lif_rows<LTAB, 4>(u, p, T, lt_desc);
+}
+// rows j < n of y * 2^13 as an fp16 plane (+ the lo plane `plane` halfs behind it when PL2), row stride C
+template <int PL2, int NV>
+__device__ __forceinline__ void store_h(__half* o, int64_t C, int64_t plane, const float (&u)[NV], int n) {
+#pragma unroll
+  for (int j = 0; j < NV; ++j)
+    if (j < n) {
+      const float ys = u[j] * 8192.0f;
+      const __half hv = __float2half_rn(ys);
+      o[j * C] = hv;
+      if (PL2) o[plane + j * C] = __float2half_rn(ys - __half2float(hv));
+    }
+}
 // PL2: also write the lo plane (y * 2^13 - hi) `plane` halfs behind the hi plane -- the (hi, lo) hand-over format of the
 // parity-grade tensor-core mode, whose LIF^T chains may use the same tables.
 template <int LTAB, int CT, int PL2 = 0>     // CT: compile-time channel count (row stride of the output: store offsets become immediates), 0 = run-time
@@ -178,37 +214,109 @@ edge_pos_lif_fast_kernel(const float* __restrict__ xyz, const int32_t* __restric
     if (!cv) continue;
     __half* o = out + patch0 * kk * (int64_t)C + c + (int64_t)(part * 4) * C;   // this thread's first row; rounds advance it by 16 rows
     auto group = [&](int e0, bool full) {                                      // 4 consecutive edges of this thread's channel
+      float4 d[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) d[j] = pd[(full || (e0 + j) < EP) ? (e0 + j) : (EP - 1)];
       float u[4];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const float4 d = pd[(full || (e0 + j) < EP) ? (e0 + j) : (EP - 1)];
-        u[j] = fmaf(w2, d.z, fmaf(w1, d.y, fmaf(w0, d.x, b0)));
-      }
-      if (LTAB) {
-        float x0[4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) x0[j] = u[j];
-        if (lif_table_eval_vec<4>(u, lt_desc)) {
-#pragma unroll
-          for (int j = 0; j < 4; ++j) if (lif_table_oob(x0[j])) u[j] = lif_chain<false>(x0[j] + p.th0, p, T);
-        }
-      } else {
-        lif_chain_vec_fast2<4>(u, p, T);
-      }
-#pragma unroll
-      for (int j = 0; j < 4; ++j)
-        if (full || e0 + j < EP) {
-          const float ys = u[j] * 8192.0f;
-          const __half hv = __float2half_rn(ys);
-          o[j * C] = hv;
-          if (PL2) o[plane + j * C] = __float2half_rn(ys - __half2float(hv));
-        }
+      pos_lif4<LTAB>(d, w0, w1, w2, b0, p, T, lt_desc, u);
+      store_h<PL2, 4>(o, C, plane, u, full ? 4 : EP - e0);
       o += 16 * C;
     };
     const int EPfull = EP & ~15;                                               // whole rounds of 4 phases x 4 edges: no bounds checks
 #pragma unroll 1
     for (int e0 = part * 4; e0 < EPfull; e0 += 16) group(e0, true);
     if (EPfull + part * 4 < EP) group(EPfull + part * 4, false);
+  }
+}
+
+// edge_pos_lif_fast (table flavour, (hi, lo) planes) on pair rows: row u's offset is delta[u]; persistent CTAs (grid.y = 128-channel block), 4 threads per channel
+// each take 4 consecutive rows, the first *U_dev rows only.  `plane`: halfs between the hi and the lo plane (capacity * C).
+template <int CT>
+__global__ void __launch_bounds__(EPF_THREADS)
+pair_pos_lif_kernel(const float4* __restrict__ delta, const int* __restrict__ U_dev, int C_rt, const float* __restrict__ W,
+                    const float* __restrict__ bias, const float* __restrict__ scale, const float* __restrict__ shift,
+                    const float* __restrict__ np, int T, __half* __restrict__ out, const uint8_t* __restrict__ tab, uint32_t tab_stride,
+                    int64_t plane) {
+  extern __shared__ __align__(16) uint8_t epf_sm[];
+  const int C = CT ? CT : C_rt;
+  const int tid = threadIdx.x;
+  const int cl = tid & 127, part = tid >> 7;
+  const int c = blockIdx.y * 128 + cl;
+  const bool cv = c < C;
+  const int cc = cv ? c : 0;
+  lif_table_load(tab + (size_t)blockIdx.y * tab_stride, epf_sm, tab_stride, tid, EPF_THREADS);
+  const uint32_t lt_desc = (uint32_t)__cvta_generic_to_shared(epf_sm) + (uint32_t)cl * 8u;
+  const float sc = scale[cc];
+  const float w0 = W[3 * cc] * sc, w1 = W[3 * cc + 1] * sc, w2 = W[3 * cc + 2] * sc;
+  const NeuronParams p{np[cc], np[C + cc], np[2 * C + cc], np[3 * C + cc]};
+  const float b0 = fmaf(bias[cc], sc, shift[cc]) - p.th0;
+  __syncthreads();                                                             // the table landed
+  if (!cv) return;
+  const int64_t U = *U_dev;
+  for (int64_t r0 = ((int64_t)blockIdx.x * 4 + part) * 4; r0 < U; r0 += (int64_t)gridDim.x * 16) {
+    float4 d[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) d[j] = delta[r0 + j < U ? r0 + j : U - 1];
+    float u[4];
+    pos_lif4<1>(d, w0, w1, w2, b0, p, T, lt_desc, u);
+    store_h<1, 4>(out + r0 * C + c, C, plane, u, (int)(U - r0 < 4 ? U - r0 : 4));
+  }
+}
+
+// fc_gamma's table-flavour epilogue per edge, with the contraction W_gamma pos done per pair (WP, fp32, accumulator scale
+// already undone): x = fmaf(WP[pid[e]], sc, fmaf(Wq[pt] - Wk[nb], sc, fmaf(bias, sc, shift) - theta0)) -- the expression of
+// gemm_tc2_kernel's LT epilogue with the edge bias -- then the tabulated chain; (hi, lo) planes out as that epilogue writes them.
+// Warp w of a CTA: channels (w & 3) * 32 + lane of the CTA's 128-channel block, rows in chunks of 32: lane l resolves row
+// chunk*32 + l once (pair row, point, neighbour -> three element offsets), and the warp takes them by shuffle, 8 rows at a time,
+// so no index arithmetic is repeated per channel.
+constexpr int EGL_THREADS = 512;
+template <int CT>
+__global__ void __launch_bounds__(EGL_THREADS)
+edge_gamma_lif_kernel(const float* __restrict__ WP, const int32_t* __restrict__ pid, const float* __restrict__ QK,
+                      const int32_t* __restrict__ idx, int kk, int ldi, int Mpts, int64_t E, int C_rt, const float* __restrict__ bias,
+                      const float* __restrict__ scale, const float* __restrict__ shift, const float* __restrict__ np, int T,
+                      __half* __restrict__ out, const uint8_t* __restrict__ tab, uint32_t tab_stride, int64_t plane) {
+  extern __shared__ __align__(16) uint8_t epf_sm[];
+  const int C = CT ? CT : C_rt;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int cl = (warp & 3) * 32 + lane, part = warp >> 2;
+  const int c = blockIdx.y * 128 + cl;
+  const bool cv = c < C;
+  const int cc = cv ? c : 0;
+  lif_table_load(tab + (size_t)blockIdx.y * tab_stride, epf_sm, tab_stride, tid, EGL_THREADS);
+  const uint32_t lt_desc = (uint32_t)__cvta_generic_to_shared(epf_sm) + (uint32_t)cl * 8u;
+  const float sc = scale[cc];
+  const NeuronParams p{np[cc], np[C + cc], np[2 * C + cc], np[3 * C + cc]};
+  const float bx = fmaf(bias[cc], sc, shift[cc]) - p.th0;
+  __syncthreads();
+  if (!cv) return;                                                // whole warps: C is a multiple of 32
+  const float* wq = QK + c;
+  const float* wk = QK + C + c;
+  const float* wp = WP + c;
+  const int64_t nch = (E + 31) / 32;
+  for (int64_t ch = (int64_t)blockIdx.x * 4 + part; ch < nch; ch += (int64_t)gridDim.x * 4) {
+    const int64_t r0 = ch * 32;
+    uint32_t po, qo, ko;                                         // this lane's row: element offsets of WP, Wq and Wk
+    {
+      const uint32_t e = (uint32_t)(r0 + lane < E ? r0 + lane : E - 1);
+      const uint32_t pt = e / (uint32_t)kk, jj = e - pt * (uint32_t)kk;
+      const uint32_t nb = (pt / (uint32_t)Mpts) * (uint32_t)Mpts + (uint32_t)idx[(size_t)pt * ldi + jj];
+      po = (uint32_t)pid[e] * (uint32_t)C; qo = pt * (uint32_t)(2 * C); ko = nb * (uint32_t)(2 * C);
+    }
+    const int nrow = (int)(E - r0 < 32 ? E - r0 : 32);
+#pragma unroll
+    for (int g = 0; g < 4; ++g) {
+      if (g * 8 >= nrow) break;                                   // warp-uniform
+      float u[8];
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const uint32_t a = __shfl_sync(0xffffffffu, po, g * 8 + j), b = __shfl_sync(0xffffffffu, qo, g * 8 + j),
+                       d = __shfl_sync(0xffffffffu, ko, g * 8 + j);
+        u[j] = fmaf(wp[a], sc, fmaf(wq[b] - wk[d], sc, bx));
+      }
+      lif_rows<1, 8>(u, p, T, lt_desc);
+      store_h<1, 8>(out + (r0 + g * 8) * C + c, C, plane, u, nrow - g * 8);
+    }
   }
 }
 
@@ -471,6 +579,74 @@ int launch_fn_head(const float* H, int K, int64_t S, const float* W, const float
                    const float* lnb, float* out, cudaStream_t st) {
   if (S == 0) return 0;
   fn_head_kernel<<<(unsigned)ceil_div(S * 32, 256), 256, 0, st>>>(H, K, S, W, b, lnw, lnb, out);
+  SAPCU_LAUNCH_CHECK();
+  return 0;
+}
+
+}  // namespace sapcu
+
+namespace sapcu {
+
+#define SAPCU_TRY_RC(e) do { const int _r = (e); if (_r) return _r; } while (0)
+
+namespace {
+// persistent grid: as many CTAs per channel block as fit the SMs, never more than `steps` (rows / rows a CTA takes per step)
+template <class K> int epf_grid(K kern, size_t smem, int nblk, int64_t steps, dim3& grid) {
+  SAPCU_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+  int occ = 1;
+  SAPCU_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, EPF_THREADS, smem));
+  if (occ < 1) occ = 1;
+  int64_t gx = ((int64_t)kNumSMs * occ + nblk - 1) / nblk;
+  if (gx > steps) gx = steps;
+  if (gx < 1) gx = 1;
+  grid = dim3((unsigned)gx, (unsigned)nblk);
+  return 0;
+}
+}  // namespace
+
+int launch_pair_pos_lif(const float4* delta, const int* U_dev, int64_t rows, int C, const float* W, const float* bias,
+                        const float* scale, const float* shift, const float* np, int T, float* out_h, const float* tab,
+                        uint32_t tab_stride, cudaStream_t st) {
+  if (rows == 0) return 0;
+  SAPCU_REQUIRE(tab != nullptr && tab_stride > 0 && tab_stride <= LT_SMEM_BUDGET, "pair_pos_lif: needs the layer's LIF table");
+  const size_t smem = tab_stride;
+  const int nblk = (int)ceil_div(C, 128);
+  const uint8_t* tabp = reinterpret_cast<const uint8_t*>(tab);
+  __half* o = reinterpret_cast<__half*>(out_h);
+  const int64_t plane = rows * (int64_t)C;
+  dim3 grid;
+#define SAPCU_PPL_GO(CQ)                                                                                                \
+  do {                                                                                                                  \
+    SAPCU_TRY_RC(epf_grid(pair_pos_lif_kernel<CQ>, smem, nblk, ceil_div(rows, 16), grid));                              \
+    pair_pos_lif_kernel<CQ><<<grid, EPF_THREADS, smem, st>>>(delta, U_dev, C, W, bias, scale, shift, np, T, o, tabp, tab_stride, plane); \
+  } while (0)
+  if (C == 128) SAPCU_PPL_GO(128); else if (C == 256) SAPCU_PPL_GO(256); else if (C == 512) SAPCU_PPL_GO(512); else SAPCU_PPL_GO(0);
+#undef SAPCU_PPL_GO
+  SAPCU_LAUNCH_CHECK();
+  return 0;
+}
+
+int launch_edge_gamma_lif(const float* WP, const int32_t* pid, const float* QK, const int32_t* idx, int kk, int ldi, int Mpts,
+                          int64_t rows, int C, const float* bias, const float* scale, const float* shift, const float* np, int T,
+                          float* out_h, const float* tab, uint32_t tab_stride, cudaStream_t st) {
+  if (rows == 0) return 0;
+  SAPCU_REQUIRE(tab != nullptr && tab_stride > 0 && tab_stride <= LT_SMEM_BUDGET, "edge_gamma_lif: needs the layer's LIF table");
+  SAPCU_REQUIRE(C % 32 == 0 && kk >= 1 && Mpts >= 1 && rows % ((int64_t)Mpts * kk) == 0, "edge_gamma_lif: edge rows must be whole patches, C %% 32 == 0");
+  SAPCU_REQUIRE(rows < (1ll << 31) && (rows / kk) * 2 * C < (1ll << 32) && rows * C < (1ll << 32), "edge_gamma_lif: element offsets must fit 32 bits");
+  const size_t smem = tab_stride;
+  const int nblk = (int)ceil_div(C, 128);
+  const uint8_t* tabp = reinterpret_cast<const uint8_t*>(tab);
+  __half* o = reinterpret_cast<__half*>(out_h);
+  const int64_t plane = rows * (int64_t)C;
+  dim3 grid;
+#define SAPCU_EGL_GO(CQ)                                                                                                \
+  do {                                                                                                                  \
+    SAPCU_TRY_RC(epf_grid(edge_gamma_lif_kernel<CQ>, smem, nblk, ceil_div(rows, 128), grid));                                \
+    edge_gamma_lif_kernel<CQ><<<grid, EGL_THREADS, smem, st>>>(WP, pid, QK, idx, kk, ldi, Mpts, rows, C, bias, scale, shift, np, T, \
+                                                               o, tabp, tab_stride, plane);                             \
+  } while (0)
+  if (C == 128) SAPCU_EGL_GO(128); else if (C == 256) SAPCU_EGL_GO(256); else if (C == 512) SAPCU_EGL_GO(512); else SAPCU_EGL_GO(0);
+#undef SAPCU_EGL_GO
   SAPCU_LAUNCH_CHECK();
   return 0;
 }

@@ -33,8 +33,10 @@ struct Bump {
 struct FnPlan {
   int32_t* idx; uint32_t* idx8; float *F0, *FCAT, *X, *QKV, *QK, *E1, *E2, *E3, *RES, *R1, *G, *GM, *H0, *H1, *H2, *H3;
   size_t bytes; int kmax; int Dl, kl;
+  PairBufs pairs;        // sapcu_fn_forward_indexed: the chunk's pair table (Ncloud > 0)
 };
-FnPlan fn_plan(const FnNet& f, int64_t s, int M, void* base) {
+// Ncloud > 0: also the pair table of a chunk whose patch points are rows of a cloud of Ncloud points
+FnPlan fn_plan(const FnNet& f, int64_t s, int M, void* base, int64_t Ncloud = 0) {
   FnPlan p; Bump b(base);
   const int64_t P = s * M;
   p.kmax = 0; size_t emax = 0;
@@ -52,6 +54,13 @@ FnPlan fn_plan(const FnNet& f, int64_t s, int M, void* base) {
   p.RES = b.take<float>(P * 512); p.R1 = b.take<float>(P * 512);
   p.G = b.take<float>(P * f.emb); p.GM = b.take<float>(s * f.emb);
   p.H0 = b.take<float>(s * 2048); p.H1 = b.take<float>(s * 1024); p.H2 = b.take<float>(s * 512); p.H3 = b.take<float>(s * 256);
+  if (Ncloud > 0) {
+    int kk[3];
+    for (int i = 0; i < 3; ++i) kk[i] = f.blk[i].k < M ? f.blk[i].k : M;
+    char* pb = b.take<char>(0);
+    p.pairs = pair_plan(P, p.kmax, kk, Ncloud, base ? pb : nullptr);
+    b.off += p.pairs.bytes;
+  }
   p.bytes = align_up(b.off, 256);
   p.Dl = f.blk[2].D; p.kl = f.blk[2].k < M ? f.blk[2].k : M;
   return p;
@@ -84,9 +93,9 @@ FdPlan fd_plan(const FdNet& f, int64_t s, int M, void* base) {
   return p;
 }
 
-int64_t pick_chunk(const sapcu_model* m, int64_t S, int M, size_t ws_bytes) {
+int64_t pick_chunk(const sapcu_model* m, int64_t S, int M, size_t ws_bytes, int64_t Ncloud = 0) {
   auto need = [&](int64_t s) {
-    return m->kind == SAPCU_MODEL_FN ? fn_plan(m->fn, s, M, nullptr).bytes : fd_plan(m->fd, s, M, nullptr).bytes;
+    return m->kind == SAPCU_MODEL_FN ? fn_plan(m->fn, s, M, nullptr, Ncloud).bytes : fd_plan(m->fd, s, M, nullptr).bytes;
   };
   if (need(S) <= ws_bytes) return S;
   int64_t lo = 0, hi = S;   // need(lo) fits (lo = 0 trivially), need(hi) does not
@@ -112,6 +121,7 @@ struct G {
       w.bytes = (double)g.R * g.K * 4.0 + out_rows * g.N * 4.0 + (double)g.N * g.K * 4.0;
       if (g.at_pos) w.bytes += (double)g.R * g.N * 4.0;             // pos rows read by the fused attention tail
     }
+    if (g.R_dev) { w = ProfWork{}; w.gemm = true; }          // rows counted on the device: no algorithmic work recorded
     const bool prof = prof_begin(st, g.label, w, &slot);
     int rc;
     g.tc_passes = passes();
@@ -163,7 +173,11 @@ struct BlockPlan {
   bool attn_out = false; // fc_gamma2 with the fused softmax + weighted-sum tail
 };
 
-int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* normals, const FnPlan& p, int mode, int stop_block, cudaStream_t st) {
+// Where the chunk's patch points come from (sapcu_fn_forward_indexed): gidx[s*ldg + i] = cloud row of patch point i
+struct PatchSource { const double* cloud = nullptr; int64_t N = 0; const int32_t* gidx = nullptr; int64_t ldg = 0; };
+
+int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* normals, const FnPlan& p, int mode, int stop_block, cudaStream_t st,
+             const PatchSource* src = nullptr) {
   const FnNet& f = mdl->fn;
   const int64_t P = s * M;
   const bool precise = mode == SAPCU_MODE_FP32;
@@ -171,6 +185,10 @@ int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
   { ProfWork w; w.flops = (double)s * M * M * 3; w.bytes = (double)P * (12 + 4.0 * p.kmax);
     SAPCU_PROF(st, "fn.intra_knn(xyz)", w, launch_intra_knn(xyz, 3, s, M, 3, p.kmax, p.idx, st)); }
   if (mode != SAPCU_MODE_FP32 && M <= 256) SAPCU_TRY(launch_pack_idx_u8(p.idx, p.kmax, P, p.idx8, st));
+  // the pair table serves the blocks that evaluate pos once per distinct point pair (see `pairs` below), built by the first
+  // of them (parity-grade mode only: in the fast mode the per-edge schedule measured faster, 112 vs 115 ms per 8,192 seeds)
+  const bool indexed = src && mode == SAPCU_MODE_TC;
+  bool table_built = false;
   { ProfWork w; w.elsteps = (double)P * 64 * f.T_enc; w.bytes = (double)P * (12 + 256);
     SAPCU_PROF(st, "fn.conv1+lif", w, launch_pointwise3_lif(false, precise, xyz, nullptr, 0, 0, M, P, 64, f.conv1.W, f.conv1.bias, f.conv1.scale,
                                   f.conv1.shift, f.snn_init.np, f.T_enc, p.F0, st)); }
@@ -220,8 +238,8 @@ int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
       a.Q = p.QK; a.Kf = p.QK + D; a.ldq = 2 * D; a.idx = p.idx; a.ldi = p.kmax; a.kk = kk; a.Mpts = M; a.edge_bias = true;
       return a;
     };
-    auto gamma2_args = [&](const BlockPlan& q) {
-      GemmArgs a = edge(g.args(k.fc_gamma2, p.E1, D, E, p.RES, D, ACT_NONE, nullptr, 0, nullptr, 0, true), q.gamma, 0, nullptr, false);
+    auto gamma2_args = [&](const BlockPlan& q, float* gin = nullptr) {
+      GemmArgs a = edge(g.args(k.fc_gamma2, gin ? gin : p.E1, D, E, p.RES, D, ACT_NONE, nullptr, 0, nullptr, 0, true), q.gamma, 0, nullptr, false);
       a.idx = p.idx; a.ldi = p.kmax; a.kk = kk; a.Mpts = M; a.idx8 = p.idx8; a.ldi8w = (p.kmax + 3) / 4;
       a.at_pos = q.pos32 ? p.E3 : p.E2; a.pos_h2 = q.pos != 0 && !q.pos32;
       a.at_v = p.QKV + 2 * D; a.at_ldv = 3 * D; a.at_sqrt = sq;
@@ -284,12 +302,62 @@ int fn_chunk(const sapcu_model* mdl, const float* xyz, int64_t s, int M, float* 
       return q;
     };
     const BlockPlan q = plan();
+    // Pair schedule (indexed entry): pos = LIF(BN(W_d2 LIF(BN(W_d (p_i - p_j))))) is a function of the offset alone, and fc_gamma's
+    // first layer is linear, so fc_delta, fc_delta2 and W_gamma pos run once per distinct point pair of the chunk (U_b rows,
+    // counted on the device) on the engines and flavours the per-edge launches use; per edge remain the table-flavour
+    // epilogue of fc_gamma (edge_gamma_lif) and the attention tail, which reads pos through pid.  Buffers: h -> E1, pos ->
+    // E2 (+ its fp32 copy in E3 when the tail reads that), W_gamma pos -> whichever of E1 / E3 is free, fc_gamma's spikes ->
+    // the other free one.
+    Layer Lwp = k.fc_gamma;
+    Lwp.bias = nullptr; Lwp.scale = nullptr; Lwp.shift = nullptr;
+    float* const WPbuf = q.pos32 ? p.E1 : p.E3;
+    float* const GAbuf = q.pos32 ? p.E2 : p.E1;
+    auto wp_args = [&]() {
+      GemmArgs a = edge(g.args(Lwp, p.E2, D, E, WPbuf, D, ACT_NONE, nullptr, 0, nullptr, 0, true), q.pos, 0, nullptr, false);
+      a.R_dev = p.pairs.U + b;
+      return a;
+    };
+    const bool pairs = indexed && q.attn_in && q.attn_out && q.tab_gamma &&
+                       q.pos == 1 && q.gamma == 1 && q.pos32 && sup2(wp_args()) && gemm_tc2_fp16x3(wp_args());
     mdl->tap_snn1.store(q.x_planes, std::memory_order_relaxed);
     mdl->tap_delta2.store(q.pos, std::memory_order_relaxed);
     mdl->tap_gamma.store(q.gamma, std::memory_order_relaxed);
     // ---- the block's launches
     SAPCU_TRY(g.L("fn.fc1+lif").run(fc1_args(q), A_PLAIN));
     SAPCU_TRY(g.L("fn.qkv+lif").run(qkv_args(q), A_PLAIN));
+    if (pairs && !table_built) {
+      int* err = tc_err_flag();
+      SAPCU_REQUIRE(err != nullptr, "fn_forward_indexed: cannot allocate the error flag");
+      ProfWork w; w.bytes = (double)P * p.kmax * 40.0;
+      SAPCU_PROF(st, "fn.edge_pairs", w, build_pairs(p.pairs, p.idx, M, src->gidx, src->ldg, src->cloud, src->N, err, st));
+      table_built = true;
+    }
+    if (pairs) {
+      const Neuron& n = k.snn_delta;
+      ProfWork w0;                                       // pair rows: counted on the device only, no algorithmic work recorded
+      SAPCU_PROF(st, "fn.fc_delta(K=3)+lif (pairs)", w0,
+                 launch_pair_pos_lif(p.pairs.delta[b], p.pairs.U + b, E, D, k.fc_delta.W, k.fc_delta.bias, k.fc_delta.scale,
+                                     k.fc_delta.shift, n.np, 4, p.E1, n.tab, n.tab_stride, st));
+      GemmArgs d2 = delta2_args(q);
+      d2.R_dev = p.pairs.U + b;
+      SAPCU_TRY(g.L("fn.fc_delta2+lif (pairs)").run(d2, A_PLAIN));
+      Layer Lw = k.fc_gamma;
+      Lw.bias = nullptr; Lw.scale = nullptr; Lw.shift = nullptr;
+      for (int h = 0; h < 2; ++h)   // [W q | W k], [P, 2D]
+        SAPCU_TRY(g.L("fn.fc_gamma(Wq|Wk per point)").layer(Lw, p.QKV + h * D, 3 * D, P, p.QK + h * D, 2 * D, ACT_NONE));
+      SAPCU_TRY(g.L("fn.fc_gamma(W pos per pair)").run(wp_args(), A_PLAIN));
+      const Neuron& ng = k.snn_gamma;
+      ProfWork w1; w1.elsteps = (double)E * D * 4; w1.bytes = (double)E * D * (q.gamma == 2 ? 2.0 : 4.0);
+      SAPCU_PROF(st, "fn.edge_gamma+lif", w1,
+                 launch_edge_gamma_lif(WPbuf, p.pairs.pid[b], p.QK, p.idx, kk, p.kmax, M, E, D, k.fc_gamma.bias, k.fc_gamma.scale,
+                                       k.fc_gamma.shift, ng.np, 4, GAbuf, ng.tab, ng.tab_stride, st));
+      GemmArgs a2 = gamma2_args(q, GAbuf);
+      a2.at_pid = p.pairs.pid[b];
+      SAPCU_TRY(g.L("fn.fc_gamma2+softmax+sum(attention tail)").run(a2, A_PLAIN));
+      SAPCU_TRY(g.L("fn.out_proj").layer(k.out_proj, p.RES, D, P, p.R1, D, ACT_NONE));
+      SAPCU_TRY(g.L("fn.fc2+residual").layer(k.fc2, p.R1, D, P, p.FCAT + 64 * b, 192, ACT_NONE, nullptr, 0, fin, ldin));
+      continue;
+    }
     {   // pos-enc layer 1 (fc_delta, K = 3) into E1: edge_pos_lif_fast writes one plane, or (hi, lo) planes from the table
       const Neuron& n = k.snn_delta;
       ProfWork w; w.elsteps = (double)E * D * 4; w.bytes = (double)E * D * (q.delta == 2 ? 2.0 : 4.0);
@@ -500,6 +568,68 @@ int sapcu_fn_forward(const sapcu_model* m, const float* d_patches, int64_t S, in
     SAPCU_TRY(fn_chunk(m, d_patches + s0 * M * 3, s, M, d_normals + s0 * 3, p, mode & 0xFF, mode >> 8, st));
   }
   if ((mode & 0xFF) != SAPCU_MODE_FP32) SAPCU_TRY(gemm_tc_check(st));
+  return 0;
+}
+
+size_t sapcu_fn_indexed_workspace_bytes(const sapcu_model* m, int64_t S, int M, int64_t N, int mode) {
+  if (!m || m->kind != SAPCU_MODEL_FN || S < 0 || M < 1 || N < 1) return 0;
+  if (S == 0) S = 1;
+  return fn_plan(m->fn, S, M, nullptr, mode == SAPCU_MODE_TC ? N : 0).bytes;    // the pair table serves SAPCU_MODE_TC only
+}
+
+// Test hook: the pair table of `graph` ([S*M, kmax] patch-local neighbour lists, as intra_knn writes them) for neighbour counts
+// kk[3], written into d_ws; h_off[0..6] = byte offsets of pid_0..2 ([S*M*kk_b] int32), delta_0..2 ([U_b] float4), U ([3] int32).
+size_t sapcu_pair_table_workspace_bytes(int64_t S, int M, int kmax, const int* kk, int64_t N) {
+  if (S < 1 || M < 1 || kmax < 1 || !kk || N < 1) return 0;
+  return pair_plan(S * M, kmax, kk, N, nullptr).bytes;
+}
+int sapcu_pair_table(const int32_t* d_graph, int64_t S, int M, int kmax, const int* kk, const int32_t* d_gidx, int64_t ld_gidx,
+                     const double* d_cloud, int64_t N, void* d_ws, size_t ws_bytes, int64_t* h_off, void* stream) {
+  SAPCU_REQUIRE(d_graph && kk && d_gidx && d_cloud && d_ws && h_off && S >= 1 && M >= 1 && kmax >= 1 && kmax <= M && ld_gidx >= M && N >= 1,
+                "pair_table: bad argument");
+  for (int b = 0; b < 3; ++b) SAPCU_REQUIRE(kk[b] >= 1 && kk[b] <= kmax, "pair_table: need 1 <= kk <= kmax");
+  SAPCU_REQUIRE(pair_key_fits(N, kmax), "pair_table: %lld points x %d ranks do not fit a 64-bit pair key", (long long)N, kmax);
+  const PairBufs q = pair_plan(S * M, kmax, kk, N, d_ws);
+  SAPCU_REQUIRE(q.bytes <= ws_bytes, "pair_table: workspace of %zu bytes, need %zu", ws_bytes, q.bytes);
+  int* err = tc_err_flag();
+  SAPCU_REQUIRE(err != nullptr, "pair_table: cannot allocate the error flag");
+  SAPCU_TRY(build_pairs(q, d_graph, M, d_gidx, ld_gidx, d_cloud, N, err, reinterpret_cast<cudaStream_t>(stream)));
+  const char* base = reinterpret_cast<const char*>(d_ws);
+  for (int b = 0; b < 3; ++b) {
+    h_off[b] = reinterpret_cast<const char*>(q.pid[b]) - base;
+    h_off[3 + b] = reinterpret_cast<const char*>(q.delta[b]) - base;
+  }
+  h_off[6] = reinterpret_cast<const char*>(q.U) - base;
+  return gemm_tc_check(reinterpret_cast<cudaStream_t>(stream));
+}
+
+int sapcu_fn_forward_indexed(const sapcu_model* m, const float* d_patches, int64_t S, int M, const double* d_cloud, int64_t N,
+                             const int32_t* d_gidx, int64_t ld_gidx, float* d_normals, void* d_ws, size_t ws_bytes, int mode,
+                             void* stream) {
+  SAPCU_TRY(check_common(m, SAPCU_MODEL_FN, d_patches, S, M, d_normals, d_ws, mode));
+  SAPCU_REQUIRE((mode >> 8) == 0, "fn_forward_indexed: no debug field");
+  if (S == 0) return 0;
+  SAPCU_REQUIRE(M != 3, "fn_forward_indexed: M == 3 is ambiguous in the reference ([B,3,N] layout) and unsupported");
+  SAPCU_REQUIRE(d_cloud && d_gidx && N >= 1 && ld_gidx >= M, "fn_forward_indexed: need the cloud, N >= 1 and a gidx row stride >= M");
+  SAPCU_REQUIRE(N <= (1ll << 31), "fn_forward_indexed: cloud of %lld points exceeds 32-bit point indices", (long long)N);
+  {
+    int kmax = 0;
+    for (int b = 0; b < 3; ++b) { const int kb = m->fn.blk[b].k < M ? m->fn.blk[b].k : M; kmax = kb > kmax ? kb : kmax; }
+    SAPCU_REQUIRE(pair_key_fits(N, kmax), "fn_forward_indexed: a cloud of %lld points needs more than the 64 bits of a pair key", (long long)N);
+  }
+  // the pair table serves the parity-grade schedule only: the other modes run exactly as sapcu_fn_forward
+  const int64_t Nc = mode == SAPCU_MODE_TC ? N : 0;
+  const int64_t chunk = pick_chunk(m, S, M, ws_bytes, Nc);
+  if (chunk < 1) { set_error("fn_forward_indexed: workspace of %zu bytes cannot hold one patch (need %zu)", ws_bytes, sapcu_fn_indexed_workspace_bytes(m, 1, M, N, mode)); return SAPCU_EWORKSPACE; }
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  for (int64_t s0 = 0; s0 < S; s0 += chunk) {
+    const int64_t s = (S - s0) < chunk ? (S - s0) : chunk;
+    const FnPlan p = fn_plan(m->fn, s, M, d_ws, Nc);
+    PatchSource src;
+    src.cloud = d_cloud; src.N = N; src.gidx = d_gidx + s0 * ld_gidx; src.ldg = ld_gidx;
+    SAPCU_TRY(fn_chunk(m, d_patches + s0 * M * 3, s, M, d_normals + s0 * 3, p, mode, 0, st, Nc ? &src : nullptr));
+  }
+  if (mode != SAPCU_MODE_FP32) SAPCU_TRY(gemm_tc_check(st));
   return 0;
 }
 

@@ -54,6 +54,9 @@ struct GemmArgs {
   // of x * 2^13; lif_tab: tabulated LIF^T chain of the epilogue's neuron (nullptr: reduced-MUFU recurrence)
   bool fast = false; const float* lif_tab = nullptr; uint32_t lif_tab_stride = 0;
   bool edge_bias = false;   // tensor-core engines, A_PLAIN: add Q[pt,c] - Kf[nb,c] (per-point products) to the accumulator, see tc_ptx.cuh
+  // 2-CTA tensor-core engine: rows actually present, in device memory (R is then the capacity the buffers and TMA maps are
+  // sized for); at_pid: the fused attention tail reads pos row at_pid[e] for edge e (pos held once per distinct point pair)
+  const int* R_dev = nullptr; const int32_t* at_pid = nullptr;
   int group = 0;   // 0 or 32
   const char* label = "gemm";   // kernel label of the live profiler (sapcu_profile_report)
 };

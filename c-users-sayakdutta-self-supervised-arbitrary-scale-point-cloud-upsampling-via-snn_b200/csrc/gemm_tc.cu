@@ -408,6 +408,7 @@ int launch_gemm_tc(const GemmArgs& g, int amode, cudaStream_t st) {
   SAPCU_REQUIRE(gemm_tc_supported(g, amode), "gemm_tc: unsupported problem");
   int* err = tc_err_flag();
   SAPCU_REQUIRE(err != nullptr, "gemm_tc: cannot allocate the watchdog flag");
+  SAPCU_REQUIRE(!g.R_dev && !g.at_pid, "gemm_tc: device-side row counts and pair-indexed pos are 2-CTA engine features");
   const bool presplit = g.Whi != nullptr && g.Wlo != nullptr;
   CUtensorMap mw, mwlo, mx;
   int rc = tc_make_map(&mw, presplit ? g.Whi : g.W, g.N, g.K, g.K, TC_BM);
@@ -425,6 +426,7 @@ int launch_gemm_tc(const GemmArgs& g, int amode, cudaStream_t st) {
   p.pool = nullptr; p.pool_T = 0; p.pool_rows = 0; p.acc_scale = 1.0f; p.x_scale = 1.0f; p.out_h2 = 0; p.pos_h2 = 0;
   p.Y2 = nullptr; p.idx8 = g.idx8; p.ldi8w = g.ldi8w; p.at_pos = g.at_pos; p.at_v = g.at_v; p.at_ldv = g.at_ldv; p.at_sqrt = g.at_sqrt; p.tile_rows = tile_rows;
   p.split_w = presplit ? 0 : 1; p.passes = g.tc_passes == 1 ? 1 : 3;
+  p.at_pid = nullptr; p.R_dev = nullptr;   // pair-indexed pos and device-side row counts: 2-CTA engine only
   const int64_t total = p.n_tiles * p.m_tiles;
   const int grid = (int)(total < kNumSMs ? total : kNumSMs);
   if (g.at_pos)
@@ -448,7 +450,10 @@ int gemm_tc_check(cudaStream_t st) {
   int* h;
   { std::lock_guard<std::mutex> lk(g_flag_mu); h = g_flag_host[dev]; }
   if (h && *reinterpret_cast<volatile int*>(h)) {
+    const int v = *reinterpret_cast<volatile int*>(h);
     *reinterpret_cast<volatile int*>(h) = 0;
+    // bit 1: a pair table met a patch point index outside its cloud (edge_pairs.cu); else the pipeline watchdog (value 1)
+    if (v & 2) { set_error("fn_forward_indexed / pair_table: a patch point index lies outside the cloud"); return -1; }   // SAPCU_EINVAL
     set_error("gemm_tc: pipeline watchdog fired (mbarrier protocol stall)");
     return -2;
   }

@@ -19,4 +19,5 @@ bool gemm_tc2_fp16x3(const GemmArgs& g);
 // layers, output are single fp16 planes of x * 2^13)
 bool gemm_tc2_fast(const GemmArgs& g);
 bool gemm_tc2_fast_tf32(const GemmArgs& g);
+int* tc_err_flag();   // the device's mapped error flag (pipeline watchdog, pair-table index check)
 }  // namespace sapcu

@@ -222,8 +222,10 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant
   const uint32_t rank = CG == 2 ? __shfl_sync(0xffffffffu, cluster_ctarank(), 0) : 0u;  // 0 = leader
   const int64_t pair = blockIdx.x / CG, npairs = gridDim.x / CG;
   const int nk = p.K / BKE;
-  const int64_t total_tiles = p.n_tiles * p.m_tiles;       // m_tiles = N / 256 (channel pairs), n_tiles = ceil(R / tile_rows)
   const int TR = p.tile_rows;                              // rows a tile advances by (256; whole points only when EXTRA == 3)
+  // m_tiles = N / 256 (channel pairs), n_tiles = ceil(R / tile_rows); R_dev: only the row tiles that hold the rows present
+  // (every role reads the same count, so the tile walk stays identical across them)
+  const int64_t total_tiles = (p.R_dev ? min(p.n_tiles, ((int64_t)*p.R_dev + TR - 1) / TR) : p.n_tiles) * p.m_tiles;
   constexpr int HALF = T2_BN / CG;                         // rows staged by each CTA: the MMA always spans 256 rows
   // instruction descriptor: D = F32, A = B = TF32 (2) or F16 (0), K-major, M = 256 (pair), N = 256
   constexpr uint32_t idesc = (1u << 4) | ((H16 ? 0u : 2u) << 7) | ((H16 ? 0u : 2u) << 10) | ((uint32_t)(T2_BN >> 3) << 17) | ((uint32_t)(CW >> 4) << 24);
@@ -462,8 +464,9 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant
             const int64_t row0 = (tn / p.m_tiles) * TR;
             const int cb = (int)(tn % p.m_tiles) * CW + (int)rank * 128;
             for (int i = (warp - T2_EPI_WARP0) * 32 + lane; i < TR * 4; i += T2_EPI * 32) {
-              const int64_t row = row0 + (i >> 2);
-              if (row >= p.R) continue;
+              const int64_t e = row0 + (i >> 2);
+              if (e >= p.R) continue;
+              const int64_t row = p.at_pid ? (int64_t)p.at_pid[e] : e;
               if (p.pos_h2 == 2) { if (!(i & 2)) prefetch_l2(reinterpret_cast<const __half*>(p.at_pos) + row * p.N + cb + (i & 1) * 64); }
               else if (p.pos_h2) prefetch_l2(reinterpret_cast<const __half*>(p.at_pos) + ((i & 2) ? p.R * (int64_t)p.N : 0) + row * p.N + cb + (i & 1) * 64);
               else prefetch_l2(p.at_pos + row * p.N + cb + (i & 3) * 32);
@@ -732,7 +735,7 @@ int launch_gemm_tc2(const GemmArgs& g, cudaStream_t st) {
   SAPCU_REQUIRE(!fast || (g.x_h2 && g.lda == g.K && (!g.out_h2 || (g.act == ACT_LIF && g.ldc == g.N))), "gemm_tc2(fast): needs a single-plane fp16 input with lda == K");
   const bool h16 = fast || gemm_tc2_fp16x3(g);
   const bool pre = h16 && g.x_h2;                            // activations already stored as fp16 (hi, lo) planes
-  SAPCU_REQUIRE(fast || !g.x_h2 || (h16 && g.lda == g.K && (g.at_pos || g.act == ACT_LIF || (g.act == ACT_LEAKY && g.pool))), "gemm_tc2: fp16-plane input needs the fp16x3 path and lda == K");
+  SAPCU_REQUIRE(fast || !g.x_h2 || (h16 && g.lda == g.K && (g.at_pos || g.act == ACT_LIF || g.act == ACT_NONE || (g.act == ACT_LEAKY && g.pool))), "gemm_tc2: fp16-plane input needs the fp16x3 path and lda == K");
   SAPCU_REQUIRE(!g.out_h2 || (g.act == ACT_LIF && g.ldc == g.N), "gemm_tc2: fp16-plane output is a LIF epilogue with ldc == N");
   CUtensorMap mw, mwlo, mx, mx2;
   int rc = h16 ? tc_make_map_f16(&mw, g.Wh, g.N, g.K, 128) : tc_make_map(&mw, g.Whi, g.N, g.K, g.K, 128);
@@ -759,7 +762,7 @@ int launch_gemm_tc2(const GemmArgs& g, cudaStream_t st) {
   p.idx8 = g.idx8; p.ldi8w = g.ldi8w;
   p.at_pos = g.at_pos; p.at_v = g.at_v; p.at_ldv = g.at_ldv; p.at_sqrt = g.at_sqrt; p.tile_rows = tile_rows;
   p.m_tiles = g.N / (128 * cg); p.n_tiles = ceil_div(g.R, tile_rows); p.err = err; p.split_w = 0; p.passes = g.tc_passes == 1 ? 1 : 3;
-  p.out_h2 = g.out_h2 ? 1 : 0; p.pos_h2 = g.pos_h2 ? 1 : 0;
+  p.out_h2 = g.out_h2 ? 1 : 0; p.pos_h2 = g.pos_h2 ? 1 : 0; p.at_pid = g.at_pid; p.R_dev = g.R_dev;
   p.lif_tab = nullptr; p.lif_tab_stride = 0;
   p.x_scale = h16 ? 8192.0f : 1.0f;                         // soft spikes lie in (0, 0.7): x * 2^13 < 2^13, residual * 2^13 >= fp16's normal range
   p.acc_scale = h16 ? g.winv / 8192.0f : 1.0f;
@@ -805,13 +808,14 @@ int launch_gemm_tc2(const GemmArgs& g, cudaStream_t st) {
   }
   if (pre && cg == 1) {
     // 128-channel layer on (hi, lo) planes: the single-CTA flavour (fp16x3 products; LIF table next to ONE 96 KiB stage)
-    SAPCU_REQUIRE(g.at_pos || g.act == ACT_LIF, "gemm_tc2: the single-CTA plane path serves the LIF layers and the attention tail");
+    SAPCU_REQUIRE(g.at_pos || g.act == ACT_LIF || g.act == ACT_NONE, "gemm_tc2: the single-CTA plane path serves the LIF layers, plain products and the attention tail");
     const bool lt = g.act == ACT_LIF && g.lif_tab && g.lif_tab_stride > 0 && g.lif_tab_stride <= LT_SMEM_BUDGET;
     if (lt) { pairs = (pairs / p.m_tiles) * p.m_tiles; p.lif_tab = reinterpret_cast<const uint8_t*>(g.lif_tab); p.lif_tab_stride = g.lif_tab_stride; }
     SAPCU_REQUIRE(pairs >= 1, "gemm_tc2(single-CTA planes): empty grid");
     const size_t smem = (size_t)(lt ? 1 : 2) * 6 * TC_TILE_BYTES + 1024 + 256 + (lt ? g.lif_tab_stride : 0);
     if (g.at_pos)
       return with_kk(g.kk, [&](auto KQ) { return tc_launch<gemm_tc2_kernel<ACT_NONE, 3, decltype(KQ)::value, 2, 0, 1>>(pairs, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p); });
+    if (g.act == ACT_NONE) return tc_launch<gemm_tc2_kernel<ACT_NONE, 0, 1, 2, 0, 1>>(pairs, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
     if (g.edge_bias) return lt ? tc_launch<gemm_tc2_kernel<ACT_LIF, 2, 1, 2, 1, 1>>(pairs, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p) : tc_launch<gemm_tc2_kernel<ACT_LIF, 2, 1, 2, 0, 1>>(pairs, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
     return lt ? tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 2, 1, 1>>(pairs, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p) : tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 2, 0, 1>>(pairs, T2_THREADS, smem, st, mw, mwlo, mx, mx2, p);
   }
@@ -828,6 +832,7 @@ int launch_gemm_tc2(const GemmArgs& g, cudaStream_t st) {
   if (pre) {
     if (g.at_pos) return with_kk(g.kk, [&](auto KQ) { return tc_launch<gemm_tc2_kernel<ACT_NONE, 3, decltype(KQ)::value, 2>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p); });
     if (g.act == ACT_LEAKY) return tc_launch<gemm_tc2_kernel<ACT_LEAKY, 4, 1, 2>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
+    if (g.act == ACT_NONE) return tc_launch<gemm_tc2_kernel<ACT_NONE, 0, 1, 2>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
     if (g.edge_bias) return tc_launch<gemm_tc2_kernel<ACT_LIF, 2, 1, 2>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
     return tc_launch<gemm_tc2_kernel<ACT_LIF, 0, 1, 2>>(grid, T2_THREADS, T2_SMEM_BYTES, st, mw, mwlo, mx, mx2, p);
   }

@@ -26,6 +26,29 @@ int launch_pointwise3_lif(bool edge, bool precise, const float* xyz, const int32
 int launch_edge_pos_lif_fast(const float* xyz, const int32_t* idx, int kk, int ldi, int Mpts, int64_t rows, int C,
                              const float* W, const float* bias, const float* scale, const float* shift, const float* np, int T,
                              float* out_h, const float* tab, uint32_t tab_stride, cudaStream_t st, bool two_planes = false);
+// fc_delta + BN + tabulated LIF^T on the offsets delta[u] of the first *U_dev pair rows, (hi, lo) planes out (capacity `rows`:
+// the lo plane's offset)
+int launch_pair_pos_lif(const float4* delta, const int* U_dev, int64_t rows, int C, const float* W, const float* bias,
+                        const float* scale, const float* shift, const float* np, int T, float* out_h, const float* tab,
+                        uint32_t tab_stride, cudaStream_t st);
+// fc_gamma's BN + tabulated LIF^T per edge from the per-pair product WP[pid[e]] and the per-point edge bias QK (= [W q | W k])
+int launch_edge_gamma_lif(const float* WP, const int32_t* pid, const float* QK, const int32_t* idx, int kk, int ldi, int Mpts,
+                          int64_t rows, int C, const float* bias, const float* scale, const float* shift, const float* np, int T,
+                          float* out_h, const float* tab, uint32_t tab_stride, cudaStream_t st);
+// edge_pairs.cu: the pair table of an fn chunk (views into the workspace; pair_plan(.., nullptr) only sizes it)
+struct PairBufs {
+  int64_t E = 0; int kmax = 0, jb = 0, bits = 0, kk[3] = {0, 0, 0};
+  uint64_t* key[2] = {nullptr, nullptr}; int32_t* val[2] = {nullptr, nullptr};
+  int* flag[3] = {nullptr, nullptr, nullptr};
+  int32_t* pid[3] = {nullptr, nullptr, nullptr};       // [P * kk_b] pair row of every edge of block b
+  float4* delta[3] = {nullptr, nullptr, nullptr};      // [U_b] offsets cloud[gi] - cloud[gj]
+  int* U = nullptr;                                    // [3] pair counts (device)
+  void* tmp = nullptr; size_t tmp_bytes = 0, bytes = 0;
+};
+PairBufs pair_plan(int64_t P, int kmax, const int kk[3], int64_t N, void* base);
+bool pair_key_fits(int64_t N, int kmax);     // the key ((gi * N + gj) << bits(kmax)) | j fits 64 bits
+int build_pairs(const PairBufs& q, const int32_t* idx, int M, const int32_t* gidx, int64_t ldg, const double* cloud, int64_t N,
+                int* err, cudaStream_t st);
 int launch_pack_idx_u8(const int32_t* idx, int ldi, int64_t P, uint32_t* out, cudaStream_t st);
 int launch_attn_out(bool precise, const float* logits, const float* pos, const float* V, int64_t ldv,
                     const int32_t* idx, int ldi, int kk, int Mpts, int64_t P, int D, float sqrt_hd, float* out,

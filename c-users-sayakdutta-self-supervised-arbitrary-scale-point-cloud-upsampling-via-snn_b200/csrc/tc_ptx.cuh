@@ -188,6 +188,8 @@ struct TcParams {
   // EXTRA == 4 (fd conv5, 2-CTA kernel): rows are (point*T + t); the epilogue keeps one running maximum per step and
   // merges them into pool[(patch*T + t), c] with float atomic max -- the [P*T, N] activation never reaches HBM
   float* pool; int pool_T; int64_t pool_rows;     // pool_rows = points per patch * T
+  const int32_t* at_pid;      // EXTRA == 3, optional: pos row of edge e is at_pid[e] (rows of distinct point pairs) instead of e
+  const int* R_dev;           // 2-CTA kernel, optional: rows present (device memory, <= R); tiles past them are skipped
   int pos_h2;                 // EXTRA == 3: at_pos is stored as fp16 (hi, lo) planes of pos * 2^13 ([R, N] halfs each); 2 = hi plane only (fast mode)
   int out_h2;                 // LIF epilogue of the 2-CTA kernel: write Y as fp16 (hi, lo) planes of y * 2^13 (ldc == N, [R, N] each); 2 = hi plane only (fast mode)
   // SAPCU_MODE_FAST, LIF epilogue: tabulated chain (lif_table.cuh): image of the 128-channel block b at lif_tab + b * lif_tab_stride
@@ -231,7 +233,9 @@ __device__ __forceinline__ void edge_fetch8(const TcParams& p, int my_qo, int my
 // the TMEM read and the softmax run under them, the weighted sum consumes them last.
 // NC > 0: the channel count (row stride of pos and of the output) as a compile-time constant -- the KK pos loads of a point
 // become immediate offsets from one base address; NC == 0: run-time p.N.
-template <int KK, int NC = 0>
+// PID: pos is held once per distinct point pair and edge e reads row p.at_pid[e]; lane j fetches the point's j-th row
+// index and the loads take it by shuffle (the KK indices of a point are the same for the whole warp).
+template <int KK, int NC = 0, bool PID = false>
 __device__ __forceinline__ void attn_tail_points(const TcParams& p, uint32_t tmem_cols, int part, int parts, int npts,
                                                  int64_t n_t, int c, float bia, float sc, float sh, float acc_scale) {
   const int64_t Nn = NC ? (int64_t)NC : (int64_t)p.N;
@@ -260,7 +264,10 @@ __device__ __forceinline__ void attn_tail_points(const TcParams& p, uint32_t tme
     const int64_t pt = n_t * npts + pp;
     if (pt >= P_total) break;                                    // warp-uniform
     while (prem >= p.Mpts) { prem -= p.Mpts; patch0 += p.Mpts; }
-    const float* ps = p.at_pos + (pt * KK) * Nn + c;
+    int pidl = 0;
+    if (PID) { const int l = (int)(threadIdx.x & 31); pidl = p.at_pid[pt * KK + (l < KK ? l : KK - 1)]; }
+    // element offset of edge j's pos row from row 0
+    auto roff = [&](int j) -> int64_t { return PID ? (int64_t)__shfl_sync(0xffffffffu, pidl, j) * Nn : (pt * KK + j) * Nn; };
     float vr[KK], pr[KK];
     __half prh[KK];                                              // fast mode: the raw halves, converted only where they are consumed
     // v[nb_j]: one 64-bit base per point, then byte extract (PRMT) + one 32 x 32 -> 64-bit multiply-add (IMAD.WIDE) per neighbour
@@ -275,17 +282,18 @@ __device__ __forceinline__ void attn_tail_points(const TcParams& p, uint32_t tme
       asm("ld.global.f32 %0, [%1];" : "=f"(vr[j]) : "l"(a));     // v was written by an earlier kernel of the stream
     }
     if (p.pos_h2 == 2) {                                         // fast mode: one fp16 plane of pos * 2^13
-      const __half* ph = reinterpret_cast<const __half*>(p.at_pos) + (pt * KK) * Nn + c;
+      const __half* ph = reinterpret_cast<const __half*>(p.at_pos) + c;
 #pragma unroll
-      for (int j = 0; j < KK; ++j) prh[j] = ph[(int64_t)j * Nn];
+      for (int j = 0; j < KK; ++j) prh[j] = ph[roff(j)];
     } else if (p.pos_h2) {
-      const __half* ph = reinterpret_cast<const __half*>(p.at_pos) + (pt * KK) * Nn + c;
+      const __half* ph = reinterpret_cast<const __half*>(p.at_pos) + c;
       const __half* pl = ph + p.R * Nn;
 #pragma unroll
-      for (int j = 0; j < KK; ++j) pr[j] = (__half2float(ph[(int64_t)j * Nn]) + __half2float(pl[(int64_t)j * Nn])) * (1.0f / 8192.0f);
+      for (int j = 0; j < KK; ++j) pr[j] = (__half2float(ph[roff(j)]) + __half2float(pl[roff(j)])) * (1.0f / 8192.0f);
     } else {
+      const float* ps = p.at_pos + c;
 #pragma unroll
-      for (int j = 0; j < KK; ++j) pr[j] = ps[(int64_t)j * Nn];
+      for (int j = 0; j < KK; ++j) pr[j] = ps[roff(j)];
     }
     fetch_row(pt + parts);                                       // indices of this warp's next point (clamped at the end)
     float av[KK];
@@ -312,7 +320,10 @@ template <int KK>
 __device__ __forceinline__ void attn_tail_dispatch(const TcParams& p, uint32_t tmem_cols, int part, int parts, int npts,
                                                    int64_t n_t, int c, float bia, float sc, float sh, float acc_scale) {
   constexpr int NY = KK == 24 ? 128 : KK == 18 ? 256 : KK == 12 ? 512 : 0;
-  if (NY != 0 && p.N == NY && p.ldc == NY) attn_tail_points<KK, NY>(p, tmem_cols, part, parts, npts, n_t, c, bia, sc, sh, acc_scale);
+  if (NY != 0 && p.N == NY && p.ldc == NY) {
+    if (p.at_pid) attn_tail_points<KK, NY, true>(p, tmem_cols, part, parts, npts, n_t, c, bia, sc, sh, acc_scale);
+    else attn_tail_points<KK, NY>(p, tmem_cols, part, parts, npts, n_t, c, bia, sc, sh, acc_scale);
+  } else if (p.at_pid) attn_tail_points<KK, 0, true>(p, tmem_cols, part, parts, npts, n_t, c, bia, sc, sh, acc_scale);
   else attn_tail_points<KK, 0>(p, tmem_cols, part, parts, npts, n_t, c, bia, sc, sh, acc_scale);
 }
 

@@ -123,3 +123,28 @@ class ImprovedSNNNormalEstimation(NativeModel):
                 N.check(N.lib().sapcu_fn_forward(h, N.ptr(x), S, M, N.ptr(out), N.ptr(ws), ws_bytes, self.mode | (int(_stop_after_block) << 8),
                                                  N.stream_ptr(x.device)), "sapcu_fn_forward")
         return out.view(*lead, 3) if lead else out
+
+    @torch.no_grad()
+    def forward_indexed(self, patches, cloud, gidx):
+        """forward() of [S,M,3] patches whose point i of patch s is row gidx[s,i] of `cloud` (f64 [N,3]; the patches are
+        cloud[gidx] - seed): the positional encoding is then evaluated once per distinct pair of cloud points
+        (sapcu_fn_forward_indexed).  gidx: int32 [S, >= M] on the patches' device, rows may be strided."""
+        x = self._prep_input(patches)
+        if x.ndim != 3 or x.shape[2] != 3:
+            raise N.SapcuError("fn forward_indexed expects [S,M,3] patches, got shape %s" % (tuple(patches.shape),))
+        if cloud.dtype != torch.float64 or cloud.ndim != 2 or cloud.shape[1] != 3 or not cloud.is_contiguous():
+            raise N.SapcuError("fn forward_indexed: cloud must be a contiguous float64 [N,3] tensor")
+        S, M = x.shape[0], x.shape[1]
+        if gidx.dtype != torch.int32 or gidx.ndim != 2 or gidx.shape[0] != S or gidx.shape[1] < M or gidx.stride(1) != 1:
+            raise N.SapcuError("fn forward_indexed: gidx must be int32 [S, >= M] with unit column stride")
+        if cloud.device != x.device or gidx.device != x.device:
+            raise N.SapcuError("fn forward_indexed: patches, cloud and gidx must share a device")
+        out = torch.empty(S, 3, dtype=torch.float32, device=x.device)
+        if S:
+            with torch.cuda.device(x.device):
+                h = self._ensure_handle(x.device)
+                ncl = cloud.shape[0]
+                ws, ws_bytes = self._workspace(S, M, x.device, ncloud=ncl)
+                N.check(N.lib().sapcu_fn_forward_indexed(h, N.ptr(x), S, M, N.ptr(cloud), ncl, N.ptr(gidx), gidx.stride(0), N.ptr(out),
+                                                         N.ptr(ws), ws_bytes, self.mode, N.stream_ptr(x.device)), "sapcu_fn_forward_indexed")
+        return out

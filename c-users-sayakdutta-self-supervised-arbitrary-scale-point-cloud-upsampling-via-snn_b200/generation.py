@@ -245,7 +245,10 @@ class Generator3D6(object):
                 p = patches[:n]
                 N.check(L.sapcu_gather_center_rotate(N.ptr(d_cloud), Ncl, N.ptr(d_seeds[s0:]), N.ptr(idx[s0:]), n, K, None,
                                                      N.ptr(p), st), "gather_center")
-                normals[s0:s1] = self.model1(p)
+                if hasattr(self.model1, "forward_indexed"):      # the native shim: pos once per distinct cloud-point pair
+                    normals[s0:s1] = self.model1.forward_indexed(p, d_cloud, idx[s0:s1])
+                else:
+                    normals[s0:s1] = self.model1(p)
                 N.check(L.sapcu_renormalize(N.ptr(normals[s0:]), n, st), "renormalize")
                 N.check(L.sapcu_gather_center_rotate(N.ptr(d_cloud), Ncl, N.ptr(d_seeds[s0:]), N.ptr(idx[s0:]), n, K,
                                                      N.ptr(normals[s0:]), N.ptr(p), st), "gather_center_rotate")

@@ -227,7 +227,29 @@ size_t sapcu_model_workspace_bytes(const sapcu_model* m, int64_t S, int M);
 int sapcu_fn_forward(const sapcu_model* m, const float* d_patches, int64_t S, int M,
                      float* d_normals, void* d_ws, size_t ws_bytes, int mode, void* stream);
 
-/* fd: EnhancedSNNDistanceEstimation.forward([S,M,3]) -> [S] distances (fd/snn_coder.py:853-871).
+/* fn on patches whose points are rows of a cloud: d_cloud = f64 [N,3], d_gidx[s * ld_gidx + i] = cloud row of patch point i
+ * (the seed kNN result the patches were gathered from; with a batch of clouds, rows of their concatenation).  In
+ * SAPCU_MODE_TC the positional encoding of every block whose plan hands pos over as tabulated planes
+ * is evaluated once per distinct (cloud row, cloud row) pair of a chunk instead of once per patch edge, on the offset
+ * (float)(cloud[i] - cloud[j]); everything downstream is bit-for-bit the per-edge schedule on equal offsets.  Other modes
+ * and blocks run exactly as sapcu_fn_forward.  Never synchronises the stream; an index outside [0, N) is never read and
+ * makes this (or the next) check of the device's error flag return SAPCU_EINVAL: the check shares the device's mapped flag
+ * with the pipeline watchdog (sapcu_device_status), so it may surface in the next forward of any model on that device.  The
+ * pair key ((i * N + j) << ceil(log2 kmax)) | rank must fit 64 bits, else SAPCU_EINVAL before any launch (2 ceil(log2 N) +
+ * ceil(log2 kmax) <= 64: up to about 2^29 points).  Workspace: sapcu_fn_indexed_workspace_bytes(m, S, M, N, mode) for one
+ * chunk of all S patches (less chunks the work); only SAPCU_MODE_TC adds the pair table to sapcu_model_workspace_bytes. */
+size_t sapcu_fn_indexed_workspace_bytes(const sapcu_model* m, int64_t S, int M, int64_t N, int mode);
+int sapcu_fn_forward_indexed(const sapcu_model* m, const float* d_patches, int64_t S, int M, const double* d_cloud, int64_t N,
+                             const int32_t* d_gidx, int64_t ld_gidx, float* d_normals, void* d_ws, size_t ws_bytes, int mode,
+                             void* stream);
+/* Test hook of the pair table behind sapcu_fn_forward_indexed: for patch-local neighbour lists d_graph ([S*M, kmax] int32) and
+ * neighbour counts kk[3] (<= kmax) writes pid_b ([S*M*kk_b] int32: pair row of edge (pt, j < kk_b)), delta_b ([U_b] x 4 floats:
+ * (float)(cloud[gi] - cloud[gj]), w = 0) and U ([3] int32) into d_ws at the byte offsets h_off[0..2], h_off[3..5], h_off[6]. */
+size_t sapcu_pair_table_workspace_bytes(int64_t S, int M, int kmax, const int* kk, int64_t N);
+int sapcu_pair_table(const int32_t* d_graph, int64_t S, int M, int kmax, const int* kk, const int32_t* d_gidx, int64_t ld_gidx,
+                     const double* d_cloud, int64_t N, void* d_ws, size_t ws_bytes, int64_t* h_off, void* stream);
+
+/* fd:EnhancedSNNDistanceEstimation.forward([S,M,3]) -> [S] distances (fd/snn_coder.py:853-871).
  * d_forced_idx (nullable): int32 [3][S][M][k] feature-space neighbour lists for blocks 1..3 taken
  * from the oracle ("teacher-forced" parity runs, SURVEY.md section 7 hard-part 4). */
 int sapcu_fd_forward(const sapcu_model* m, const float* d_patches, int64_t S, int M,
