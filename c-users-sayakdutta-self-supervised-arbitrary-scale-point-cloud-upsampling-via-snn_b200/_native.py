@@ -87,6 +87,22 @@ def _build_variant(extra, out):
     return out
 
 
+class GemmCaseArgs(ctypes.Structure):
+    """sapcu_gemm_case_args (include/sapcu_b200.h): one contraction of the forwards for sapcu_gemm_case."""
+    _i, _i64, _f, _p = ctypes.c_int, ctypes.c_int64, ctypes.c_float, ctypes.c_void_p
+    _fields_ = [("amode", _i), ("act", _i), ("T", _i), ("use_table", _i),
+                ("R", _i64), ("K", _i), ("N", _i), ("lda", _i64), ("ldc", _i64), ("ldr", _i64),
+                ("h_w", _p), ("h_bias", _p), ("h_scale", _p), ("h_shift", _p), ("h_params4", _p),
+                ("d_x", _p), ("x_format", _i), ("x_unit", _i), ("fast", _i),
+                ("d_y", _p), ("out_h2", _i), ("d_y2", _p),
+                ("d_residual", _p),
+                ("d_f", _p), ("ldf", _i64), ("C", _i),
+                ("edge_bias", _i), ("d_q", _p), ("d_kf", _p), ("ldq", _i64), ("d_idx", _p), ("ldi", _i), ("kk", _i), ("mpts", _i),
+                ("d_pool", _p), ("pool_T", _i), ("pool_M", _i),
+                ("d_at_pos", _p), ("d_at_v", _p), ("at_ldv", _i64), ("at_sqrt", _f), ("d_at_pid", _p), ("pos_h2", _i),
+                ("d_R_dev", _p), ("tc2_any_rows", _i), ("group", _i)]
+
+
 _SIGS = {
     "sapcu_last_error": (ctypes.c_char_p, []),
     "sapcu_abi_version": (ctypes.c_int, []),
@@ -161,6 +177,9 @@ _SIGS = {
                                        ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]),
     "sapcu_gemm": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_void_p, ctypes.c_int,
                                   ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p]),
+    "sapcu_gemm_case_workspace_bytes": (ctypes.c_size_t, [ctypes.POINTER(GemmCaseArgs)]),
+    "sapcu_gemm_case": (ctypes.c_int, [ctypes.POINTER(GemmCaseArgs), ctypes.c_void_p, ctypes.c_size_t, ctypes.c_int,
+                                       ctypes.c_void_p]),
 }
 
 EXPORTS = tuple(_SIGS)

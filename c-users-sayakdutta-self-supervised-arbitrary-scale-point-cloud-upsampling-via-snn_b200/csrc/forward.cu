@@ -653,6 +653,84 @@ int sapcu_fd_forward(const sapcu_model* m, const float* d_patches, int64_t S, in
   return 0;
 }
 
+}  // extern "C"
+
+// Test hook: one contraction through G::run.  Workspace: W, its tf32 and fp16 splits, bias / scale / shift, the neuron rows,
+// the LIF table and the byte-packed graph of the attention tail, each 256-byte aligned.
+namespace {
+struct CaseWs { float *W, *Whi, *Wlo, *bias, *scale, *shift, *np, *tab; uint16_t *Wh, *Wl; uint32_t* idx8; size_t bytes; };
+CaseWs case_plan(const sapcu_gemm_case_args& a, size_t tab_bytes, void* base) {
+  CaseWs w; Bump b(base);
+  const size_t nk = (size_t)a.N * a.K;
+  w.W = b.take<float>(nk); w.Whi = b.take<float>(nk); w.Wlo = b.take<float>(nk);
+  w.Wh = b.take<uint16_t>((nk + 1) & ~(size_t)1); w.Wl = b.take<uint16_t>((nk + 1) & ~(size_t)1);
+  w.bias = b.take<float>(a.h_bias ? a.N : 0); w.scale = b.take<float>(a.h_scale ? a.N : 0); w.shift = b.take<float>(a.h_shift ? a.N : 0);
+  w.np = b.take<float>(a.h_params4 ? 4 * (size_t)a.N : 0);
+  w.tab = b.take<float>(tab_bytes / 4);
+  const bool pack = a.d_at_pos && a.d_idx && a.kk > 0;
+  w.idx8 = b.take<uint32_t>(pack ? (size_t)(a.R / a.kk) * ((a.ldi + 3) / 4) : 0);
+  w.bytes = align_up(b.off, 256);
+  return w;
+}
+bool case_table(const sapcu_gemm_case_args& a) { return a.use_table && a.act == ACT_LIF && a.h_params4 && a.T >= 1 && a.T <= 16; }
+}  // namespace
+
+extern "C" {
+
+size_t sapcu_gemm_case_workspace_bytes(const sapcu_gemm_case_args* a) {
+  if (!a || a->N < 1 || a->K < 1 || a->R < 0 || (a->d_at_pos && a->kk < 1)) return 0;
+  LifTablePacked t;
+  if (case_table(*a)) lif_table_pack(a->h_params4, a->N, a->T, &t);
+  return case_plan(*a, t.img.size() * 4, nullptr).bytes;
+}
+
+int sapcu_gemm_case(const sapcu_gemm_case_args* a, void* d_ws, size_t ws_bytes, int mode, void* stream) {
+  SAPCU_REQUIRE(a && d_ws && a->R >= 1 && a->K >= 1 && a->N >= 1 && a->h_w && a->d_y && (a->amode == A_EDGECAT ? a->d_f != nullptr : a->d_x != nullptr),
+                "gemm_case: bad argument");
+  SAPCU_REQUIRE(a->amode >= A_PLAIN && a->amode <= A_ATTNIN && a->act >= ACT_NONE && a->act <= ACT_LIF && a->x_format >= 0 && a->x_format <= 2,
+                "gemm_case: bad amode / act / x_format");
+  SAPCU_REQUIRE(a->act != ACT_LIF || (a->h_params4 && a->T >= 1), "gemm_case: a LIF epilogue needs its parameters and T >= 1");
+  SAPCU_REQUIRE(mode >= SAPCU_MODE_FP32 && mode <= SAPCU_MODE_FAST, "gemm_case: unknown mode %d", mode);
+  SAPCU_REQUIRE(!(a->d_idx || a->d_at_pos) || (a->kk >= 1 && a->R % a->kk == 0 && a->ldi >= a->kk && a->mpts >= 1),
+                "gemm_case: edge rows need kk >= 1 dividing R, ldi >= kk and mpts >= 1");
+  LifTablePacked t;
+  if (case_table(*a)) lif_table_pack(a->h_params4, a->N, a->T, &t);
+  const CaseWs w = case_plan(*a, t.img.size() * 4, d_ws);
+  SAPCU_REQUIRE(w.bytes <= ws_bytes, "gemm_case: workspace of %zu bytes, need %zu", ws_bytes, w.bytes);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const size_t nk = (size_t)a->N * a->K;
+  WeightSplit s;
+  split_weights(a->h_w, nk, &s);
+  // pageable sources: each copy returns once its bytes are staged, so the host vectors may go out of scope afterwards
+  auto up = [&](void* dst, const void* src, size_t bytes) { return src && bytes ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st) : cudaSuccess; };
+  SAPCU_CUDA_CHECK(up(w.W, a->h_w, nk * 4));
+  SAPCU_CUDA_CHECK(up(w.Whi, s.hi.data(), nk * 4)); SAPCU_CUDA_CHECK(up(w.Wlo, s.lo.data(), nk * 4));
+  SAPCU_CUDA_CHECK(up(w.Wh, s.h.data(), s.h.size() * 2)); SAPCU_CUDA_CHECK(up(w.Wl, s.l.data(), s.l.size() * 2));
+  SAPCU_CUDA_CHECK(up(w.bias, a->h_bias, (size_t)a->N * 4)); SAPCU_CUDA_CHECK(up(w.scale, a->h_scale, (size_t)a->N * 4));
+  SAPCU_CUDA_CHECK(up(w.shift, a->h_shift, (size_t)a->N * 4)); SAPCU_CUDA_CHECK(up(w.np, a->h_params4, (size_t)a->N * 16));
+  SAPCU_CUDA_CHECK(up(w.tab, t.img.data(), t.img.size() * 4));
+  GemmArgs g;
+  g.A = a->d_x; g.lda = a->lda; g.R = a->R; g.K = a->K; g.N = a->N;
+  g.W = w.W; g.Whi = w.Whi; g.Wlo = w.Wlo; g.Wh = reinterpret_cast<const float*>(w.Wh); g.Wl = reinterpret_cast<const float*>(w.Wl); g.winv = s.winv;
+  g.bias = a->h_bias ? w.bias : nullptr; g.scale = a->h_scale ? w.scale : nullptr; g.shift = a->h_shift ? w.shift : nullptr;
+  g.act = a->act; g.T = a->T; g.nparams = a->h_params4 ? w.np : nullptr;
+  g.residual = a->d_residual; g.ldr = a->ldr; g.Y = a->d_y; g.ldc = a->ldc; g.Y2 = a->d_y2;
+  g.F = a->d_f; g.ldf = a->ldf; g.C = a->C;
+  g.Q = a->d_q; g.Kf = a->d_kf; g.ldq = a->ldq; g.idx = a->d_idx; g.ldi = a->ldi; g.kk = a->kk; g.Mpts = a->mpts;
+  g.edge_bias = a->edge_bias != 0;
+  g.x_h2 = a->x_format != 0; g.x_unit = a->x_unit != 0; g.out_h2 = a->out_h2 != 0; g.fast = a->fast != 0;
+  if (case_table(*a) && t.usable) { g.lif_tab = w.tab; g.lif_tab_stride = t.stride; }
+  g.pool = a->d_pool; g.pool_T = a->pool_T; g.pool_M = a->pool_M;
+  g.at_pos = a->d_at_pos; g.at_v = a->d_at_v; g.at_ldv = a->at_ldv; g.at_sqrt = a->at_sqrt; g.at_pid = a->d_at_pid; g.pos_h2 = a->pos_h2 != 0;
+  if (a->d_at_pos && a->d_idx && mode != SAPCU_MODE_FP32 && a->mpts <= 256) {          // as fn_chunk: the byte-packed graph
+    SAPCU_TRY(launch_pack_idx_u8(a->d_idx, a->ldi, a->R / a->kk, w.idx8, st));
+    g.idx8 = w.idx8; g.ldi8w = (a->ldi + 3) / 4;
+  }
+  g.R_dev = a->d_R_dev; g.tc2_any_rows = a->tc2_any_rows != 0; g.group = a->group;
+  const G run{mode, st};
+  return run.L("gemm_case").run(g, a->amode);
+}
+
 int sapcu_device_status(void) {
   // watchdog flag of the current device, read from host-visible memory (no stream is touched): call after synchronising
   return gemm_tc_check(nullptr) ? SAPCU_ECUDA : 0;

@@ -69,34 +69,15 @@ struct Builder {
     fixes.push_back({dst, off});
     return off;
   }
-  // weight matrix + its tf32 (hi, lo) split for the tensor-core engine: hi = w rounded to 10 mantissa bits
-  // (round-to-nearest, ties away), lo = w - hi (exact in fp32)
+  // weight matrix + its tensor-core splits (split_weights)
   void put_w(Layer& L, const float* w, size_t n) {
     put(w, n, &L.W);
-    std::vector<float> hi(n), lo(n);
-    for (size_t i = 0; i < n; ++i) {
-      uint32_t b; memcpy(&b, &w[i], 4);
-      if ((b & 0x7F800000u) != 0x7F800000u) b = (b + 0x1000u) & 0xFFFFE000u;
-      float h; memcpy(&h, &b, 4);
-      hi[i] = h; lo[i] = w[i] - h;
-    }
-    put(hi.data(), n, &L.Whi); put(lo.data(), n, &L.Wlo);
-    // fp16 (hi, lo) of w * 2^e with max |w| * 2^e in [2^13, 2^14): both halves stay in fp16's normal range for every
-    // weight within 2^-9 of the largest one, smaller ones keep 6e-8 absolute (scaled) precision
-    float mx = 0.0f;
-    for (size_t i = 0; i < n; ++i) if (std::isfinite(w[i])) mx = std::max(mx, std::fabs(w[i]));
-    int e = 0;
-    if (mx > 0.0f) { int ex; std::frexp(mx, &ex); e = 14 - ex; }          // mx = f * 2^ex, f in [0.5, 1)
-    const float sc = std::ldexp(1.0f, e);
-    std::vector<uint16_t> hh((n + 1) & ~(size_t)1), hl((n + 1) & ~(size_t)1);
-    for (size_t i = 0; i < n; ++i) {
-      const float ws = w[i] * sc;                                         // exact (power of two)
-      const uint16_t h = f32_to_f16_rn(ws);
-      hh[i] = h; hl[i] = f32_to_f16_rn(ws - f16_to_f32(h));
-    }
-    put(reinterpret_cast<const float*>(hh.data()), hh.size() / 2, &L.Wh);
-    put(reinterpret_cast<const float*>(hl.data()), hl.size() / 2, &L.Wl);
-    L.winv = std::ldexp(1.0f, -e);
+    WeightSplit s;
+    split_weights(w, n, &s);
+    put(s.hi.data(), n, &L.Whi); put(s.lo.data(), n, &L.Wlo);
+    put(reinterpret_cast<const float*>(s.h.data()), s.h.size() / 2, &L.Wh);
+    put(reinterpret_cast<const float*>(s.l.data()), s.l.size() / 2, &L.Wl);
+    L.winv = s.winv;
   }
   // conv/linear `wname`.weight [N,K(,1,1)], optional .bias; optional BatchNorm `bnname`
   void layer(Layer& L, const std::string& wname, const std::string& bnname, int N, int K, bool bias) {
@@ -169,15 +150,10 @@ struct Builder {
     put(np.data(), np.size(), &nr.np);
     if (eif) put(ep.data(), ep.size(), &nr.ep);
     if (tab_T > 0 && !eif) {
-      LifTableHost t;
-      lif_table_build(np.data(), C, tab_T, &t);
-      // re-pack with one fixed stride per block so a kernel finds its block from (base, stride, block index) alone
-      const uint32_t stride = (t.max_block_bytes + 255u) / 256u * 256u;
-      std::vector<float> img((size_t)stride / 4 * t.blocks.size(), 0.0f);
-      for (size_t b = 0; b < t.blocks.size(); ++b)
-        memcpy(reinterpret_cast<uint8_t*>(img.data()) + b * stride, t.image.data() + t.blocks[b].off_bytes, t.blocks[b].bytes);
-      put(img.data(), img.size(), &nr.tab);
-      nr.tab_stride = stride; nr.tab_T = tab_T; nr.tab_ok = t.usable; nr.tab_err = (float)t.max_err;
+      LifTablePacked t;
+      lif_table_pack(np.data(), C, tab_T, &t);
+      put(t.img.data(), t.img.size(), &nr.tab);
+      nr.tab_stride = t.stride; nr.tab_T = tab_T; nr.tab_ok = t.usable; nr.tab_err = t.max_err;
     }
   }
   void raw(const std::string& name, size_t n, const float** dst) {
@@ -283,6 +259,44 @@ void build_fd(Builder& B) {
 }
 
 }  // namespace
+
+namespace sapcu {
+
+void split_weights(const float* w, size_t n, WeightSplit* s) {
+  s->hi.resize(n); s->lo.resize(n);
+  for (size_t i = 0; i < n; ++i) {
+    uint32_t b; memcpy(&b, &w[i], 4);
+    if ((b & 0x7F800000u) != 0x7F800000u) b = (b + 0x1000u) & 0xFFFFE000u;
+    float h; memcpy(&h, &b, 4);
+    s->hi[i] = h; s->lo[i] = w[i] - h;                                    // lo exact in fp32
+  }
+  // fp16 (hi, lo) of w * 2^e with max |w| * 2^e in [2^13, 2^14): both halves stay in fp16's normal range for every
+  // weight within 2^-9 of the largest one, smaller ones keep 6e-8 absolute (scaled) precision
+  float mx = 0.0f;
+  for (size_t i = 0; i < n; ++i) if (std::isfinite(w[i])) mx = std::max(mx, std::fabs(w[i]));
+  int e = 0;
+  if (mx > 0.0f) { int ex; std::frexp(mx, &ex); e = 14 - ex; }          // mx = f * 2^ex, f in [0.5, 1)
+  const float sc = std::ldexp(1.0f, e);
+  s->h.assign((n + 1) & ~(size_t)1, 0); s->l.assign((n + 1) & ~(size_t)1, 0);
+  for (size_t i = 0; i < n; ++i) {
+    const float ws = w[i] * sc;                                           // exact (power of two)
+    const uint16_t h = f32_to_f16_rn(ws);
+    s->h[i] = h; s->l[i] = f32_to_f16_rn(ws - f16_to_f32(h));
+  }
+  s->winv = std::ldexp(1.0f, -e);
+}
+
+void lif_table_pack(const float* np4, int C, int T, LifTablePacked* out) {
+  LifTableHost t;
+  lif_table_build(np4, C, T, &t);
+  const uint32_t stride = (t.max_block_bytes + 255u) / 256u * 256u;
+  out->img.assign((size_t)stride / 4 * t.blocks.size(), 0.0f);
+  for (size_t b = 0; b < t.blocks.size(); ++b)
+    memcpy(reinterpret_cast<uint8_t*>(out->img.data()) + b * stride, t.image.data() + t.blocks[b].off_bytes, t.blocks[b].bytes);
+  out->stride = stride; out->usable = t.usable; out->max_err = (float)t.max_err;
+}
+
+}  // namespace sapcu
 
 extern "C" {
 

@@ -23,6 +23,16 @@ struct Neuron {    // clamped per-channel parameters: np = [4][C] (d, a, r, th0)
   const float* tab = nullptr; uint32_t tab_stride = 0; int tab_T = 0; bool tab_ok = false; float tab_err = 0.0f;
 };
 
+// The tensor-core copies of one weight matrix w [n] (host fp32), as sapcu_model_finalize uploads them: tf32 (hi, lo) with
+// hi = w rounded to 10 mantissa bits (round-to-nearest, ties away) and lo = w - hi, and fp16 (hi, lo) of w * 2^e with
+// max |w| * 2^e in [2^13, 2^14), winv = 2^-e.  h / l are padded to an even count (the float blob's granularity).
+struct WeightSplit { std::vector<float> hi, lo; std::vector<uint16_t> h, l; float winv = 1.0f; };
+void split_weights(const float* w, size_t n, WeightSplit* out);
+// The LIF^T table of np4 ([4][C] rows {d, a, r, th0}, clamped) for T steps, re-packed with one fixed stride per 128-channel
+// block so that a kernel finds its block from (base, stride, block index) alone
+struct LifTablePacked { std::vector<float> img; uint32_t stride = 0; bool usable = false; float max_err = 0.0f; };
+void lif_table_pack(const float* np4, int C, int T, LifTablePacked* out);
+
 struct FnBlock {
   int D = 0, k = 0;
   Layer fc1, qkv, fc_delta, fc_delta2, fc_gamma, fc_gamma2, out_proj, fc2;

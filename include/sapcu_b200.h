@@ -297,6 +297,44 @@ int sapcu_intra_knn(const float* d_feat, int64_t ld, int64_t S, int M, int C, in
 int sapcu_gemm(const float* d_x, int64_t R, int K, const float* d_w, int N, const float* d_bias,
                float* d_y, int mode, void* stream);
 
+/* Test hook: ONE contraction of the forwards, Y = epilogue(A * W^T), run through the forwards' own dispatcher (engine choice
+ * tc2 -> tc -> SIMT, the fast-mode switches) so that a test can reach every GEMM flavour on its own.  h_* fields are HOST
+ * arrays: the weights are split and the LIF table is built by the same code as sapcu_model_finalize, then copied into d_ws
+ * (sapcu_gemm_case_workspace_bytes(a) bytes, 256-byte aligned); d_* fields are device arrays the caller owns.  Allocates
+ * nothing, synchronises nothing; the watchdog surfaces through sapcu_device_status.
+ *   amode: 0 plain A[r, c] = x[r * lda + c]; 1 EdgeConv cat(F[nb] - F[pt], F[nb]) (d_f, ldf, C; K = 2C); 2 attention input
+ *          Q[pt] - Kf[nb] + x[r] (d_q, d_kf, ldq); edge rows r = pt * kk + j, nb = pt - pt % mpts + d_idx[pt * ldi + j].
+ *   act: 0 none, 1 LeakyReLU(0.2), 2 exact GELU, 3 the LIF^T chain of T steps with h_params4 = [4][N] {d, a, r, th0}
+ *          (clamped); use_table: evaluate that chain from the layer's table (built for T) where the engine takes one.
+ *   x_format: 0 fp32 [R, lda]; 1 fp16 (hi, lo) planes of x * 2^13 ([R, K] halfs each, lda == K); 2 one such plane.
+ *   x_unit: the inputs are LIF outputs in [0, 0.7) (enables the fp16 operand paths).  fast: the single-product formats of
+ *          SAPCU_MODE_FAST (one fp16 plane in / out, compact single-pass TF32 stages), as that mode's producers set it.
+ *   out_h2: LIF output as planes in x_format's convention (ldc == N), d_y2 (nullable) = fp32 copy [R, N].
+ *   edge_bias: add Q[pt, c] - Kf[nb, c] before the epilogue (d_q, d_kf, ldq, d_idx, ldi, kk, mpts).
+ *   d_pool: pool[(patch * pool_T + t), c] = max over the patch's pool_M points of the LeakyReLU output, rows = (point * pool_T + t);
+ *          the buffer must be pre-filled with -inf.
+ *   d_at_pos: fused attention tail, Y[pt, c] = sum_j softmax_j(y[pt * kk + j, c] / at_sqrt) (at_v[nb_j * at_ldv + c] +
+ *          pos[e_j, c]), e_j = d_at_pid ? d_at_pid[pt * kk + j] : pt * kk + j, pos as planes when pos_h2.
+ *   d_R_dev (nullable): rows actually present, in device memory (R is the capacity): the row tiles that hold a row < *d_R_dev
+ *          are computed in full from the capacity rows (rows *d_R_dev .. the end of that tile hold the result of whatever the
+ *          inputs hold there), later tiles are not written; tc2_any_rows: the 2-CTA engine from
+ *          1024 rows on; group: 0 or 32 (max over 32 consecutive rows, SIMT engine). */
+typedef struct sapcu_gemm_case_args {
+  int amode, act, T, use_table;
+  int64_t R; int K, N; int64_t lda, ldc, ldr;
+  const float* h_w; const float* h_bias; const float* h_scale; const float* h_shift; const float* h_params4;
+  const float* d_x; int x_format, x_unit, fast;
+  float* d_y; int out_h2; float* d_y2;
+  const float* d_residual;
+  const float* d_f; int64_t ldf; int C;
+  int edge_bias; const float* d_q; const float* d_kf; int64_t ldq; const int32_t* d_idx; int ldi, kk, mpts;
+  float* d_pool; int pool_T, pool_M;
+  const float* d_at_pos; const float* d_at_v; int64_t at_ldv; float at_sqrt; const int32_t* d_at_pid; int pos_h2;
+  const int* d_R_dev; int tc2_any_rows, group;
+} sapcu_gemm_case_args;
+size_t sapcu_gemm_case_workspace_bytes(const sapcu_gemm_case_args* a);
+int sapcu_gemm_case(const sapcu_gemm_case_args* a, void* d_ws, size_t ws_bytes, int mode, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -209,9 +209,38 @@ def _agree(a, b):
     return float(((a > HARD) == (b > HARD)).mean())
 
 
+# Per-tap max-abs bounds of the model-level parity tests: 10x the deviation measured on a B200 at a 1,000 W limit, rounded up to
+# one significant digit (profiles/r02_parity.json where it holds the tap, else profiles/r03_parity.json), and never above the
+# blanket bound these tests used before (2e-3; 5e-3 for fcat; 3e-3 in the fast mode).  A bound far above what the kernels
+# reach would hide a wrong plane, table or product.
+FN_TAP_BOUND = {
+    ('default', 'fp32'): {'fcat': 5e-06, 'gmax': 3e-07, 'snn_final': 5e-07, 'snn_init': 4e-07, 'trans3.snn1': 5e-07, 'trans3.snn_delta2': 4e-07, 'trans3.snn_gamma': 4e-07, 'trans3.snn_qkv': 4e-07},
+    ('default', 'tc'): {'fcat': 7e-05, 'gmax': 9e-07, 'snn_final': 2e-06, 'snn_init': 5e-07, 'trans3.snn1': 7e-05, 'trans3.snn_delta2': 6e-05, 'trans3.snn_gamma': 7e-05, 'trans3.snn_qkv': 7e-05},
+    ('stress', 'fp32'): {'fcat': 6e-05, 'gmax': 4e-06, 'snn_final': 6e-06, 'snn_init': 5e-07, 'trans3.snn1': 8e-06, 'trans3.snn_delta2': 6e-07, 'trans3.snn_gamma': 9e-07, 'trans3.snn_qkv': 2e-06},
+    ('stress', 'tc'): {'fcat': 0.003, 'gmax': 0.0003, 'snn_final': 0.0003, 'snn_init': 7e-07, 'trans3.snn1': 0.0004, 'trans3.snn_delta2': 0.0004, 'trans3.snn_gamma': 0.0004, 'trans3.snn_qkv': 0.0004},
+}
+FD_TAP_BOUND = {
+    ('default', 'fp32'): {'pool': 9e-06, 'spikes': 9e-06},
+    ('default', 'tc'): {'pool': 4e-05, 'spikes': 1e-05},
+    ('stress', 'fp32'): {'pool': 8e-05, 'spikes': 0.0009},
+    ('stress', 'tc'): {'pool': 0.0007, 'spikes': 0.002},
+}
+BLOCK_TAP_BOUND = {
+    'fp32': {'trans1.snn1': 5e-07, 'trans1.snn_delta2': 5e-07, 'trans1.snn_gamma': 7e-07, 'trans1.snn_qkv': 6e-07, 'trans2.snn1': 3e-06, 'trans2.snn_delta2': 8e-07, 'trans2.snn_gamma': 2e-06, 'trans2.snn_qkv': 6e-07},
+    'tc': {'trans1.snn1': 2e-06, 'trans1.snn_delta2': 0.0004, 'trans1.snn_gamma': 0.0004, 'trans1.snn_qkv': 2e-06, 'trans2.snn1': 0.0001, 'trans2.snn_delta2': 0.0004, 'trans2.snn_gamma': 0.0004, 'trans2.snn_qkv': 0.0004},
+    'fast': {'trans1.snn1': 0.0006, 'trans1.snn_delta2': 0.001, 'trans1.snn_gamma': 0.0009, 'trans1.snn_qkv': 0.0005, 'trans2.snn1': 0.003, 'trans2.snn_delta2': 0.001, 'trans2.snn_gamma': 0.0009, 'trans2.snn_qkv': 0.0005},
+}
+FAST_TAP_BOUND = {
+    ('lif_tables', 'default'): {'trans3.snn_delta2': 0.0007, 'trans3.snn_gamma': 0.0007},
+    ('lif_tables', 'stress'): {'trans3.snn_delta2': 0.001, 'trans3.snn_gamma': 0.001},
+    ('reduced_mufu', 'default'): {'trans3.snn_delta2': 0.0007, 'trans3.snn_gamma': 0.0007},
+    ('reduced_mufu', 'stress'): {'trans3.snn_delta2': 0.0009, 'trans3.snn_gamma': 0.0008},
+}
+
+
 @pytest.mark.parametrize("mode", ["fp32", "tc"])
 @pytest.mark.parametrize("stress", [False, True], ids=["default_init", "stress_init"])
-def test_fn_forward_parity(lib, sphere, golden, stress, mode):
+def test_fn_forward_parity(lib, sphere, golden, parity_log, stress, mode):
     cloud, seeds = sphere
     tag = "stress" if stress else "default"
     mfn, _, sd_fn, _ = _models(stress)
@@ -244,18 +273,22 @@ def test_fn_forward_parity(lib, sphere, golden, stress, mode):
               ("trans3.snn_qkv", np.concatenate([cf(k3["q"]), cf(k3["k"]), cf(k3["v"])], 1)),
               ("trans3.snn_delta2", cf(k3["pos"])), ("trans3.snn_gamma", cf(k3["a1"])),
               ("snn_final", cf(taps["snn_final"]))]
+    rec = {}
     for name, r in checks:
         t = tap(name)
         assert t.shape == r.shape, name
-        assert np.abs(t - r).max() < 2e-3, (name, np.abs(t - r).max())
+        rec[name] = float(np.abs(t - r).max())
         assert _agree(t, r) >= 0.999, (name, _agree(t, r))
-    np.testing.assert_allclose(tap("fcat"), taps["fcat"].numpy().reshape(P, 192), rtol=0, atol=5e-3)
-    np.testing.assert_allclose(tap("gmax"), taps["gmax"].numpy(), rtol=0, atol=2e-3)
+    rec["fcat"] = float(np.abs(tap("fcat") - taps["fcat"].numpy().reshape(P, 192)).max())
+    rec["gmax"] = float(np.abs(tap("gmax") - taps["gmax"].numpy()).max())
+    parity_log.record("fn_forward_parity[%s,%s]" % (tag, mode), **rec)
+    for name, e in rec.items():
+        assert e < FN_TAP_BOUND[tag, mode][name], (name, e)
 
 
 @pytest.mark.parametrize("mode", ["fp32", "tc"])
 @pytest.mark.parametrize("stress", [False, True], ids=["default_init", "stress_init"])
-def test_fd_forward_parity(lib, sphere, golden, stress, mode):
+def test_fd_forward_parity(lib, sphere, golden, parity_log, stress, mode):
     tag = "stress" if stress else "default"
     _, mfd, _, sd_fd = _models(stress)
     mfd.set_mode(mode)
@@ -276,9 +309,11 @@ def test_fd_forward_parity(lib, sphere, golden, stress, mode):
     got_tf = mfd(p.to(DEV), forced_idx=forced).cpu().numpy()
     spk = mfd.tap("spikes", B, 100).cpu().numpy().reshape(B, 100, 7, 960)
     ref_spk = taps["spikes"].permute(1, 3, 0, 2).numpy()                                # [T,B,960,M] -> [B,M,T,960]
-    assert np.abs(spk - ref_spk).max() < 2e-3
+    rec = {"spikes": float(np.abs(spk - ref_spk).max()),
+           "pool": float(np.abs(mfd.tap("pool", B, 100).cpu().numpy().reshape(B, 7, 768) - taps["pool"].permute(1, 0, 2).numpy()).max())}
+    parity_log.record("fd_forward_parity[%s,%s]" % (tag, mode), **rec)
+    assert rec["spikes"] < FD_TAP_BOUND[tag, mode]["spikes"] and rec["pool"] < FD_TAP_BOUND[tag, mode]["pool"], rec
     assert _agree(spk, ref_spk) >= 0.999
-    np.testing.assert_allclose(mfd.tap("pool", B, 100).cpu().numpy().reshape(B, 7, 768), taps["pool"].permute(1, 0, 2).numpy(), rtol=0, atol=2e-3)
     rel_tf = np.abs(got_tf - ref) / np.maximum(np.abs(ref), 1e-6)
     assert rel_tf.max() < 1e-3, rel_tf
     assert np.abs(got_tf[:3] - g[tag + "_dist"]).max() / np.abs(g[tag + "_dist"]).max() < 1e-3
@@ -762,7 +797,8 @@ def test_fast_mode_deviation(lib, sphere, golden, parity_log, tables, tmp_path):
         v = out[tag]
         assert v["normal_angle_deg_max"] < 0.5, v
         assert v["dist_rel_teacher_forced_max"] < 2e-2, v
-        assert v["tap_max_abs"]["trans3.snn_delta2"] < 3e-3 and v["tap_max_abs"]["trans3.snn_gamma"] < 3e-3, v
+        bound = FAST_TAP_BOUND["lif_tables" if tables else "reduced_mufu", tag]
+        assert all(v["tap_max_abs"][k] < b for k, b in bound.items()), (v["tap_max_abs"], bound)
         assert v["spike_agreement_min"] >= 0.99, v
 
 
@@ -923,7 +959,7 @@ def test_fn_block_taps_trans1_trans2(lib, sphere, parity_log, mode):
     taps = {}
     with torch.no_grad():
         orc.fn_forward(sd_fn, p, taps=taps)
-    tol, agr = (2e-3, 0.999) if mode != "fast" else (3e-3, 0.995)
+    agr = 0.999 if mode != "fast" else 0.995
     rec = {}
     for b in (1, 2):
         mfn(p.to(DEV), _stop_after_block=b)
@@ -935,7 +971,7 @@ def test_fn_block_taps_trans1_trans2(lib, sphere, parity_log, mode):
             assert t.shape == r.shape, (b, name, t.shape, r.shape)
             err, ag = float(np.abs(t - r).max()), _agree(t, r)
             rec["trans%d.%s" % (b, name)] = dict(max_abs=err, spike_agreement=ag)
-            assert err < tol and ag >= agr, (mode, b, name, err, ag)
+            assert err < BLOCK_TAP_BOUND[mode]["trans%d.%s" % (b, name)] and ag >= agr, (mode, b, name, err, ag)
     parity_log.record("fn_block_taps[%s]" % mode, **rec)
 
 
