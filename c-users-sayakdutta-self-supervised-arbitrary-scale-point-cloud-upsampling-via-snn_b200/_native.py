@@ -13,10 +13,10 @@ _CSRC = os.path.join(_HERE, "csrc")
 _SO = os.path.join(_HERE, "libsapcu_b200.so")
 _SOURCES = ["api.cu", "model.cu", "forward.cu", "gemm.cu", "gemm_tc.cu", "gemm_tc2.cu", "knn_seed.cu", "patch_ops.cu",
             "intra_knn.cu", "fn_kernels.cu", "fd_kernels.cu", "seedgen.cu", "post_ops.cu", "lif_table.cu", "orient.cu",
-            "mesh_dist.cu", "edge_pairs.cu"]
+            "mesh_dist.cu", "edge_pairs.cu", "emd.cu"]
 # per-file flags: the fp64 geometry of seedgen.cu must round like the g++ build of dense.cpp (no FMA contraction), and that
-# of mesh_dist.cu like its numpy restatement
-_FILE_FLAGS = {"seedgen.cu": ["-fmad=false"], "mesh_dist.cu": ["-fmad=false"]}
+# of mesh_dist.cu and emd.cu like their numpy restatements
+_FILE_FLAGS = {"seedgen.cu": ["-fmad=false"], "mesh_dist.cu": ["-fmad=false"], "emd.cu": ["-fmad=false"]}
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
 
@@ -145,6 +145,9 @@ _SIGS = {
     "sapcu_mesh_distance": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p,
                                            ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t,
                                            ctypes.c_void_p]),
+    "sapcu_emd_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int64]),
+    "sapcu_emd": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_double, ctypes.c_void_p,
+                                 ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]),
     "sapcu_model_create": (ctypes.c_void_p, [ctypes.c_int, ctypes.c_void_p, ctypes.c_int]),
     "sapcu_model_set_tensor": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_void_p, ctypes.c_int64]),
     "sapcu_model_finalize": (ctypes.c_int, [ctypes.c_void_p]),

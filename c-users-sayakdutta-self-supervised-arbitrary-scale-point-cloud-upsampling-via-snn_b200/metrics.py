@@ -1,21 +1,25 @@
-"""Quality metrics of upsampled clouds on the GPU: Chamfer (CD), Hausdorff (HD), point-to-mesh (P2F) distances and the
-normal error against the closest mesh face.
+"""Quality metrics of upsampled clouds on the GPU: Chamfer (CD), Hausdorff (HD), Earth Mover's (EMD) and point-to-mesh
+(P2F) distances and the normal error against the closest mesh face.
 
     read_off(path)                              -> vertices [V,3] f64, faces [F,3] int32 (plain-text OFF, triangles only)
     nn_distances(a, b)                          -> [len(a)] f64, distance from each row of a to its nearest row of b
     chamfer_hausdorff(pred, gt)                 -> {"cd", "cd_sq", "hd"}
+    emd_match(a, b, rel_tol)                    -> certified optimal matching of two equal-size clouds and its bounds
+    emd(a, b, rel_tol)                          -> mean distance of that matching (raises when not certified)
     point_to_mesh(points, vertices, faces)      -> [S] f64 exact distance to the mesh (and the closest face)
     normal_errors(points, normals, vertices, faces)
-    evaluate(pred, gt, vertices, faces, normals, normalize)
+    evaluate(pred, gt, vertices, faces, normals, normalize, emd)
 
 The nearest neighbours come from sapcu_knn with K = 1 (exact fp64), the point-to-mesh distances from sapcu_mesh_distance (an
-LBVH built and queried on the device, bitwise the brute-force minimum; include/sapcu_b200.h).  Point arrays may be numpy
+LBVH built and queried on the device, bitwise the brute-force minimum; include/sapcu_b200.h), the EMD from sapcu_emd (an
+auction solver on the device that certifies its result with a lower bound).  Point arrays may be numpy
 arrays or CUDA tensors; numpy inputs go to the current CUDA device.  Results are host (numpy / float) values.
 
-    python -m sapcu_b200.metrics PRED_DIR GT_DIR [--mesh-dir DIR] [--json OUT]
+    python -m sapcu_b200.metrics PRED_DIR GT_DIR [--mesh-dir DIR] [--emd] [--json OUT]
 
 pairs PRED_DIR/<stem>.xyz with GT_DIR/<stem>.xyz (and MESH_DIR/<stem>.off), prints one line per file and the means.  A
-prediction with six columns (generate.process_file(..., with_normals=True)) is graded on its normals too.
+prediction with six columns (generate.process_file(..., with_normals=True)) is graded on its normals too.  --emd adds the
+EMD of files whose prediction and ground truth have the same number of points; for the others one line says it was skipped.
 """
 import argparse
 import json
@@ -122,6 +126,77 @@ def cd_hd_from_dist2(pg2, gp2):
             "hd": float(torch.maximum(pg.max(), gp.max()))}
 
 
+# ----------------------------------------------------------------------------------------------------------------- EMD
+def _rows(x, name):
+    """Row count of an [n,3] point array, checked on the host (numpy: also finite) before anything touches a device."""
+    if isinstance(x, torch.Tensor):
+        shape = tuple(x.shape)
+    else:
+        arr = np.asarray(x, dtype=np.float64)
+        shape = arr.shape
+        if arr.ndim == 2 and arr.shape[1] == 3 and not np.isfinite(arr).all():
+            raise ValueError("%s: non-finite coordinates" % name)
+    if len(shape) != 2 or shape[1] != 3:
+        raise ValueError("%s: [n,3] coordinates expected, got shape %s" % (name, shape))
+    return shape[0]
+
+
+def emd_match(a, b, rel_tol=1e-6):
+    """Earth Mover's Distance between two clouds of the same size n, with its certificate:
+
+        EMD(a, b) = min over permutations s of (1/n) sum_i |a_i - b_s(i)|
+
+    the mean over points of the UNSQUARED Euclidean distances of an optimal one-to-one matching.  sapcu_emd solves it on the
+    device (forward auction with eps-scaling, include/sapcu_b200.h); its prices give a lower bound, so the optimum lies in
+    [emd_lower, emd] and, when converged, emd - emd_lower <= rel_tol * emd + eps_min with eps_min = max|a_i - b_j| * 2^-40.
+    Returns {"emd": primal / n, "emd_lower": dual / n, "assignment": [n] int32 (row of b matched to row i of a),
+    "cost": [n] float64 (that pair's distance), "phases", "rounds", "converged"} with host values.  Unequal sizes, shapes
+    other than [n,3], non-finite values, n = 0, n > 131,072 and clouds whose bounding box has a diagonal beyond about
+    1.3e154 (its square overflows fp64, as the costs of its farthest pairs would) raise ValueError; partial transport is not
+    offered.  Clouds with many coincident points are slow: see sapcu_emd in include/sapcu_b200.h.
+    Whether external/Meta-PU_evaluation uses this convention (mean, unsquared) has not been checked against it here: that
+    needs a SAPCU_REFERENCE checkout."""
+    na, nb = _rows(a, "a"), _rows(b, "b")
+    if na != nb:
+        raise ValueError("emd: the clouds differ in size (%d and %d points); EMD needs equal sizes" % (na, nb))
+    if not 1 <= na <= 131072:
+        raise ValueError("emd: n=%d outside 1 <= n <= 131,072" % na)
+    if not rel_tol >= 0:
+        raise ValueError("emd: rel_tol must be >= 0")
+    d_a = _device_f64(a, "a")
+    d_b = _device_f64(b, "b", d_a.device)
+    both = torch.cat([d_a, d_b])
+    ext = both.max(0).values - both.min(0).values
+    if not bool(torch.isfinite((ext[0] * ext[0] + ext[1] * ext[1]) + ext[2] * ext[2])):
+        raise ValueError("emd: the clouds span more than about 1.3e154; their squared distances overflow fp64")
+    L = N.lib()
+    n, dev = na, d_a.device
+    with torch.cuda.device(dev):
+        assign = torch.empty(n, dtype=torch.int32, device=dev)
+        cost = torch.empty(n, dtype=torch.float64, device=dev)
+        stats = torch.empty(6, dtype=torch.float64, device=dev)
+        ws = torch.empty(L.sapcu_emd_workspace_bytes(n), dtype=torch.uint8, device=dev)
+        N.check(L.sapcu_emd(N.ptr(d_a), N.ptr(d_b), n, float(rel_tol), N.ptr(assign), N.ptr(cost), N.ptr(stats), N.ptr(ws),
+                            ws.numel(), N.stream_ptr(dev)), "sapcu_emd")
+        st = stats.cpu().numpy()
+    return {"emd": float(st[0]) / n, "emd_lower": float(st[1]) / n, "assignment": assign.cpu().numpy(),
+            "cost": cost.cpu().numpy(), "phases": int(st[3]), "rounds": int(st[4]), "converged": bool(st[5] == 1.0)}
+
+
+def _certified_emd(a, b, rel_tol):
+    r = emd_match(a, b, rel_tol)
+    if not r["converged"]:
+        raise N.SapcuError("emd: the certificate did not close: emd %.17g, lower bound %.17g (gap %.3g) after %d rounds"
+                           % (r["emd"], r["emd_lower"], r["emd"] - r["emd_lower"], r["rounds"]))
+    return r["emd"]
+
+
+def emd(a, b, rel_tol=1e-6):
+    """emd_match(a, b, rel_tol)["emd"]: the mean unsquared distance of the matching, within rel_tol of the optimum (plus the
+    2^-40 floor of emd_match).  Raises SapcuError with the gap when the solver stopped before its certificate closed."""
+    return _certified_emd(a, b, rel_tol)
+
+
 # ----------------------------------------------------------------------------------------------------------------- P2F
 def _mesh_arrays(vertices, faces, device):
     d_v = _device_f64(vertices, "vertices", device)
@@ -208,11 +283,12 @@ def unit_ball(gt):
     return c, (r if r > 0 else 1.0)
 
 
-def evaluate(pred, gt, vertices=None, faces=None, normals=None, normalize=True):
+def evaluate(pred, gt, vertices=None, faces=None, normals=None, normalize=True, emd=False):
     """CD / HD between pred and gt and, given a mesh, P2F (mean and std of the point-to-mesh distances of pred) and, given
-    normals of pred, normal_errors.  normalize: pred, gt and the mesh are first mapped by x -> (x - c) / r with c the gt
-    cloud's centroid and r its largest distance from c (the gt then lies in the unit ball), so numbers of differently
-    scaled shapes are comparable; normals are unchanged by that map."""
+    normals of pred, normal_errors.  emd: also the EMD (emd(), mean unsquared distance of the optimal matching; pred and gt
+    must have the same size) on the same coordinates as CD.  normalize: pred, gt and the mesh are first mapped by
+    x -> (x - c) / r with c the gt cloud's centroid and r its largest distance from c (the gt then lies in the unit ball), so
+    numbers of differently scaled shapes are comparable; normals are unchanged by that map."""
     pred, gt = _host(pred)[:, :3], _host(gt)[:, :3]
     if vertices is not None:
         vertices = _host(vertices)
@@ -221,7 +297,11 @@ def evaluate(pred, gt, vertices=None, faces=None, normals=None, normalize=True):
         pred, gt = (pred - c) / r, (gt - c) / r
         if vertices is not None:
             vertices = (vertices - c) / r
+    if emd and len(pred) != len(gt):
+        raise ValueError("evaluate: emd needs pred and gt of the same size (%d and %d points)" % (len(pred), len(gt)))
     out = chamfer_hausdorff(pred, gt)
+    if emd:
+        out["emd"] = _certified_emd(pred, gt, 1e-6)
     if vertices is not None and faces is not None:
         p2f = point_to_mesh(pred, vertices, faces)
         out["p2f_mean"], out["p2f_std"] = float(p2f.mean()), float(p2f.std())
@@ -236,6 +316,7 @@ def main(argv=None):
     ap.add_argument("pred_dir")
     ap.add_argument("gt_dir")
     ap.add_argument("--mesh-dir", default=None, help="<stem>.off meshes for P2F (and normals, when pred has six columns)")
+    ap.add_argument("--emd", action="store_true", help="add the Earth Mover's Distance (files with equal point counts)")
     ap.add_argument("--json", default=None, help="write the per-file results and the means here")
     a = ap.parse_args(argv)
     if not torch.cuda.is_available():
@@ -254,7 +335,12 @@ def main(argv=None):
             off = os.path.join(a.mesh_dir, stem + ".off")
             if os.path.exists(off):
                 mesh = read_off(off)
-        r = evaluate(pred[:, :3], gt, *(mesh or (None, None)), normals=pred[:, 3:6] if pred.shape[1] >= 6 else None)
+        with_emd = a.emd and len(pred) == len(gt)
+        if a.emd and not with_emd:
+            print("%s: EMD skipped: the prediction has %d points and the ground truth %d (EMD needs equal sizes)"
+                  % (stem, len(pred), len(gt)))
+        r = evaluate(pred[:, :3], gt, *(mesh or (None, None)), normals=pred[:, 3:6] if pred.shape[1] >= 6 else None,
+                     emd=with_emd)
         rows[stem] = r
         print(stem + "  " + "  ".join("%s %.6g" % kv for kv in r.items()))
     keys = sorted({k for r in rows.values() for k in r})

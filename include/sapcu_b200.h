@@ -197,6 +197,42 @@ int sapcu_mesh_distance(const double* d_vertices, int64_t V, const int32_t* d_fa
                         void* d_ws, size_t ws_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------
+ * Earth Mover's Distance (no reference counterpart; the EMD metric of the upsampling literature, computed there on the host
+ * with an O(n^3) assignment solver or by an approximate matching kernel): the min-cost perfect matching between two clouds
+ * of n points each, EMD = primal / n (csrc/emd.cu).
+ *   cost      c_ij = sqrt(((dx*dx)+(dy*dy))+(dz*dz)) in fp64 without contraction, d = a_i - b_j (a numpy restatement gives
+ *             the same bits); recomputed from the coordinates, no n x n matrix is stored.
+ *   method    forward auction with eps-scaling (Bertsekas), one cooperative persistent kernel, no host round trip.  Per
+ *             phase at one eps, Jacobi rounds until every row of a owns a row of b: each unassigned row i finds the lowest
+ *             v = c_ij + p_j (lowest j on ties) and the second lowest value and bids p_j1 + (v2 - v1) + eps (p + eps when
+ *             n = 1); an object goes to its highest bid, ties to the lowest row i.  eps starts at c_max / 4 and is divided by
+ *             5 per phase, not below eps_min = c_max * 2^-40 (2^-40 when c_max = 0); the prices carry over.
+ *   bounds    after a phase, primal = sum_i c_i,assign(i) and dual = sum_i min_j (c_ij + p_j) - sum_j p_j, a lower bound of
+ *             the optimum for any prices.  The solve stops when primal - dual <= rel_tol * primal + n * eps_min
+ *             (converged = 1); a phase at eps_min that misses it is returned with converged = 0.
+ *   outputs   d_assign[i] (int32 [n]) the row of b matched to row i of a, a permutation of [0, n); d_cost[i] (f64 [n]) its
+ *             c; d_stats (f64 [6]) = {primal, dual, eps of the returned phase, phases, rounds (through that phase),
+ *             converged}.  Sums run in a fixed order, so repeat calls, other streams and other grids give the same bits.
+ *   bounded   at most max(2^20, 256 n) bidding rounds in all; SAPCU_EMD_MAX_ROUNDS (> 0; read once per process, tests
+ *             only) replaces that cap.  At the cap the last COMPLETED phase is returned with converged = 0; when none
+ *             completed, d_assign is all -1, d_cost +inf and d_stats = {+inf, 0, 0, 0, 0, 0}.
+ *   limits    1 <= n <= 131,072, rel_tol >= 0, non-null pointers, else SAPCU_EINVAL; a short workspace: SAPCU_EWORKSPACE.
+ *   overflow  when some ((dx*dx)+(dy*dy))+(dz*dz) is not finite (points about 1.3e154 apart), or a bid is not finite, the
+ *             call returns the "no phase completed" outputs above (or the last completed phase) with converged = 0; no
+ *             input makes a kernel read or write outside its arrays.
+ *   work      about 50 n scans of n points on spread-out clouds (DESIGN.md section 9).  Many COINCIDENT points are the slow
+ *             case: equal values go to the lowest index, so the bidders of one position all bid for the same object and
+ *             one wins per round -- n copies of one point take n rounds and about n^3 / 2 cost evaluations.  The round cap
+ *             bounds the rounds, not that work.
+ * d_a, d_b: [n,3] f64.  Allocates nothing and does not synchronise the stream.  The workspace size is a closed form of n
+ * (76 bytes per point plus about 330 KB), computed without a device.
+ * ---------------------------------------------------------------------------------- */
+size_t sapcu_emd_workspace_bytes(int64_t n);   /* 0 outside the limits above */
+int    sapcu_emd(const double* d_a, const double* d_b, int64_t n, double rel_tol,
+                 int32_t* d_assign, double* d_cost, double* d_stats,
+                 void* d_ws, size_t ws_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------
  * Models.  A handle is built from the same hyper-parameters get_model() consumes
  * (fn/config.py:183-210, fd/config.py:89-117) and the tensors of the module's
  * state_dict (host fp32 pointers, names = state_dict keys, SURVEY.md section 8b).

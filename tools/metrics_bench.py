@@ -2,7 +2,8 @@
 """Time the evaluation metrics on the GPU: the exact point-to-mesh distance (sapcu_mesh_distance, LBVH built and queried on
 the device) and Chamfer / Hausdorff (sapcu_knn with K = 1, both directions), next to the numpy brute force on the host.
 
-    python tools/metrics_bench.py [--levels 5 7 9] [--queries 8192 388467 2000000] [--reps 5] [--warmup 2] [--out FILE]
+    python tools/metrics_bench.py [--levels 5 7 9] [--queries 8192 388467 2000000] [--emd-n 2048 8192 32768]
+                                  [--sections mesh chamfer emd] [--reps 5] [--warmup 2] [--out FILE]
 
 Meshes: synthetic.sphere_mesh(level), 20 * 4**level faces (level 5: 20,480; 7: 327,680; 9: 5,242,880).  Queries: points
 uniformly within 0.01 of that sphere (radius 0.49 .. 0.51), seeded.  8,192 is one PU-style test shape, 388,467 the output
@@ -16,6 +17,12 @@ of configuration 1's pipeline, 2,000,000 a scan-sized cloud.  Per (mesh, queries
   host         the numpy brute force (the restatement of tests/test_metrics.py) on the first `host_points` query points,
                wall time on the host cores, and whether the GPU's distances and faces equal it bitwise on that subsample
 CD/HD cases: 8,192 x 8,192 and 388,467 x 8,192 points (pred x gt), both directions, CUDA events.
+EMD cases (--emd-n, default 2,048, 8,192 and 32,768 points): the sapcu_emd call (auction on the device, rel_tol 1e-6) between
+two seeded shells, CUDA events, median after warm-up; its phases, rounds and certified relative gap; and, up to 4,096
+points, scipy's linear_sum_assignment on the host (cdist + solve, wall time) and whether its optimum lies in [lower, emd].
+The slow case is timed too (--emd-coincident-n, default 2,048 and 8,192): both clouds n copies of one point, n rounds with
+one winner each, about n^3 / 2 cost evaluations.
+--sections selects which of mesh, chamfer and emd run.
 A 256 MiB buffer is overwritten before every timed run, so no run starts from an L2 (126 MB) left warm by the last one.
 The GPU's name, power limit and SM clock are read with nvidia-smi (read-only queries) in the same run.
 """
@@ -75,6 +82,9 @@ def main():
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=2)
     ap.add_argument("--host-points", type=int, default=256, help="host brute force subsample (points) per mesh, fewer on meshes above 2^18 faces")
+    ap.add_argument("--emd-n", type=int, nargs="+", default=[2048, 8192, 32768])
+    ap.add_argument("--emd-coincident-n", type=int, nargs="*", default=[2048, 8192])
+    ap.add_argument("--sections", nargs="+", default=["mesh", "chamfer", "emd"], choices=["mesh", "chamfer", "emd"])
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
     if not torch.cuda.is_available():
@@ -91,8 +101,8 @@ def main():
     st = torch.cuda.current_stream(dev)
     sp = N.stream_ptr(dev)
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
-    C = counters_library(N)
-    res = {"gpu": gpu_info(), "cases": [], "chamfer": []}
+    C = counters_library(N) if "mesh" in a.sections else None
+    res = {"gpu": gpu_info(), "cases": [], "chamfer": [], "emd": []}
 
     def timed(fn):
         for _ in range(a.warmup):
@@ -109,7 +119,7 @@ def main():
         N.check_device("metrics_bench")
         return sorted(ms)[len(ms) // 2]
 
-    for level in a.levels:
+    for level in (a.levels if "mesh" in a.sections else []):
         v, f = syn.sphere_mesh(level)
         V, F = len(v), len(f)
         d_v, d_f = torch.from_numpy(v).to(dev), torch.from_numpy(f).to(dev)
@@ -161,13 +171,47 @@ def main():
         del d_v, d_f, ws
         torch.cuda.empty_cache()
 
-    for sp_n, sg_n in ((8192, 8192), (388467, 8192)):
+    for sp_n, sg_n in (((8192, 8192), (388467, 8192)) if "chamfer" in a.sections else ()):
         pred = torch.from_numpy(shell(sp_n, 7)).to(dev)
         gt = torch.from_numpy(shell(sg_n, 8)).to(dev)
         ms = timed(lambda: (M._nn_dist2(pred, gt), M._nn_dist2(gt, pred)))
         r = {"pred": sp_n, "gt": sg_n, "both_directions_ms": ms}
         res["chamfer"].append(r)
         print(json.dumps(r), flush=True)
+
+    emd_cases = [("shells", n) for n in a.emd_n] + [("coincident", n) for n in a.emd_coincident_n]
+    for kind, n in (emd_cases if "emd" in a.sections else []):
+        if kind == "shells":
+            pa, pb = shell(n, 2 * n + 1), shell(n, 2 * n + 2)
+        else:
+            pa = pb = np.tile([[0.1, -0.2, 0.3]], (n, 1))
+        d_a, d_b = torch.from_numpy(pa).to(dev), torch.from_numpy(pb).to(dev)
+        assign = torch.empty(n, dtype=torch.int32, device=dev)
+        cost = torch.empty(n, dtype=torch.float64, device=dev)
+        stats = torch.empty(6, dtype=torch.float64, device=dev)
+        ws = torch.empty(L.sapcu_emd_workspace_bytes(n), dtype=torch.uint8, device=dev)
+
+        def solve():
+            N.check(L.sapcu_emd(N.ptr(d_a), N.ptr(d_b), n, 1e-6, N.ptr(assign), N.ptr(cost), N.ptr(stats), N.ptr(ws), ws.numel(),
+                                sp), "sapcu_emd")
+        ms = timed(solve)
+        st_ = stats.cpu().numpy()
+        r = {"cloud": kind, "n": n, "call_ms": ms, "phases": int(st_[3]), "rounds": int(st_[4]), "converged": bool(st_[5] == 1.0),
+             "emd": st_[0] / n, "emd_lower": st_[1] / n, "rel_gap": float((st_[0] - st_[1]) / st_[0]) if st_[0] > 0 else float(st_[0] - st_[1]),
+             "workspace_bytes": ws.numel()}
+        if kind == "shells" and n <= 4096:
+            from scipy.optimize import linear_sum_assignment
+            from scipy.spatial.distance import cdist
+            t0 = time.perf_counter()
+            row, col = linear_sum_assignment(cdist(pa, pb))
+            host_s = time.perf_counter() - t0
+            d = pa - pb[col]
+            opt = float(np.sqrt((d[:, 0] * d[:, 0] + d[:, 1] * d[:, 1]) + d[:, 2] * d[:, 2]).sum())
+            r["scipy"] = {"seconds": host_s, "emd": opt / n,
+                          "within_bounds": bool(st_[1] <= opt * (1 + 1e-12) and opt <= st_[0] * (1 + 1e-12))}
+        res["emd"].append(r)
+        print(json.dumps(r), flush=True)
+        del d_a, d_b, assign, cost, stats, ws
 
     res["gpu_end"] = gpu_info()
     line = json.dumps(res)
