@@ -145,6 +145,7 @@ int sapcu_knn(const double* d_cloud, int64_t N, const double* d_seeds, int64_t S
               void* d_ws, size_t ws_bytes, void* stream) {
   SAPCU_REQUIRE(N >= 1 && S >= 0, "sapcu_knn: bad sizes N=%lld S=%lld", (long long)N, (long long)S);
   SAPCU_REQUIRE(d_cloud && (S == 0 || (d_seeds && d_idx)) && d_ws, "sapcu_knn: null pointer");
+  SAPCU_REQUIRE(reinterpret_cast<uintptr_t>(d_ws) % 16 == 0, "sapcu_knn: workspace %p is not 16-byte aligned", d_ws);
   if (ws_bytes < sapcu_knn_workspace_bytes(N)) {
     set_error("sapcu_knn: workspace %zu < %zu bytes", ws_bytes, sapcu_knn_workspace_bytes(N));
     return SAPCU_EWORKSPACE;
@@ -165,6 +166,7 @@ int sapcu_knn_batched(const double* d_clouds, const int64_t* h_cloud_off, const 
   const int64_t N = h_cloud_off[B], S = h_seed_off[B];
   SAPCU_REQUIRE(N >= 1 && S >= 0, "sapcu_knn_batched: bad sizes N=%lld S=%lld", (long long)N, (long long)S);
   SAPCU_REQUIRE(d_clouds && (S == 0 || (d_seeds && d_idx)) && d_ws, "sapcu_knn_batched: null pointer");
+  SAPCU_REQUIRE(reinterpret_cast<uintptr_t>(d_ws) % 16 == 0, "sapcu_knn_batched: workspace %p is not 16-byte aligned", d_ws);
   if (ws_bytes < sapcu_knn_batched_workspace_bytes(N, B)) {
     set_error("sapcu_knn_batched: workspace %zu < %zu bytes", ws_bytes, sapcu_knn_batched_workspace_bytes(N, B));
     return SAPCU_EWORKSPACE;

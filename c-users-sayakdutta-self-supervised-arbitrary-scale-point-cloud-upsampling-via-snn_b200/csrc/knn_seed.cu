@@ -31,7 +31,9 @@ constexpr int KNN_THREADS = 256;     // seeds per CTA
 constexpr int KNN_TILE = 2048;       // cloud points per shared-memory tile (32 KiB)
 
 // fp32 SoA copy (x[npad], y[npad], z[npad]) of a [n,3] fp64 array and the running max |coordinate|; rows n .. npad-1 are
-// padding far outside any cloud (they can pass the filter only while a heap is not full; `consider` drops them by index)
+// padding far outside any cloud.  The thread-per-seed kernel copies whole 16-byte groups of rows, so a tile may also hold
+// rows outside the seed's cloud: the padding, and in batched launches up to 3 rows of the previous cloud before it and
+// rows of the next cloud after it.  They can pass the filter; `consider` drops them by index.
 constexpr float KNN_PAD = 3.0e18f;
 __host__ __device__ inline int64_t knn_npad(int64_t n) { return (n + 3) / 4 * 4 + 4; }
 __global__ void cloud_to_f32_kernel(const double* __restrict__ cloud, int64_t n, float* __restrict__ out, float* __restrict__ rmax) {
@@ -74,7 +76,9 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
 // Batched launches (sapcu_knn_batched): the grid is the concatenation of per-cloud block ranges.  blk_off / cloud_off /
 // seed_off are [B+1] prefix tables (device); a CTA finds its cloud by binary search and works on that cloud's rows and
 // its own seeds only.  B == 0: the single-cloud launch (whole arrays).  Emitted indices are rows of the CONCATENATED
-// cloud array, so the gather that follows needs no per-cloud bookkeeping.
+// cloud array, so the gather that follows needs no per-cloud bookkeeping.  A cloud may start at any row c0: the bulk
+// copies of the thread-per-seed kernel need 16-byte-aligned sources, so its tiles start at the aligned row c0 & ~3 and
+// the first c0 & 3 rows they hold belong to the previous cloud.
 struct KnnSegs { const int64_t* blk_off; const int64_t* cloud_off; const int64_t* seed_off; int B; };
 __device__ __forceinline__ void knn_resolve(const KnnSegs& g, int per_block, int64_t& c0, int64_t& N, int64_t& s0, int64_t& s_end) {
   if (g.B == 0) { c0 = 0; s0 = (int64_t)blockIdx.x * per_block; return; }      // N, s_end stay as passed
@@ -98,8 +102,14 @@ knn_seed_kernel(const double* __restrict__ cloud, const float* __restrict__ clou
   const uint32_t bar0 = smem_u32(knn_sm + 2 * 3 * KNN_TILE * sizeof(float));
   int64_t c0, sb;
   knn_resolve(segs, KNN_THREADS, c0, N, sb, S);
+  // the bulk copies need 16-byte-aligned sources: tiles start at the aligned row c0 & ~3 and rows are numbered from there,
+  // so this cloud's rows are lead .. lead + N - 1 (lead == 0 in the single-cloud launch); the shift is the same for every
+  // row, so the heap's (distance, index) order is the cloud-local one
+  const int lead = (int)(c0 & 3);
+  c0 -= lead;
+  const int64_t NT = N + lead;
   cloud += 3 * c0;
-  const float* cx = cloud32 + c0; const float* cy = cx + npad_all; const float* cz = cy + npad_all;   // SoA rows of this cloud
+  const float* cx = cloud32 + c0; const float* cy = cx + npad_all; const float* cz = cy + npad_all;
   const int64_t s = sb + threadIdx.x;
   const bool active = s < S;
   const float rmax = *rmax_p;
@@ -114,7 +124,7 @@ knn_seed_kernel(const double* __restrict__ cloud, const float* __restrict__ clou
   float tau32 = FLT_MAX;
 
   auto consider = [&](int gi) {
-    if (gi >= N) return;                                                // padding row
+    if ((uint32_t)(gi - lead) >= (uint32_t)N) return;                   // padding row or another cloud's row
     const double ex = cloud[3 * (int64_t)gi] - sx, ey = cloud[3 * (int64_t)gi + 1] - sy, ez = cloud[3 * (int64_t)gi + 2] - sz;
     const double d = __dadd_rn(__dadd_rn(__dmul_rn(ex, ex), __dmul_rn(ey, ey)), __dmul_rn(ez, ez));
     if (!key_less(d, gi, tau, tau_i)) return;
@@ -141,10 +151,10 @@ knn_seed_kernel(const double* __restrict__ cloud, const float* __restrict__ clou
   // double-buffered SoA tiles: thread 0 asks the TMA engine for tile t+1 while the CTA works on tile t
   if (threadIdx.x == 0) { mbar_init(bar0, 1); mbar_init(bar0 + 8, 1); fence_barrier_init(); }
   __syncthreads();
-  const int64_t ntiles = (N + KNN_TILE - 1) / KNN_TILE;
+  const int64_t ntiles = (NT + KNN_TILE - 1) / KNN_TILE;
   auto issue = [&](int64_t t) {
     const int64_t base = t * KNN_TILE;
-    const int64_t rows = (N - base) < KNN_TILE ? ((N - base + 3) / 4 * 4) : KNN_TILE;     // the padding rows make every copy 16-byte granular
+    const int64_t rows = (NT - base) < KNN_TILE ? ((NT - base + 3) / 4 * 4) : KNN_TILE;   // the padding rows make every copy 16-byte granular
     const uint32_t bytes = (uint32_t)rows * 4u, bar = bar0 + 8u * (uint32_t)(t & 1);
     const uint32_t dst = smem_u32(tile + (t & 1) * 3 * KNN_TILE);
     mbar_expect_tx(bar, 3 * bytes);
@@ -157,7 +167,7 @@ knn_seed_kernel(const double* __restrict__ cloud, const float* __restrict__ clou
     if (threadIdx.x == 0 && t + 1 < ntiles) issue(t + 1);               // its buffer was released by the barrier that ended tile t-1
     while (!mbar_try_wait(bar0 + 8u * (uint32_t)(t & 1), (uint32_t)((t >> 1) & 1))) { }
     const int64_t base = t * KNN_TILE;
-    const int tn = (N - base) < KNN_TILE ? (int)((N - base + 3) / 4 * 4) : KNN_TILE;
+    const int tn = (NT - base) < KNN_TILE ? (int)((NT - base + 3) / 4 * 4) : KNN_TILE;
     if (active) {
       const float4* xs = reinterpret_cast<const float4*>(tile + (t & 1) * 3 * KNN_TILE);
       const float4* ys = xs + KNN_TILE / 4;

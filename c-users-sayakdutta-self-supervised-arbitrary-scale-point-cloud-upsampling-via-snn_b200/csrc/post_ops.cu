@@ -14,7 +14,8 @@ namespace cg = cooperative_groups;
 
 namespace sapcu {
 
-// avg[i] = mean_j sqrt(|p_i - p_idx[i][j]|^2), numpy's pairwise summation order for a row of K doubles
+// avg[i] = mean_j sqrt(|p_i - p_idx[i][j]|^2), numpy's pairwise summation order for a row of K <= 128 doubles (numpy
+// halves longer rows recursively, an order this kernel does not restate)
 // qry: the S query points (== pts for the single-GPU filter; a rank's own rows of the gathered points when sharded)
 __global__ void knn_mean_dist_kernel(const double* __restrict__ pts, const double* __restrict__ qry, const int32_t* __restrict__ idx,
                                      int64_t S, int K, double* __restrict__ avg) {
@@ -129,6 +130,7 @@ size_t sapcu_outlier_workspace_bytes(int64_t S) { return S < 0 ? 0 : align_up((s
 int sapcu_outlier_mask(const double* d_points, int64_t S, const int32_t* d_idx, int K, double threshold, uint8_t* d_keep,
                        void* d_ws, size_t ws_bytes, void* stream) {
   SAPCU_REQUIRE(S >= 0 && K >= 1 && (S == 0 || (d_points && d_idx && d_keep && d_ws)), "outlier_mask: bad argument");
+  SAPCU_REQUIRE(K <= 128, "outlier_mask: K=%d > 128", K);
   if (ws_bytes < sapcu_outlier_workspace_bytes(S)) { set_error("outlier_mask: workspace too small"); return SAPCU_EWORKSPACE; }
   if (S == 0) return 0;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
@@ -146,6 +148,7 @@ int sapcu_outlier_mask(const double* d_points, int64_t S, const int32_t* d_idx, 
 int sapcu_knn_mean_dist(const double* d_points, int64_t S, const double* d_query, int64_t rows, const int32_t* d_idx, int K,
                         double* d_mean, void* stream) {
   SAPCU_REQUIRE(S >= 1 && rows >= 0 && K >= 1 && d_points && (rows == 0 || (d_query && d_idx && d_mean)), "knn_mean_dist: bad argument");
+  SAPCU_REQUIRE(K <= 128, "knn_mean_dist: K=%d > 128", K);
   if (rows == 0) return 0;
   knn_mean_dist_kernel<<<(unsigned)ceil_div(rows, 128), 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(d_points, d_query, d_idx, rows, K, d_mean);
   SAPCU_LAUNCH_CHECK();
@@ -170,6 +173,7 @@ int sapcu_fps(const float* d_xyz, int64_t N, int64_t npoint, int64_t start, int3
               void* stream) {
   SAPCU_REQUIRE(d_xyz && d_out && d_ws && N >= 1 && npoint >= 0 && start >= 0 && start < N, "fps: bad argument");
   SAPCU_REQUIRE(ws_bytes >= 32, "fps: workspace of 32 bytes needed");
+  SAPCU_REQUIRE(reinterpret_cast<uintptr_t>(d_ws) % 8 == 0, "fps: workspace %p is not 8-byte aligned", d_ws);
   SAPCU_REQUIRE(N < ((int64_t)1 << 31) && npoint < ((int64_t)1 << 31), "fps: sizes must fit 32 bits");
   if (npoint == 0) return 0;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);

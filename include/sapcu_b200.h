@@ -75,18 +75,21 @@ int64_t sapcu_profile_report(char* h_buf, size_t cap);
  * K1  seed -> input-cloud kNN.  Replaces sklearn KDTree(data).query(chunk, K)
  *     (generation.py:110,127,153).  Exact: ordering by fp64 squared distance
  *     accumulated as ((dx*dx)+(dy*dy))+(dz*dz) without contraction, ties broken by the lowest
- *     cloud index; d_idx[s*K + j] ascending in distance.  K <= 128, K <= N.
+ *     cloud index; d_idx[s*K + j] ascending in distance.  K <= 128, K <= N.  d_ws must be 16-byte
+ *     aligned (the cloud's fp32 copy is read with bulk copies), else SAPCU_EINVAL before any launch.
  * ---------------------------------------------------------------------------------- */
 size_t sapcu_knn_workspace_bytes(int64_t N);   /* fp32 SoA copy of the cloud + one scalar */
 int sapcu_knn(const double* d_cloud, int64_t N, const double* d_seeds, int64_t S, int K,
               int32_t* d_idx, void* d_ws, size_t ws_bytes, void* stream);
 
 /* Batched form: B independent (cloud, seed set) problems in ONE launch -- the per-file loop of generate.py:135-160
- * (one KDTree per input file) for a batch of small clouds.  d_clouds / d_seeds are the concatenated [N_total,3] /
+ * (one KDTree per input file) for a batch of clouds of any sizes; the kernel flavour follows the largest cloud, and the
+ * clouds may start at any row of the concatenated array.  d_clouds / d_seeds are the concatenated [N_total,3] /
  * [S_total,3] fp64 arrays, h_cloud_off / h_seed_off HOST prefix tables of B+1 entries (first 0, last the total).
  * Seeds of problem b see only cloud b; d_idx[s*K + j] is a row of the CONCATENATED cloud array (cloud-local index +
  * h_cloud_off[b]), so sapcu_gather_center_rotate runs on the concatenated arrays unchanged.  Same exactness and
- * tie-break as sapcu_knn; every non-empty problem needs N_b >= K.  Synchronises the stream once (offset upload). */
+ * tie-break as sapcu_knn; every non-empty problem needs N_b >= K; d_ws 16-byte aligned as for sapcu_knn.  Synchronises
+ * the stream once (offset upload). */
 size_t sapcu_knn_batched_workspace_bytes(int64_t N_total, int B);
 int sapcu_knn_batched(const double* d_clouds, const int64_t* h_cloud_off, const double* d_seeds,
                       const int64_t* h_seed_off, int B, int K, int32_t* d_idx,
@@ -125,6 +128,9 @@ int sapcu_seedgen(const double* d_cloud, int64_t N, double cell, int quirk_origi
 /* ------------------------------------------------------------------------------------
  * Outlier filter ("next" row 2), generation.py:176-183: with d_idx = the k = 30 self-neighbours of every output point
  * (sapcu_knn with cloud == seeds == points), keep[i] = mean_j |p_i - p_idx[i][j]| < threshold * (global mean).
+ * Each row mean sums its K distances in numpy's pairwise order for K <= 128 (np.mean of the [S,K] distances, bit for
+ * bit); K > 128, where numpy changes its order and which sapcu_knn cannot produce, is refused with SAPCU_EINVAL.  The
+ * same holds for sapcu_knn_mean_dist below.
  * ---------------------------------------------------------------------------------- */
 size_t sapcu_outlier_workspace_bytes(int64_t S);
 int sapcu_outlier_mask(const double* d_points, int64_t S, const int32_t* d_idx, int K, double threshold,
@@ -143,8 +149,11 @@ int sapcu_outlier_mask_from_means(const double* d_mean_all, int64_t S, int64_t r
 
 /* ------------------------------------------------------------------------------------
  * Farthest point sampling ("next" row 3), generate.py:56-74: fp32, start index `start` (the reference uses N/2),
- * running distances initialised to 1e32, ties -> lowest index.  d_out: int32 [npoint] selected indices in order.
- * One cooperative persistent kernel (a grid barrier per selected point); workspace: 32 bytes.
+ * running distances initialised to 1e32, ties -> lowest index.  d_out: int32 [npoint] selected indices in order; once
+ * every running distance is 0 (every distinct point picked, e.g. npoint > N) further picks are index 0, as in the
+ * reference.  One cooperative persistent kernel (a
+ * grid barrier per selected point) holding 8 points per thread in registers: N beyond what the co-resident CTAs hold is
+ * refused with SAPCU_EINVAL.  Workspace: 32 bytes, 8-byte aligned (64-bit atomics), else SAPCU_EINVAL.
  * ---------------------------------------------------------------------------------- */
 int sapcu_fps(const float* d_xyz, int64_t N, int64_t npoint, int64_t start, int32_t* d_out,
               void* d_ws, size_t ws_bytes, void* stream);

@@ -32,6 +32,28 @@ void oracle_knn_f64(const double* cloud, int64_t n, const double* seeds, int64_t
     free(bd);
 }
 
+/* farthest_point_sample (reference generate.py:56-74) in fp32 from any start index: running distances 1e32, squared
+ * distance (dx*dx + dy*dy) + dz*dz, `dist < distance` update, arg-max with the first maximum (lowest index). */
+void oracle_fps_f32(const float* xyz, int64_t n, int64_t npoint, int64_t start, int64_t* out) {
+    float* dist = (float*)malloc(sizeof(float) * (size_t)n);
+    for (int64_t i = 0; i < n; ++i) dist[i] = 1e32f;
+    int64_t far = start;
+    for (int64_t it = 0; it < npoint; ++it) {
+        out[it] = far;
+        const float cx = xyz[3 * far], cy = xyz[3 * far + 1], cz = xyz[3 * far + 2];
+        int64_t best = 0;
+        float bd = -1.0f;
+        for (int64_t p = 0; p < n; ++p) {
+            const float dx = xyz[3 * p] - cx, dy = xyz[3 * p + 1] - cy, dz = xyz[3 * p + 2] - cz;
+            const float d = (dx * dx + dy * dy) + dz * dz;
+            if (d < dist[p]) dist[p] = d;
+            if (dist[p] > bd) { bd = dist[p]; best = p; }
+        }
+        far = best;
+    }
+    free(dist);
+}
+
 static float clampf(float v, float lo, float hi) { return fminf(fmaxf(v, lo), hi); }
 
 /* eval-mode soft spike (reference fn/snn_coder.py:135-153) */

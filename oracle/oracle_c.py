@@ -37,6 +37,16 @@ def knn(cloud, seeds, k):
     return idx
 
 
+def fps(xyz, npoint, start=None):
+    """farthest_point_sample in fp32 (sapcu_oracle.fps restated in C, any start; default N // 2) -> int64 [npoint]"""
+    xyz = np.ascontiguousarray(xyz, np.float32)
+    n = xyz.shape[0]
+    out = np.empty(npoint, np.int64)
+    lib().oracle_fps_f32(_p(xyz), ctypes.c_int64(n), ctypes.c_int64(npoint), ctypes.c_int64(n // 2 if start is None else start),
+                         _p(out))
+    return out
+
+
 def neuron_chain(x, prm4, T, eif2=None):
     x = np.ascontiguousarray(x, np.float32)
     prm4 = np.ascontiguousarray(prm4, np.float32)

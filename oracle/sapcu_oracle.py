@@ -361,14 +361,14 @@ def outlier_filter(xyz, threshold=1.5, k=30):
     return np.where(avg < avgtotal * threshold)[0]
 
 
-def fps(xyz, npoint):
-    """farthest_point_sample (generate.py:56-74) restated in numpy float32: start at N // 2, distances 1e32,
+def fps(xyz, npoint, start=None):
+    """farthest_point_sample (generate.py:56-74) restated in numpy float32: start at N // 2 (or `start`), distances 1e32,
     `dist < distance` update, arg-max (first maximum)."""
     xyz = np.asarray(xyz, dtype=np.float32)
     n = xyz.shape[0]
     out = np.zeros(npoint, dtype=np.int64)
     distance = np.full(n, 1e32, dtype=np.float32)
-    far = n // 2
+    far = n // 2 if start is None else int(start)
     for i in range(npoint):
         out[i] = far
         d = xyz - xyz[far]

@@ -150,3 +150,28 @@ def test_outlier_filter_and_fps_oracles(golden):
     assert np.array_equal(orc.fps(g["fps_xyz"], 512), g["fps_idx"])
     grid = np.stack(np.meshgrid(np.arange(12), np.arange(12), np.arange(12), indexing="ij"), -1).reshape(-1, 3).astype(np.float64)
     assert np.array_equal(orc.fps(grid, 200), g["fps_grid_idx"])
+
+
+def test_fps_c_oracle_matches_numpy_oracle_and_reference(golden):
+    """oracle_c.fps (the plain-C FPS the GPU tests compare whole pick sequences with) equals the numpy restatement and the
+    reference's own picks, ties included."""
+    g = golden.post
+    assert np.array_equal(oracle_c.fps(g["fps_xyz"], 512), g["fps_idx"])
+    grid = np.stack(np.meshgrid(np.arange(12), np.arange(12), np.arange(12), indexing="ij"), -1).reshape(-1, 3).astype(np.float64)
+    assert np.array_equal(oracle_c.fps(grid, 200), g["fps_grid_idx"])
+    rng = np.random.default_rng(21)
+    pts = rng.normal(size=(5000, 3))
+    assert np.array_equal(oracle_c.fps(pts, 700), orc.fps(pts, 700))
+    # tie-heavy: the grid stored twice (every distance is shared by at least two rows), 1e4 + a unit sphere (fp32 at
+    # magnitude), identical points, and more picks than points (the picks after exhaustion are index 0)
+    twice = np.concatenate([grid, grid], 0)
+    assert np.array_equal(oracle_c.fps(twice, 300), orc.fps(twice, 300))
+    far = rng.normal(size=(3000, 3)); far = 1e4 + far / np.linalg.norm(far, axis=1, keepdims=True)
+    assert np.array_equal(oracle_c.fps(far, 400), orc.fps(far, 400))
+    same = np.full((100, 3), 0.25)
+    assert np.array_equal(oracle_c.fps(same, 5), orc.fps(same, 5))
+    assert np.array_equal(oracle_c.fps(pts[:40], 45), orc.fps(pts[:40], 45))
+    assert (oracle_c.fps(pts[:40], 45)[40:] == 0).all()
+    for start in (0, 1234, 4999):
+        assert np.array_equal(oracle_c.fps(pts, 200, start=start), orc.fps(pts, 200, start=start))
+        assert np.array_equal(oracle_c.fps(twice, 100, start=start % 3456), orc.fps(twice, 100, start=start % 3456))
