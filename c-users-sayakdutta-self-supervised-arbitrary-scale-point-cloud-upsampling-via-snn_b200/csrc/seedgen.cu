@@ -11,7 +11,8 @@
 // Faithful quirks (dense.cpp line numbers): the kd-tree is built over po[0..pnumber] INCLUSIVE (:193), i.e. with one
 // extra all-zero point (`quirk_origin`); voxel ids use int arithmetic that may alias at the grid border (:189,:203-208,
 // :237-240); comparisons against 0.0f / 1.0f literals; the emitted coordinates pass through "%lf" (6 decimals,
-// :232) before generation.py reads them back (`round6`).  The reference's 5000-point cap (po[5001], :64) does not apply.
+// :232) before generation.py reads them back (`round6`, restated exactly by round6_text).  The reference's 5000-point
+// cap (po[5001], :64) does not apply.
 // All geometry is fp64 and this file is compiled with -fmad=false so every product/sum rounds as in the g++ build.
 // Roofline: FP64 issue for the brute-force 10-NN (N+1 pair evaluations per visited voxel); HBM traffic negligible.
 #include <float.h>
@@ -30,12 +31,36 @@ __device__ __forceinline__ V3 voxel_center(int id, int B, double cell) {
   return {x * cell + 0.5 * cell - 0.5, y * cell + 0.5 * cell - 0.5, z * cell + 0.5 * cell - 0.5};
 }
 
+// fprintf("%lf") + np.loadtxt (dense.cpp:232): the nearest double to c rounded to 6 decimals, half to even on the EXACT
+// decimal value of c.  p = c * 1e6 is the nearest double to the exact product; rounding p instead of the product goes
+// wrong only when p lands on a half-integer that the product is not (at cells 1/320 and 1/960 up to a third of the seeds
+// carry such a coordinate), so there the sign of the exact residual fma(c, 1e6, -p) picks the side.  m / 1e6 is then the
+// correctly rounded quotient of two exact integers, which is what strtod returns for the 6-decimal text.
+__device__ __forceinline__ double round6_text(double c) {
+  const double p = c * 1e6;
+  double m = nearbyint(p);                       // half to even: right when p is not a half-integer or is exactly one
+  const double fl = floor(p);
+  if (p - fl == 0.5) {
+    const double r = fma(c, 1e6, -p);            // exact: c * 1e6 - p
+    if (r > 0.0) m = fl + 1.0;
+    else if (r < 0.0) m = fl;
+  }
+  return m / 1e6;
+}
+
 __device__ __forceinline__ bool bit_get(const unsigned* bm, int64_t i) { return (bm[i >> 5] >> (i & 31)) & 1u; }
 
-// initial queue: voxel id of every input point (dense.cpp:186-191)
-__global__ void seed_init_kernel(const double* __restrict__ cloud, int64_t N, double cell, int B, int* __restrict__ q) {
+// initial queue: voxel id of every input point (dense.cpp:186-191); a point outside the accepted box (NaN included)
+// raises *outside and is not converted (its id could leave the int range)
+__global__ void seed_init_kernel(const double* __restrict__ cloud, int64_t N, double cell, int B, double lim, int* __restrict__ q,
+                                 int* __restrict__ outside) {
   const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (i >= N) return;
+  if (!(fabs(cloud[3 * i]) <= lim && fabs(cloud[3 * i + 1]) <= lim && fabs(cloud[3 * i + 2]) <= lim)) {
+    atomicOr(outside, 1);
+    q[i] = 0;
+    return;
+  }
   const double v = floor((cloud[3 * i] + 0.5) / cell) * B * B + floor((cloud[3 * i + 1] + 0.5) / cell) * B +
                    floor((cloud[3 * i + 2] + 0.5) / cell);
   q[i] = (int)v;
@@ -47,7 +72,7 @@ __global__ void seed_claim_kernel(const int* __restrict__ q, int n, const unsign
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const int64_t id = q[i];
-  if (id < id_lo || id >= id_hi) return;          // cannot be decoded consistently: never evaluated (see launcher note)
+  if (id < id_lo || id >= id_hi) return;          // unreachable for an accepted cloud (see seed_plan)
   if (bit_get(evaluated, id - id_lo)) return;
   atomicMin(&claim[id - id_lo], i);
 }
@@ -195,9 +220,7 @@ __global__ void seed_commit_kernel(const int* __restrict__ q, int n, const int* 
     const int64_t o = seeds_base + emit_pos[i];
     if (o < cap) {
       V3 c = voxel_center(id, B, cell);
-      if (round6) {   // fprintf("%lf") + np.loadtxt: nearest double to the 6-decimal rendering
-        c.x = nearbyint(c.x * 1e6) / 1e6; c.y = nearbyint(c.y * 1e6) / 1e6; c.z = nearbyint(c.z * 1e6) / 1e6;
-      }
+      if (round6) { c.x = round6_text(c.x); c.y = round6_text(c.y); c.z = round6_text(c.z); }
       seeds[3 * o] = c.x; seeds[3 * o + 1] = c.y; seeds[3 * o + 2] = c.z;
     }
   }
@@ -231,12 +254,16 @@ static SeedPlan seed_plan(int64_t N, double cell, int64_t cap) {
   SeedPlan p;
   p.B = (int)round(1.0 / cell);
   const int64_t B = p.B;
-  // x is the top "digit" of a voxel id, so the flood fill legitimately runs past x = B when the cloud touches the +x
-  // face (the band reaches 0.015 + one cell beyond the surface); y/z overflow and negative indices alias exactly as in
-  // the reference.  Ids outside [id_lo, id_hi) cannot be produced by an expanding voxel.
-  const int64_t xpad = (int64_t)ceil(0.015 / cell) + 4;
-  p.id_lo = -(B * B + B + 1);
-  p.id_hi = (B + xpad + 1) * B * B + 2 * (B * B + B + 1);
+  // Every cloud coordinate lies in [-0.5 - cell, 0.5 + cell] (sapcu_seedgen refuses other clouds), and so does every
+  // triangle the 10-NN can form (the quirk point is the origin).  A voxel expands only if its centre lies within 0.015
+  // of such a triangle, so its decoded indices satisfy -k0 - 1 <= x <= B + k0 + 1 and -k0 - 1 <= y, z <= B - 1
+  // (k0 = ceil(0.015 / cell); y and z of a decoded id lie in (-B, B)), and a child's indices are one step further out:
+  // with k = k0 + 2, every id the fill produces -- initial ones included -- is x B^2 + y B + z with -k <= x <= B + k and
+  // -k <= y, z <= B, i.e. in [id_lo, id_hi).  x is the top "digit" of an id, so the fill runs past x = B at the +x face
+  // and below x = 0 at the -x face; y/z overflow and negative ids alias exactly as in the reference.
+  const int64_t k = (int64_t)ceil(0.015 / cell) + 2;
+  p.id_lo = -k * (B * B + B + 1);
+  p.id_hi = (B + k) * B * B + B * B + B + 1;
   p.nvox = p.id_hi - p.id_lo;
   // a level holds 6 children per expanding voxel; a level is a thin shell of the band around the surface, bounded here
   // by 64 B^2 voxels (a unit-box surface has <= 6 B^2 cells per layer) independently of the output capacity
@@ -274,7 +301,7 @@ using namespace sapcu;
 extern "C" {
 
 size_t sapcu_seedgen_workspace_bytes(int64_t N, double cell, int64_t cap) {
-  if (N < 1 || !(cell > 0.0) || cap < 1 || 1.0 / cell > 1000.0) return 0;
+  if (N < 1 || N >= (1 << 30) || !(cell > 0.0) || cap < 1 || 1.0 / cell > 1000.0) return 0;
   return seed_plan(N, cell, cap).bytes;
 }
 
@@ -296,10 +323,16 @@ int sapcu_seedgen(const double* d_cloud, int64_t N, double cell, int quirk_origi
   int* sums = reinterpret_cast<int*>(ws + p.off_sums);
   int* totals = reinterpret_cast<int*>(ws + p.off_total);
   SAPCU_CUDA_CHECK(cudaMemsetAsync(evaluated, 0, ((size_t)p.nvox + 31) / 32 * 4, st));
+  SAPCU_CUDA_CHECK(cudaMemsetAsync(totals, 0, 3 * sizeof(int), st));
   fill_i32_kernel<<<1184, 256, 0, st>>>(claim, p.nvox, 0x7fffffff);
   SAPCU_LAUNCH_CHECK();
-  seed_init_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, st>>>(d_cloud, N, cell, p.B, q[0]);
+  const double lim = 0.5 + cell;
+  seed_init_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, st>>>(d_cloud, N, cell, p.B, lim, q[0], totals + 2);
   SAPCU_LAUNCH_CHECK();
+  int outside = 0;
+  SAPCU_CUDA_CHECK(cudaMemcpyAsync(&outside, totals + 2, sizeof(int), cudaMemcpyDeviceToHost, st));
+  SAPCU_CUDA_CHECK(cudaStreamSynchronize(st));
+  SAPCU_REQUIRE(!outside, "seedgen: a cloud coordinate lies outside [-%g, %g] (the unit box plus one cell)", lim, lim);
   int64_t n = N, emitted = 0;
   int cur = 0;
   for (int level = 0; n > 0; ++level) {

@@ -119,7 +119,11 @@ int sapcu_displace(const double* d_seeds, const float* d_normals, const float* d
  * same (FIFO) order as the reference binary.  quirk_origin != 0 keeps the reference's extra all-zero point in the
  * 10-NN search (dense.cpp:193); round6 != 0 rounds coordinates to 6 decimals like the "%lf" text round trip.
  * d_seeds: [cap,3] f64 (first min(count, cap) seeds are stored); *h_count (HOST) receives the total count.
- * Synchronises the stream once per flood-fill level.
+ * The cloud must lie in the unit box the reference normalises to, with one cell of slack for rounding: a coordinate
+ * outside [-0.5 - cell, 0.5 + cell] (or NaN) is refused with SAPCU_EINVAL, naming the bound.  Also refused
+ * (SAPCU_EINVAL): N < 1, N >= 2^30, cap < 1, cell <= 0, 1 / cell > 1000, null pointers; the workspace size function
+ * returns 0 for exactly these sizes.  A workspace below sapcu_seedgen_workspace_bytes gives SAPCU_EWORKSPACE before
+ * any launch.  Synchronises the stream once before the fill and once per flood-fill level.
  * ---------------------------------------------------------------------------------- */
 size_t sapcu_seedgen_workspace_bytes(int64_t N, double cell, int64_t cap);
 int sapcu_seedgen(const double* d_cloud, int64_t N, double cell, int quirk_origin, int round6,

@@ -77,6 +77,38 @@ def gather_center_rotate(cloud, seeds, idx, normals=None):
     return out
 
 
+def round6_text(v):
+    """fprintf("%lf") read back with strtod, elementwise"""
+    v = np.ascontiguousarray(v, np.float64)
+    out = np.empty_like(v)
+    lib().oracle_round6_text(_p(v), ctypes.c_int64(v.size), _p(out))
+    return out
+
+
+def seedgen(cloud, cell, quirk_origin=True, round6=True, cap=None, max_levels=4096):
+    """The seed generator as a serial FIFO flood fill -> (seeds [min(count, cap), 3] f64, count, level_stats [levels, 2]).
+    An explicit `cap` keeps only the first `cap` seeds (count stays the total); by default all are returned.
+    level_stats[L] = (queue entries of BFS level L, 6 * voxels of level L that expand)."""
+    cloud = np.ascontiguousarray(cloud, np.float64)
+    n = cloud.shape[0]
+    grow, cap = cap is None, (1 << 22 if cap is None else cap)
+    while True:
+        out = np.empty((cap, 3), np.float64)
+        stats = np.zeros((max_levels, 2), np.int64)
+        count = ctypes.c_int64(0)
+        f = lib().oracle_seedgen
+        f.restype = ctypes.c_int64
+        levels = f(_p(cloud), ctypes.c_int64(n), ctypes.c_double(cell), ctypes.c_int(int(quirk_origin)),
+                   ctypes.c_int(int(round6)), _p(out), ctypes.c_int64(cap), ctypes.byref(count), _p(stats),
+                   ctypes.c_int64(max_levels))
+        if levels < 0:
+            raise MemoryError("oracle_seedgen")
+        assert levels <= max_levels
+        if count.value <= cap or not grow:
+            return out[:min(count.value, cap)], count.value, stats[:levels]
+        cap = count.value
+
+
 def displace(seeds, normals, dist):
     seeds = np.ascontiguousarray(seeds, np.float64)
     normals = np.ascontiguousarray(normals, np.float32)
